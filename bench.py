@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # CPU arm: trimesh if importable, else the oracle port
+    python bench.py --gpus 1 ... --dump-outputs DIR          # also write the last timed step's results to DIR/*.npy
 
 N = 1  (config.workload = "config2"): icosphere subdivision 7 (327 680 triangles), 3840x2160 pinhole camera rays
        (8 294 400 rays, origin a stride-0 broadcast as in the reference's test/performance_test.py:36-41),
@@ -22,6 +23,11 @@ N > 1  (config.workload = "config5"): north_star's multi-GPU job — 16.8 M-tria
 Timing: W >= 3 warm-up steps; every timed step is bracketed by CUDA events on the launch stream with an L2 flush
 (512 MiB memset) between steps at N = 1 (at N > 1 a step's working set is 6 GB >> L2); the job time is the max over
 ranks of the summed step times.  Clocks are sampled through NVML during the timed region.
+
+--dump-outputs DIR (N = 1): after the timed steps, the closest-hit 5-tuple of the last step is written for a fixed,
+seeded sample of DUMP_RAYS of the frame's rays as DIR/{ray_index,hit,front,tri_idx,location,uv}.npy (float64 ray
+indices into the flattened frame, everything else float32; 40 MiB in all).  The workload is deterministic, so two
+builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -33,6 +39,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True      # the checkout may be read-only: nothing is written into it, not even __pycache__
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (os.path.join(ROOT, "trimesh-ray-optix_b200"), ROOT):
     if p not in sys.path:
@@ -50,6 +57,7 @@ CFG5_RAYS_PER_GPU = 125_000_000
 STRONG_RAYS = 8 * WIDTH * HEIGHT    # 66 355 200: one batch split N ways
 E2E_RAYS_PER_GPU = 25_000_000       # N > 1: rays per rank and step of the host-buffer end-to-end leg
 PARITY_RAYS = 1_000_000
+DUMP_RAYS = 1 << 20
 WORKLOAD2 = "config2: icosphere subdiv 7 (327680 tris), 3840x2160 pinhole rays, intersects_closest (hit, front, tri, loc, uv)"
 WORKLOAD5 = ("config5: 4096x2048 heightfield (16777216 tris) built on rank 0 + NCCL broadcast, 125M random rays per GPU "
              "(seed 100+rank), intersects_closest(stream_compaction=True)")
@@ -216,6 +224,16 @@ def parity_closest(om, res, o, d, idx=None) -> dict:
             "against": "oracle MIRROR (binary32) on the true-size mesh"}
 
 
+def dump_closest(out_dir: str, res, n: int) -> None:
+    """Writes the rows of a dense closest-hit 5-tuple over n rays picked by a fixed seed as out_dir/<name>.npy."""
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(DUMP_RAYS, n), replace=False))
+    sel = torch.from_numpy(idx).to(res[0].device)
+    np.save(os.path.join(out_dir, "ray_index.npy"), idx.astype(np.float64))
+    for name, t in zip(("hit", "front", "tri_idx", "location", "uv"), res):
+        rows = t.reshape(n, *t.shape[res[0].dim():])[sel]
+        np.save(os.path.join(out_dir, f"{name}.npy"), rows.cpu().numpy().astype(np.float32))   # tri_idx < 2^24: exact
+
+
 def parity_ints(name, got, ref) -> dict:
     nb = int((np.asarray(got).reshape(-1) != np.asarray(ref).reshape(-1)).sum())
     return {"parity": "bit-exact" if nb == 0 else "MISMATCH", "rays_checked": int(np.asarray(ref).size),
@@ -251,7 +269,7 @@ def run_reference(args):
     mesh = oracle.OracleMesh(v, f, use_bvh=True)
     for _ in range(max(min(args.warmup, 2), 1)):
         oracle.query(mesh, o_s, d_s, oracle.MIRROR, closest_only=True, want=want)
-    steps = max(1, min(args.steps, 20))
+    steps = args.steps
     t0 = time.perf_counter()
     for _ in range(steps):
         oracle.query(mesh, o_s, d_s, oracle.MIRROR, closest_only=True, want=want)
@@ -560,6 +578,9 @@ def run_b200_single(args, dev):
         torch.cuda.synchronize()
     step_ms = [a.elapsed_time(b) for a, b in ev]
     total_ms = sum(step_ms)
+    if args.dump_outputs:
+        assert len(f) < 1 << 24, "tri_idx would not be exact in float32"
+        dump_closest(args.dump_outputs, res, n)
 
     # end-to-end through the host-buffer entry points: pinned host rays in, pinned host results out
     o_host = torch.tensor([0.0, 0.0, 3.0]).pin_memory()
@@ -875,7 +896,15 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-configs", action="store_true", help="skip the per-config block and the oracle parity checks (quick runs, ncu)")
     ap.add_argument("--rays-per-gpu", type=int, default=0, help="N > 1 only: override config 5's 125 M rays per GPU (experiments)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="N = 1 only: write the last timed step's results (seeded sample) "
+                                                          "to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs:
+        if args.impl != "b200" or args.gpus != 1 or int(os.environ.get("WORLD_SIZE", "1")) != 1:
+            ap.error("--dump-outputs is implemented for the CUDA path with --gpus 1")
+        os.makedirs(args.dump_outputs, exist_ok=True)
     if args.impl == "reference":
         run_reference(args)
     else:
