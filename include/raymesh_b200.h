@@ -261,6 +261,22 @@ int rt_contains_parity(const void* blob, const rt_ray_desc* points, const rt_tra
 int rt_trace_stats(const void* blob, const rt_ray_desc* rays, const rt_trace_opts* opts, int mode,
                    uint64_t* counters_dev, void* scratch, void* stream);
 
+/* ---- Closest point on the mesh (trimesh.proximity.closest_point; no counterpart in the reference).
+ *      Outputs dense over the point batch/window: closest f32x3, distance f32, tri i32, uv f32x2 = (w0, w1).
+ *      max_distance: +inf = unbounded; NaN or negative -> RT_ERR_INVALID. counters_dev: NULL or u64[4].
+ *      `points` describes the batch through the origins fields of rt_ray_desc (directions ignored), opts supplies
+ *      the window (ray_first / ray_count); tmax and schedule are ignored.  tri_idx[i] is the triangle minimising
+ *      (d2, tri) over all triangles with d2 <= fl(max_distance * max_distance), d2 being the binary32 squared
+ *      distance of the closest point rt_point.cuh computes; ties go to the smaller index, so the result does not
+ *      depend on the BVH or the launch.  distance = correctly rounded sqrt(d2).  uv are the weights of the
+ *      triangle's vertices 0 and 1 (the convention of rt_trace_closest).  No triangle within reach (empty mesh,
+ *      non-finite point, everything beyond max_distance): tri -1, distance +inf, closest 0, uv 0.
+ *      counters_dev (instrumented kernel when not NULL): [0] BVH8 nodes fetched, [1] triangles tested, [2] points,
+ *      [3] points with an answer.  `scratch` is accepted like every trace call's and left untouched. */
+int rt_closest_point(const void* blob, const rt_ray_desc* points, const rt_trace_opts* opts, float max_distance,
+                     float* closest, float* distance, int32_t* tri_idx, float* uv, uint64_t* counters_dev,
+                     void* scratch, void* stream);
+
 /* ---- Host-buffer entry points (end-to-end path): rays and results live in (pinned) HOST memory.
  *      Copies ray chunks H2D, traces and copies results D2H on internal streams, overlapping
  *      the three; `dev_work` is caller-provided device memory of rt_host_closest_sizes() bytes.

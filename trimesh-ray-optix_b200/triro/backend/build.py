@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.normpath(os.path.join(HERE, "..", "..", "csrc"))
 INCLUDE = os.path.normpath(os.path.join(HERE, "..", "..", "..", "include"))
 LIB_PATH = os.path.join(HERE, "libtriro_b200.so")
-UNITS = ["rt_build.cu", "rt_trace.cu", "rt_compact.cu", "rt_host.cu"]
+UNITS = ["rt_build.cu", "rt_trace.cu", "rt_compact.cu", "rt_host.cu", "rt_closest.cu"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 NVCC_FLAGS = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
 

@@ -99,6 +99,7 @@ def _declare(lib):
         "rt_compact_scatter_at": (ci, [vp, i64, vp, vp, vp, vp, vp, i64, ci, vp, vp, vp, vp, vp, vp]),
         "rt_contains_parity": (ci, [vp, prd, pto, pf, pf, pf, vp, vp, vp, vp, vp, vp]),
         "rt_trace_stats": (ci, [vp, prd, pto, ci, vp, vp, vp]),
+        "rt_closest_point": (ci, [vp, prd, pto, C.c_float, vp, vp, vp, vp, vp, vp, vp]),
         "rt_host_closest_sizes": (ci, [i64, psz]),
         "rt_host_trace_closest": (ci, [vp, i64, vp, ci, vp, pto, vp, vp, vp, vp, vp, vp, sz]),
         "rt_host_trace_closest_compact": (ci, [vp, i64, vp, ci, vp, pto, vp, vp, vp, vp, vp, vp, C.POINTER(C.c_int64), vp, sz]),
@@ -774,6 +775,43 @@ def trace_stats(accel_structure, origins: torch.Tensor, dirs: torch.Tensor, mode
     rays = max(c[2], 1)
     return dict(nodes=c[0], tris=c[1], rays=c[2], hits=c[3], nodes_per_ray=c[0] / rays, tris_per_ray=c[1] / rays,
                 hit_fraction=c[3] / rays)
+
+
+def closest_point(accel_structure, points: torch.Tensor, max_distance: float = float("inf"), ray_first: int = 0,
+                  ray_count: int = -1, counters: torch.Tensor | None = None):
+    """Closest point on the mesh for every query point (trimesh.proximity.closest_point): returns
+    (closest Float32[*b,3], distance Float32[*b], tri Int32[*b], uv Float32[*b,2]) with uv = weights of the triangle's
+    vertices 0 and 1.  Only triangles within `max_distance` count; a point with none (or a non-finite point, or an
+    empty mesh) gets tri -1, distance +inf, closest 0, uv 0.  Equal distances go to the smaller triangle index.
+    With a window [ray_first, ray_first + ray_count) of the flattened batch the outputs are 1-D over the window.
+    `counters` (Int64[4] on the device, optional) selects the instrumented kernel: nodes fetched, triangles tested,
+    points, points with an answer."""
+    tensor_input_check(points)
+    md = float(max_distance)
+    if md != md or md < 0.0:
+        raise ValueError(f"max_distance must be >= 0 or inf (got {max_distance})")
+    blob = _blob_of(accel_structure, points.device)
+    rd, batch = make_ray_desc(points, None)
+    if ray_first != 0 or ray_count >= 0:
+        batch = (_window(rd.nray, ray_first, ray_count),)
+    dev = points.device
+    if counters is not None and (counters.dtype != torch.int64 or counters.device != dev or counters.numel() != 4
+                                 or not counters.is_contiguous()):
+        raise ValueError("counters must be a contiguous int64 tensor of 4 elements on the points' device")
+    with _on_device(dev):
+        closest = torch.empty((*batch, 3), dtype=torch.float32, device=dev)
+        distance = torch.empty(batch, dtype=torch.float32, device=dev)
+        tri = torch.empty(batch, dtype=torch.int32, device=dev)
+        uv = torch.empty((*batch, 2), dtype=torch.float32, device=dev)
+        if tri.numel() == 0:
+            if counters is not None:
+                counters.zero_()
+            return closest, distance, tri, uv
+        st = _stream(dev)
+        _check(get_module().rt_closest_point(_ptr(blob), C.byref(rd), C.byref(trace_opts(accel_structure, ray_first, ray_count)),
+                                             md, _ptr(closest), _ptr(distance), _ptr(tri), _ptr(uv), _ptr(counters),
+                                             _ptr(_scratch(dev, st)), st), "rt_closest_point")
+    return closest, distance, tri, uv
 
 
 def host_closest(accel_structure, origins_host: torch.Tensor, dirs_host: torch.Tensor, out: dict | None = None,

@@ -61,3 +61,15 @@ class RayMeshIntersector:
     def contains_points(self, points):
         p = torch.from_numpy(np.ascontiguousarray(np.asarray(points, dtype=np.float32).reshape(-1, 3))).to(self.device)
         return self._rmi.contains_points(p).cpu().numpy()
+
+    def _points(self, points):
+        return torch.from_numpy(np.ascontiguousarray(np.asarray(points, dtype=np.float32).reshape(-1, 3))).to(self.device)
+
+    def closest_point(self, points):
+        """trimesh.proximity.closest_point -> (closest (n,3) float64, distance (n,) float64, triangle_id (n,) int64)"""
+        c, d, t = self._rmi.closest_point(self._points(points))
+        return c.cpu().numpy().astype(np.float64), d.cpu().numpy().astype(np.float64), t.cpu().numpy().astype(np.int64)
+
+    def signed_distance(self, points):
+        """trimesh.proximity.signed_distance -> (n,) float64, positive inside the mesh"""
+        return self._rmi.signed_distance(self._points(points)).cpu().numpy().astype(np.float64)

@@ -140,6 +140,25 @@ class RayMeshIntersector:
             return tri_c, ray_idx, loc_c
         return tri_c, ray_idx
 
+    def closest_point(self, points: torch.Tensor, max_distance: Optional[float] = None, return_uv: bool = False):
+        """(closest[*b,3], distance[*b], triangle_id[*b][, uv[*b,2]]) — the nearest point of the mesh surface for
+        every query point, in the order of trimesh.proximity.closest_point.  Triangles farther than `max_distance`
+        (None = unbounded) are ignored; a point with no triangle in reach gets triangle_id -1, distance inf and
+        closest 0.  Equal distances go to the smaller triangle index.  uv are the weights of the triangle's vertices
+        0 and 1 like intersects_closest's, so `interpolate(attr, triangle_id, uv)` transfers attributes."""
+        md = float("inf") if max_distance is None else float(max_distance)
+        closest, distance, tri, uv = hops.closest_point(self.as_wrapper, points, md)
+        if return_uv:
+            return closest, distance, tri, uv
+        return closest, distance, tri
+
+    def signed_distance(self, points: torch.Tensor) -> torch.Tensor:
+        """Float32[*b] — distance to the surface, positive inside and negative outside (trimesh.proximity.signed_distance).
+        The sign is `contains_points` (with its documented decision procedure); an exact 0 is returned as +0.0."""
+        _, d, _ = self.closest_point(points)
+        inside = self.contains_points(points.reshape(-1, 3)).reshape(d.shape)
+        return torch.where(inside | (d == 0), d, -d)
+
     DEFAULT_CHECK_DIRECTION = (0.4395064455, 0.617598629942, 0.652231566745)   # reference :245-247
 
     def contains_parity(self, points: torch.Tensor, direction, active: Optional[torch.Tensor] = None, out=None,
