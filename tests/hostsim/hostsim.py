@@ -36,7 +36,8 @@ def lib():
         _LIB.hs_build.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_size_t]
         _LIB.hs_build_sah.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_size_t]
         _LIB.hs_trace.argtypes = [C.c_void_p, C.c_int, C.c_int64] + [C.c_void_p] * 10
-        _LIB.hs_check_blob.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p]
+        _LIB.hs_check_blob.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]
+        _LIB.hs_canonical.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p]
         _LIB.hs_frame_check.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]
         _LIB.hs_blob_prims.argtypes = [C.c_void_p, C.c_void_p]
         _LIB.hs_refit.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_size_t]
@@ -78,12 +79,28 @@ def refit_blob(blob: np.ndarray, vertices, faces) -> np.ndarray:
     return out
 
 
-def check_blob(blob: np.ndarray):
-    """Returns (code, info) — code 0 means structurally valid and conservative."""
+def check_blob(blob: np.ndarray, vertices=None, faces=None):
+    """Returns (code, info) — code 0 means valid: structure, conservative slot boxes, parent links, header and layout,
+    zero padding.  With vertices and faces also every record against its face and bad_index_faces (codes: hs_check_blob)."""
     blob = np.ascontiguousarray(blob, dtype=np.uint8)
     info = np.zeros(4, dtype=np.uint64)
-    rc = lib().hs_check_blob(_p(blob), blob.nbytes, _p(info))
+    v = f = None
+    if faces is not None:
+        v = np.ascontiguousarray(vertices, dtype=np.float32).reshape(-1, 3)
+        f = np.ascontiguousarray(faces, dtype=np.int32).reshape(-1, 3)
+    rc = lib().hs_check_blob(_p(blob), blob.nbytes, _p(v), 0 if v is None else len(v), _p(f), 0 if f is None else len(f),
+                             _p(info))
     return rc, dict(nodes=int(info[0]), tris=int(info[1]), depth=int(info[2]), children=int(info[3]))
+
+
+def canonical(blob: np.ndarray) -> np.ndarray:
+    """hs_canonical: the blob with nodes numbered breadth-first and records in the order the nodes reference them."""
+    blob = np.ascontiguousarray(blob, dtype=np.uint8)
+    out = np.empty_like(blob)
+    rc = lib().hs_canonical(_p(blob), blob.nbytes, _p(out))
+    if rc != 0:
+        raise RuntimeError(f"hs_canonical failed: {rc}")
+    return out
 
 
 def blob_prims(blob: np.ndarray, n_tris: int) -> np.ndarray:

@@ -39,7 +39,7 @@ MESHES = ["tri1", "tri2", "tri3", "tri4", "tri9", "ico0", "ico2", "ico4", "soup"
 def test_blob_structure_and_conservative_quantisation(name):
     v, f = mesh(name)
     blob = hostsim.build_blob(v, f)
-    code, info = hostsim.check_blob(blob)
+    code, info = hostsim.check_blob(blob, v, f)
     assert code == 0, f"hs_check_blob -> {code}"
     assert info["tris"] == len(f)
     assert np.array_equal(np.sort(hostsim.blob_prims(blob, len(f))), np.arange(len(f)))

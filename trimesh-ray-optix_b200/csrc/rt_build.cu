@@ -11,7 +11,7 @@
 //   k_refit         bottom-up boxes with one atomic counter per inner node
 //   k_collapse      persistent cooperative kernel, one grid-wide level per iteration:
 //                   greedy surface-area collapse to 8-wide quantised nodes + triangle records
-//   k_finalize      blob header
+//   k_finalize      blob header, zeroed alignment gaps of the used prefix
 #include <cooperative_groups.h>
 #include <string.h>
 #include "rt_api.h"
@@ -61,14 +61,6 @@ struct BuildState {
     uint32_t pad[6];
 };
 
-__device__ __forceinline__ uint32_t f2ord(float f) {
-    const uint32_t u = __float_as_uint(f);
-    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__device__ __forceinline__ float ord2f(uint32_t u) {
-    return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u);
-}
-
 struct Workspace {
     BuildState* state;
     uint64_t* keys;
@@ -117,34 +109,35 @@ __device__ __forceinline__ bool load_tri(const float* __restrict__ verts, int64_
 
 __global__ void __launch_bounds__(256) k_init_state(BuildState* st) {
     if (threadIdx.x == 0 && blockIdx.x == 0) {
-        for (int a = 0; a < 3; ++a) { st->bounds_lo[a] = 0xffffffffu; st->bounds_hi[a] = 0u; }
+        for (int a = 0; a < 3; ++a) { st->bounds_lo[a] = kOrdPosInf; st->bounds_hi[a] = kOrdNegInf; }
         st->node_count = 1u;
     }
 }
 
 __global__ void __launch_bounds__(256) k_scene_bounds(const float* __restrict__ verts, int64_t nv,
                                                       const int32_t* __restrict__ faces, int64_t n, BuildState* st) {
-    float lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
+    // ordered-uint encoding throughout (rt_build_core.cuh): the box does not depend on the order of the reduction
+    uint32_t lo[3] = {kOrdPosInf, kOrdPosInf, kOrdPosInf}, hi[3] = {kOrdNegInf, kOrdNegInf, kOrdNegInf};
     uint32_t bad = 0;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
         float v[9];
         if (!load_tri(verts, nv, faces, i, v)) ++bad;
         const BBox b = tri_bbox(v[0], v[1], v[2], v[3], v[4], v[5], v[6], v[7], v[8]);
-        lo[0] = fminf(lo[0], b.lx); lo[1] = fminf(lo[1], b.ly); lo[2] = fminf(lo[2], b.lz);
-        hi[0] = fmaxf(hi[0], b.hx); hi[1] = fmaxf(hi[1], b.hy); hi[2] = fmaxf(hi[2], b.hz);
+        lo[0] = min(lo[0], ord_lo(b.lx)); lo[1] = min(lo[1], ord_lo(b.ly)); lo[2] = min(lo[2], ord_lo(b.lz));
+        hi[0] = max(hi[0], ord_hi(b.hx)); hi[1] = max(hi[1], ord_hi(b.hy)); hi[2] = max(hi[2], ord_hi(b.hz));
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
 #pragma unroll
         for (int a = 0; a < 3; ++a) {
-            lo[a] = fminf(lo[a], __shfl_xor_sync(0xffffffffu, lo[a], o));
-            hi[a] = fmaxf(hi[a], __shfl_xor_sync(0xffffffffu, hi[a], o));
+            lo[a] = min(lo[a], __shfl_xor_sync(0xffffffffu, lo[a], o));
+            hi[a] = max(hi[a], __shfl_xor_sync(0xffffffffu, hi[a], o));
         }
         bad += __shfl_xor_sync(0xffffffffu, bad, o);
     }
     // block-level reduction first: one set of atomics per CTA instead of per warp
-    __shared__ float s_lo[8][3], s_hi[8][3];
+    __shared__ uint32_t s_lo[8][3], s_hi[8][3];
     __shared__ uint32_t s_bad[8];
     const int warp = threadIdx.x >> 5;
     if ((threadIdx.x & 31) == 0) {
@@ -156,15 +149,13 @@ __global__ void __launch_bounds__(256) k_scene_bounds(const float* __restrict__ 
     if (threadIdx.x == 0) {
         for (int w = 1; w < 8; ++w) {
 #pragma unroll
-            for (int a = 0; a < 3; ++a) { lo[a] = fminf(lo[a], s_lo[w][a]); hi[a] = fmaxf(hi[a], s_hi[w][a]); }
+            for (int a = 0; a < 3; ++a) { lo[a] = min(lo[a], s_lo[w][a]); hi[a] = max(hi[a], s_hi[w][a]); }
             bad += s_bad[w];
         }
 #pragma unroll
         for (int a = 0; a < 3; ++a) {
-            if (lo[a] <= hi[a]) {
-                atomicMin(&st->bounds_lo[a], f2ord(lo[a]));
-                atomicMax(&st->bounds_hi[a], f2ord(hi[a]));
-            }
+            if (lo[a] != kOrdPosInf) atomicMin(&st->bounds_lo[a], lo[a]);
+            if (hi[a] != kOrdNegInf) atomicMax(&st->bounds_hi[a], hi[a]);
         }
         if (bad) atomicAdd(&st->bad_index, bad);
     }
@@ -240,7 +231,7 @@ __global__ void __launch_bounds__(256) k_refit(const float* __restrict__ verts, 
         for (int64_t k = a + threadIdx.x; k <= b; k += blockDim.x) {
             float v[9];
             load_tri(verts, nv, faces, (int64_t)sorted_prim[k], v);
-            const BBox lb = tri_bbox(v[0], v[1], v[2], v[3], v[4], v[5], v[6], v[7], v[8]);
+            const BBox lb = leaf_bbox(tri_bbox(v[0], v[1], v[2], v[3], v[4], v[5], v[6], v[7], v[8]));
             store_box_cg(&box[(n - 1) + k], lb);
             if (n == 1) continue;
             uint32_t me = (uint32_t)((n - 1) + k);
@@ -306,11 +297,8 @@ __global__ void __launch_bounds__(256) k_fill_tris(const float* __restrict__ ver
 }
 
 // The (parent << 3 | slot) array of the wide nodes (only rt_bvh_refit reads it) is built in the workspace and placed
-// right behind the nodes actually in use, so that the used prefix of the blob - what travels over NCCL or to disk -
-// is complete: a blob received by broadcast or load can be re-fitted like the original.
-__host__ __device__ inline uint64_t parents_offset_for(uint64_t nodes_offset, uint32_t n_nodes) {
-    return (nodes_offset + (uint64_t)n_nodes * 80u + 255u) / 256u * 256u;
-}
+// right behind the nodes actually in use (parents_offset_for), so that the used prefix of the blob - what travels over
+// NCCL or to disk - is complete: a blob received by broadcast or load can be re-fitted like the original.
 
 __global__ void __launch_bounds__(256) k_place_parents(uint8_t* blob, const BuildState* st, BlobLayout lay,
                                                        const uint32_t* __restrict__ wide_parent) {
@@ -320,20 +308,35 @@ __global__ void __launch_bounds__(256) k_place_parents(uint8_t* blob, const Buil
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_nodes; i += stride) dst[i] = wide_parent[i];
 }
 
+// One warp: lane 0 writes the header (and the root of an empty mesh), all lanes zero the alignment gaps inside the
+// used prefix, so that the prefix a save() or a broadcast carries depends on the mesh alone (the blob itself comes
+// uninitialised from the caller's allocator).
 __global__ void k_finalize(rt_blob_header* hdr, const BuildState* st, int64_t n, BlobLayout lay) {
-    if (threadIdx.x != 0 || blockIdx.x != 0) return;
+    if (blockIdx.x != 0) return;
+    uint8_t* blob = reinterpret_cast<uint8_t*>(hdr);
+    const uint32_t n_nodes = n > 0 ? (st->node_count < lay.node_cap ? st->node_count : lay.node_cap) : 1u;
+    const uint64_t parents_offset = parents_offset_for(lay.nodes_offset, n_nodes);
+    const uint64_t used = used_bytes_for(parents_offset, n_nodes);
+    const uint64_t gap[4][2] = {{sizeof(rt_blob_header), lay.tris_offset},
+                                {lay.tris_offset + (uint64_t)n * 48u, lay.nodes_offset},
+                                {lay.nodes_offset + (uint64_t)n_nodes * 80u, parents_offset},
+                                {parents_offset + (uint64_t)n_nodes * 4u, used}};
+    for (int g = 0; g < 4; ++g)
+        for (uint64_t b = gap[g][0] + threadIdx.x; b < gap[g][1]; b += blockDim.x) blob[b] = 0;
+    if (threadIdx.x != 0) return;
     rt_blob_header h;
     memset(&h, 0, sizeof(h));
     h.magic = RT_BLOB_MAGIC;
     h.abi_version = RT_ABI_VERSION;
     h.n_tris = (uint32_t)n;
-    h.n_nodes = n > 0 ? (st->node_count < lay.node_cap ? st->node_count : lay.node_cap) : 1u;
+    h.n_nodes = n_nodes;
     h.depth = n > 0 ? st->depth : 1u;
     h.n_nodes_cap = lay.node_cap;
     h.tris_offset = lay.tris_offset;
     h.nodes_offset = lay.nodes_offset;
-    h.parents_offset = parents_offset_for(lay.nodes_offset, h.n_nodes);
-    h.used_bytes = (h.parents_offset + (uint64_t)h.n_nodes * 4u + 15u) / 16u * 16u;
+    h.parents_offset = parents_offset;
+    h.used_bytes = used;
+    // an empty mesh has the zero box; a mesh whose triangle boxes are all NaN has the empty box (+inf, -inf)
     for (int a = 0; a < 3; ++a) {
         h.aabb_lo[a] = n > 0 ? ord2f(st->bounds_lo[a]) : 0.0f;
         h.aabb_hi[a] = n > 0 ? ord2f(st->bounds_hi[a]) : 0.0f;
@@ -346,8 +349,8 @@ __global__ void k_finalize(rt_blob_header* hdr, const BuildState* st, int64_t n,
         Node8 nd;
         memset(&nd, 0, sizeof(nd));
         nd.ex = nd.ey = nd.ez = 1;   // imask = trimask = 0: no slot is ever reported
-        *reinterpret_cast<Node8*>(reinterpret_cast<uint8_t*>(hdr) + lay.nodes_offset) = nd;
-        *reinterpret_cast<uint32_t*>(reinterpret_cast<uint8_t*>(hdr) + h.parents_offset) = 0xffffffffu;
+        *reinterpret_cast<Node8*>(blob + lay.nodes_offset) = nd;
+        *reinterpret_cast<uint32_t*>(blob + h.parents_offset) = 0xffffffffu;
     }
 }
 

@@ -24,9 +24,12 @@ RT_HD BBox bbox_union(const BBox& a, const BBox& b) {
     return r;
 }
 
+// Written as explicit operations: the collapse compares these areas, and a sum of products left to the compiler is
+// contracted into FMAs on the device but not on the host, which picks different children when two areas tie in exact
+// arithmetic (congruent triangles of a symmetric mesh).  This is the sequence nvcc chose for the plain expression.
 RT_HD float bbox_half_area(const BBox& b) {
     const float dx = b.hx - b.lx, dy = b.hy - b.ly, dz = b.hz - b.lz;
-    return dx * dy + dy * dz + dz * dx;
+    return ffma(dz, dx, ffma(dx, dy, fmul(dy, dz)));
 }
 
 // Triangle box, widened by a few ulps so that the watertight triangle test (which may accept
@@ -36,11 +39,49 @@ RT_HD BBox tri_bbox(float v0x, float v0y, float v0z, float v1x, float v1y, float
     BBox b;
     b.lx = fminf(fminf(v0x, v1x), v2x); b.ly = fminf(fminf(v0y, v1y), v2y); b.lz = fminf(fminf(v0z, v1z), v2z);
     b.hx = fmaxf(fmaxf(v0x, v1x), v2x); b.hy = fmaxf(fmaxf(v0y, v1y), v2y); b.hz = fmaxf(fmaxf(v0z, v1z), v2z);
-    const float k = 6.0e-7f, tiny = 1.0e-30f;
-    b.lx -= fabsf(b.lx) * k + tiny; b.ly -= fabsf(b.ly) * k + tiny; b.lz -= fabsf(b.lz) * k + tiny;
-    b.hx += fabsf(b.hx) * k + tiny; b.hy += fabsf(b.hy) * k + tiny; b.hz += fabsf(b.hz) * k + tiny;
+    const float k = 6.0e-7f, tiny = 1.0e-30f;   // |x| * k + tiny as one FMA, as nvcc contracts it, on the host as well
+    b.lx -= ffma(fabsf(b.lx), k, tiny); b.ly -= ffma(fabsf(b.ly), k, tiny); b.lz -= ffma(fabsf(b.lz), k, tiny);
+    b.hx += ffma(fabsf(b.hx), k, tiny); b.hy += ffma(fabsf(b.hy), k, tiny); b.hz += ffma(fabsf(b.hz), k, tiny);
     b.pad0 = 0.f; b.pad1 = 0.f;
     return b;
+}
+
+// Leaf box of the binary hierarchy: the triangle box united with the empty box, so that an axis on which all three
+// vertices are NaN is empty (+inf, -inf) instead of NaN - the box refit_node computes for the same triangle, so that a
+// refit to the build's own vertices reproduces the built nodes bit for bit.  (fminf ignores a NaN operand, so nothing
+// changes on any other axis.)
+RT_HD BBox leaf_bbox(const BBox& tb) {
+    BBox e; e.lx = e.ly = e.lz = INFINITY; e.hx = e.hy = e.hz = -INFINITY; e.pad0 = e.pad1 = 0.f;
+    return bbox_union(e, tb);
+}
+
+// ------------------------------------------------------------------ scene bounds
+// The scene box is reduced in the ordered-uint encoding of binary32, a total order with -0 < +0 in which a NaN never
+// wins: the result does not depend on the order of the reduction (fminf leaves min(-0, +0) open), and a mesh whose
+// triangle boxes are all NaN keeps the initial values, an empty box (+inf, -inf) per axis.
+#if defined(__CUDA_ARCH__)
+RT_HD uint32_t float_bits(float f) { return __float_as_uint(f); }
+#else
+RT_HD uint32_t float_bits(float f) { union { float f; uint32_t u; } c; c.f = f; return c.u; }
+#endif
+RT_HD uint32_t f2ord(float f) {
+    const uint32_t u = float_bits(f);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+RT_HD float ord2f(uint32_t u) { return as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u); }
+constexpr uint32_t kOrdPosInf = 0xff800000u;   // f2ord(+inf): start of a min
+constexpr uint32_t kOrdNegInf = 0x007fffffu;   // f2ord(-inf): start of a max
+RT_HD uint32_t ord_lo(float f) { return f == f ? f2ord(f) : 0xffffffffu; }   // NaN: above every number, never a min
+RT_HD uint32_t ord_hi(float f) { return f == f ? f2ord(f) : 0u; }            // NaN: below every number, never a max
+
+// ------------------------------------------------------------------ blob layout behind the nodes
+// The (parent << 3 | slot) array of the wide nodes sits right behind the nodes in use, so that the used prefix of the
+// blob - what travels over NCCL or to disk - is complete; used_bytes ends 16-byte aligned behind it.
+RT_HD uint64_t parents_offset_for(uint64_t nodes_offset, uint32_t n_nodes) {
+    return (nodes_offset + (uint64_t)n_nodes * 80u + 255u) / 256u * 256u;
+}
+RT_HD uint64_t used_bytes_for(uint64_t parents_offset, uint32_t n_nodes) {
+    return (parents_offset + (uint64_t)n_nodes * 4u + 15u) / 16u * 16u;
 }
 
 // ------------------------------------------------------------------ Morton codes (21 bits per axis)
