@@ -117,11 +117,12 @@ typedef struct rt_blob_header {
  */
 #define RT_SCHED_AUTO 0
 #define RT_SCHED_DIRECT 1       /* triangles tested inside the node step, per lane (round-1 coherent schedule) */
-#define RT_SCHED_QUEUED 2       /* per-lane triangle queues (round-1 incoherent schedule) */
+#define RT_SCHED_QUEUED 2       /* removed schedule (per-lane triangle queues): accepted as RT_SCHED_COOP_INCOHERENT,
+                                   the number is not reused */
 #define RT_SCHED_COOP_COHERENT 3   /* warp-shared (ray, triangle) pair list tested by all 32 lanes, late re-fill */
 #define RT_SCHED_COOP_INCOHERENT 4 /* same, early re-fill from a pool of prepared rays */
-#define RT_SCHED_SLOTS 5           /* rays live in per-warp slots handed around by queues: lanes never wait for triangle
-                                      tests, results are written 32 rays at a time (closest / first / any / count) */
+#define RT_SCHED_SLOTS 5           /* removed schedule (rays in per-warp slots): accepted as RT_SCHED_COOP_INCOHERENT,
+                                      the number is not reused */
 #define RT_OPT_SCRATCH_ZEROED 1u
 #define RT_OPT_STOP_WHEN_BROKEN 2u /* rt_contains_parity only: the launch may stop as soon as flags_dev[1] (any broken) is
                                       known to be 1; contain / broken entries are then unspecified for the points it skipped.

@@ -471,14 +471,14 @@ def test_trace_stats_counts_agree_with_host_simulation(cuda_device):
     assert sq["rays"] == 40_000 and sq["hits"] == st["hits"] and sq["nodes"] >= st["nodes"]
 
 
-def test_direct_and_queued_schedules_give_identical_results(cuda_device):
+def test_coherent_and_incoherent_auto_schedules_give_identical_results(cuda_device):
     v, f = synth.icosphere(5)
     r = make(v, f)
     o, d = synth.pinhole_rays(640, 360, device=cuda_device)
-    a = closest_to_numpy(r.intersects_closest(o, d))                            # broadcast origin: direct
-    b = closest_to_numpy(r.intersects_closest(o.contiguous(), d))               # materialised origins: queued
+    a = closest_to_numpy(r.intersects_closest(o, d))                            # broadcast origin: coop_coherent
+    b = closest_to_numpy(r.intersects_closest(o.contiguous(), d))               # materialised origins: coop_incoherent
     for k in a:
-        assert_bits_equal(a[k], b[k], f"direct vs queued {k}")
+        assert_bits_equal(a[k], b[k], f"coherent vs incoherent {k}")
     assert torch.equal(r.intersects_count(o, d), r.intersects_count(o.contiguous(), d))
     assert torch.equal(r.intersects_any(o, d), r.intersects_any(o.contiguous(), d))
 
@@ -762,5 +762,5 @@ def test_watertight_no_leaks_on_the_gpu(cuda_device, tilt):
     got = closest_to_numpy((hit, front, tri, loc, uv))
     check_closest_vs_mirror(got, oracle.OracleMesh(v, f), flat(o), flat(d))
     assert int(r.intersects_count(o, d).min()) >= 1
-    # the same through the queued schedule (materialised per-ray origins already are) and the any-hit early exit
+    # the same through the any-hit early exit (per-ray origins: the incoherent schedule, like the queries above)
     assert bool(r.intersects_any(o, d).all())

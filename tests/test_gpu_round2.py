@@ -16,8 +16,9 @@ from triro.ray.ray_optix import RayMeshIntersector
 
 pytestmark = pytest.mark.gpu
 
-SCHEDULES = {"direct": hops.SCHED_DIRECT, "queued": hops.SCHED_QUEUED, "coop_coherent": hops.SCHED_COOP_COHERENT,
-             "coop_incoherent": hops.SCHED_COOP_INCOHERENT, "slots": hops.SCHED_SLOTS}
+# SCHED_QUEUED and SCHED_SLOTS name removed schedules: ABI v2 callers that still pass them must get the same bits
+SCHEDULES = {"direct": hops.SCHED_DIRECT, "coop_coherent": hops.SCHED_COOP_COHERENT, "coop_incoherent": hops.SCHED_COOP_INCOHERENT,
+             "legacy_queued": hops.SCHED_QUEUED, "legacy_slots": hops.SCHED_SLOTS}
 
 
 def make(v, f, **kw):
@@ -42,7 +43,7 @@ class knobs:
 # ---------------------------------------------------------------- schedules
 @pytest.mark.parametrize("scene", ["camera_ico5", "random_soup20k"])
 def test_all_schedules_give_identical_results(cuda_device, scene):
-    """direct / queued (per-lane triangle tests, round 1) and the two warp-cooperative schedules must agree bit
+    """direct (per-lane triangle tests, round 1), the two warp-cooperative schedules and the legacy numbers must agree bit
     for bit on every query, for any pair-list threshold: the closest hit is resolved by (t, primitive index),
     never by test order."""
     if scene == "camera_ico5":
@@ -56,7 +57,7 @@ def test_all_schedules_give_identical_results(cuda_device, scene):
     r = make(v, f)
     base = None
     for name, sched in SCHEDULES.items():
-        for thr in ((0,) if sched <= hops.SCHED_QUEUED else (0, 1, 7, 96)):
+        for thr in ((0,) if sched == hops.SCHED_DIRECT else (0, 1, 7, 96)):
             with knobs(schedule=sched, tri_threshold=thr):
                 got = dict(closest=closest_to_numpy(r.intersects_closest(o, d)), first=r.intersects_first(o, d).cpu().numpy(),
                            any=r.intersects_any(o, d).cpu().numpy(), count=r.intersects_count(o, d).cpu().numpy())

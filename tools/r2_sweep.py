@@ -1,4 +1,4 @@
-"""Round-2 schedule sweep on ONE GPU: every traversal schedule (direct / queued = round 1, coop_coherent /
+"""Round-2 schedule sweep on ONE GPU: every traversal schedule (direct = round 1, coop_coherent /
 coop_incoherent = warp-cooperative triangle tests) x pair-list threshold on the BASELINE scenes, with a
 bit-equality check between schedules, the nodes / triangles fetched per ray and the roofline fraction.
 
@@ -19,7 +19,7 @@ dev = torch.device("cuda:0")
 PEAK = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))["hbm_gbs"] if os.path.exists(os.path.join(ROOT, "MEASURED_PEAKS.json")) else 6650.0
 flush = torch.empty(512 << 20, dtype=torch.uint8, device=dev)
 rows = []
-NAMES = {0: "auto", 1: "direct", 2: "queued", 3: "coop_coherent", 4: "coop_incoherent", 5: "slots"}
+NAMES = {0: "auto", 1: "direct", 3: "coop_coherent", 4: "coop_incoherent"}
 
 
 def timed(fn, reps=5, warm=2):
@@ -62,13 +62,13 @@ for name in scenes:
         queries += [("any", r.intersects_any, 1, "any"), ("count", r.intersects_count, 4, "count")]
     base = {}
     for qname, fn, b_out, smode in queries:
-        for sched in [int(x) for x in os.environ.get("SWEEP_SCHEDS", "1,2,3,4,5").split(",")]:
-            thrs = [0] if sched <= 2 else ([8, 16, 24, 32, 64] if sched == 3 else [16, 32, 64, 96])
+        for sched in [int(x) for x in os.environ.get("SWEEP_SCHEDS", "1,3,4").split(",")]:
+            thrs = [0] if sched == 1 else ([8, 16, 24, 32, 64] if sched == 3 else [16, 32, 64, 96])
             if os.environ.get("SWEEP_THRS"):
-                thrs = [int(x) for x in os.environ["SWEEP_THRS"].split(",")] if sched > 2 else [0]
+                thrs = [int(x) for x in os.environ["SWEEP_THRS"].split(",")] if sched != 1 else [0]
             if sched in (1, 3) and not coherent and name != "soup1m":
                 thrs = thrs[:1]          # late re-fill on incoherent batches: one point is enough
-            if sched in (2, 4) and coherent and name == "small":
+            if sched == 4 and coherent and name == "small":
                 thrs = thrs[:1]
             refills = [int(x) for x in os.environ.get("SWEEP_REFILL", "0").split(",")] if sched >= 3 else [0]
             for thr, refill in [(t, rf) for t in thrs for rf in refills]:

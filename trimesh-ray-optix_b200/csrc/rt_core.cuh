@@ -263,18 +263,6 @@ RT_HD uint32_t shift_in_sign(float x, uint32_t acc) {
 }
 #endif
 
-// (acc << 1) | (signbit(a) | signbit(b) | signbit(c))
-#if defined(__CUDA_ARCH__)
-RT_HD uint32_t shift_in_signs(float a, float b, float c, uint32_t acc) {
-    return __funnelshift_l(__float_as_uint(a) | __float_as_uint(b) | __float_as_uint(c), acc, 1);
-}
-#else
-RT_HD uint32_t shift_in_signs(float a, float b, float c, uint32_t acc) {
-    union { float f; uint32_t u; } x, y, z; x.f = a; y.f = b; z.f = c;
-    return (acc << 1) | ((x.u | y.u | z.u) >> 31);
-}
-#endif
-
 RT_HD uint32_t spread3(uint32_t x) {   // bit i (0..7) -> bit 3i
     x = (x | (x << 8)) & 0x0000f00fu;
     x = (x | (x << 4)) & 0x000c30c3u;
@@ -339,10 +327,6 @@ RT_HD uint32_t node_test(const Ray& r, const U4& n0, const U4& n1, const U4& n2,
     // pipe, leaving one ALU-pipe instruction per child (the ALU pipe is the kernel's bottleneck)
     uint32_t miss = 0;
     const uint32_t magic = r.magic;
-#if defined(__CUDA_ARCH__) && defined(RT_NODE_FFMA2)
-    const float2 ax2 = make_float2(ax, ax), ay2 = make_float2(ay, ay), az2 = make_float2(az, az);
-    const float2 cx2 = make_float2(cnx, cfx), cy2 = make_float2(cny, cfy), cz2 = make_float2(cnz, cfz);
-#endif
 #pragma unroll
     for (int half = 1; half >= 0; --half) {
         const uint32_t lox = half ? n2.y : n2.x, loy = half ? n2.w : n2.z, loz = half ? n3.y : n3.x;
@@ -350,44 +334,18 @@ RT_HD uint32_t node_test(const Ray& r, const U4& n0, const U4& n1, const U4& n2,
         const uint32_t nx = negx ? hix : lox, fx = negx ? lox : hix;
         const uint32_t ny = negy ? hiy : loy, fy = negy ? loy : hiy;
         const uint32_t nz = negz ? hiz : loz, fz = negz ? loz : hiz;
-#if defined(__CUDA_ARCH__) && defined(RT_NODE_FFMA2)
-        // packed FP32 FMA of sm_100 (fma.rn.f32x2): the near and the far plane of one axis in one instruction - same
-        // IEEE results lane by lane, half the issue slots.  Measured: +0.8 % on camera rays, -1...-4 % on incoherent
-        // batches (profiles/r2_sweeps.md) - off by default.
-#define RT_PLANES(I)                                                                                            \
-            const float2 px2 = __ffma2_rn(make_float2(byte_plus_32768<I>(nx, magic), byte_plus_32768<I>(fx, magic)), ax2, cx2); \
-            const float2 py2 = __ffma2_rn(make_float2(byte_plus_32768<I>(ny, magic), byte_plus_32768<I>(fy, magic)), ay2, cy2); \
-            const float2 pz2 = __ffma2_rn(make_float2(byte_plus_32768<I>(nz, magic), byte_plus_32768<I>(fz, magic)), az2, cz2); \
-            const float tnx = px2.x, tfx = px2.y, tny = py2.x, tfy = py2.y, tnz = pz2.x, tfz = pz2.y;
-#else
-#define RT_PLANES(I)                                                                                            \
+        // A slot is missed iff min(tf, tmax) < max(tn, 0): clamp, subtract, collect the sign with a funnel shift.  (Sign-bit
+        // tests without the clamps and packed FFMA2 plane arithmetic were measured slower, DESIGN.md 4.1.)
+#define RT_SLAB(I)                                                                                              \
+        {                                                                                                       \
             const float tnx = fmaf(byte_plus_32768<I>(nx, magic), ax, cnx), tfx = fmaf(byte_plus_32768<I>(fx, magic), ax, cfx); \
             const float tny = fmaf(byte_plus_32768<I>(ny, magic), ay, cny), tfy = fmaf(byte_plus_32768<I>(fy, magic), ay, cfy); \
-            const float tnz = fmaf(byte_plus_32768<I>(nz, magic), az, cnz), tfz = fmaf(byte_plus_32768<I>(fz, magic), az, cfz);
-#endif
-        // A slot is missed iff min(tf, tmax) < max(tn, 0).  Default: clamp, subtract, collect the sign with a funnel shift
-        // (FADD runs on the FMA pipe, leaving one ALU-pipe instruction per slot besides the FMNMX).  RT_NODE_SIGNBITS reads
-        // the three conditions tf3 < tn3, tmax < tn3, tf3 < 0 off sign bits instead (2 FADD + 1 LOP3 for 2 FMNMX: fewer
-        // ALU-pipe instructions) - measured 1-3 % SLOWER on every workload (profiles/r2_sweeps.md), so it is off.
-#if defined(RT_NODE_SIGNBITS)
-#define RT_SLAB(I)                                                                                              \
-        {                                                                                                       \
-            RT_PLANES(I)                                                                                        \
-            const float tn3 = fmaxf(fmaxf(tnx, tny), tnz);                                                      \
-            const float tf3 = fminf(fminf(tfx, tfy), tfz);                                                      \
-            miss = shift_in_signs(tf3 - tn3, tmax - tn3, tf3, miss);                                            \
-        }
-#else
-#define RT_SLAB(I)                                                                                              \
-        {                                                                                                       \
-            RT_PLANES(I)                                                                                        \
+            const float tnz = fmaf(byte_plus_32768<I>(nz, magic), az, cnz), tfz = fmaf(byte_plus_32768<I>(fz, magic), az, cfz); \
             const float tn = fmaxf(fmaxf(tnx, tny), fmaxf(tnz, 0.0f));                                          \
             const float tf = fminf(fminf(tfx, tfy), fminf(tfz, tmax));                                          \
             miss = shift_in_sign(tf - tn, miss);                                                                \
         }
-#endif
         RT_SLAB(3) RT_SLAB(2) RT_SLAB(1) RT_SLAB(0)
-#undef RT_PLANES
 #undef RT_SLAB
     }
     const uint32_t hm8 = ~miss & 0xffu;

@@ -9,13 +9,12 @@
 // Execution model: persistent CTAs (grid = SMs x resident CTAs), one ray per lane.  A warp
 // advances all its rays one wide node at a time and, whenever too few lanes are still busy,
 // retires the finished rays and re-fills those lanes from a global ray counter with one
-// warp-aggregated atomic (Aila & Laine 2009).  Five schedules give bit-identical results
+// warp-aggregated atomic (Aila & Laine 2009).  Two schedule families give bit-identical results
 // (rt_trace_opts::schedule, DESIGN.md 4.1):
-//   this file           k_trace<MODE, STATS, QUEUED>: every lane tests its own triangles, inside the node
-//                       step (direct) or from a per-lane queue (queued; the all-hits path)
+//   this file           k_trace<MODE, STATS>: every lane tests its own triangles inside the node step (direct;
+//                       the reference path the host simulation reproduces)
 //   rt_trace_coop.cuh   k_trace_coop: (triangle, lane) pairs in a warp-shared list, tested by all 32 lanes -
-//                       the default for every query but all-hits
-//   rt_trace_slots.cuh  k_trace_slots: rays live in per-warp slots handed around by queues (opt-in)
+//                       the default for every query (coherent and incoherent variants)
 // launch() below resolves rt_trace_opts (tmax, ray window, schedule, knobs) - there is no state
 // behind a call: no environment variable, no thread-local setting, one kernel launch.
 #include <stdlib.h>
@@ -55,7 +54,8 @@ struct TraceParams {
     const uint8_t* active;       // optional per-point mask (may alias `broken`)
     int stop_on_broken;          // RT_OPT_STOP_WHEN_BROKEN
     int share_lanes;             // !RT_OPT_NO_LANE_SHARING
-    // coherent image batches [.., H, W, 3]: work index -> ray index by 8x4-pixel tiles (0 = identity), see tile_order()
+    // coherent image batches [.., H, W, 3]: work index -> ray index by 8x4-pixel tiles (0 = identity), see tile_order();
+    // tile_hw is unused and only holds the offsets of the fields after it
     uint32_t tile_per_row, tile_w, tile_hw;
     uint8_t* contain;
     uint8_t* broken;
@@ -76,7 +76,6 @@ struct LocalStack {
 
 // Every launch leaves its scratch zeroed: the last CTA to finish resets the ray counter and the CTA count, so the
 // next call on the same stream can skip its memset (RT_OPT_SCRATCH_ZEROED) and a launch is a single kernel.
-struct TraceParams;
 __device__ __forceinline__ void release_scratch(const TraceParams& p);
 
 // Work order of coherent image batches.  Lanes draw consecutive WORK indices; with the identity a warp holds 32
@@ -88,14 +87,11 @@ __device__ __forceinline__ void release_scratch(const TraceParams& p);
 #define RT_TILE_W_LOG2 3
 #endif
 constexpr uint32_t kTileWLog2 = RT_TILE_W_LOG2, kTileW = 1u << kTileWLog2, kTileH = 32u >> kTileWLog2;   // 8 x 4 pixels per warp
-#ifndef RT_TILE_FRAMES
-#define RT_TILE_FRAMES 0
-#endif
-#ifndef RT_TILE_INLINE
-#define RT_TILE_INLINE __forceinline__
-#endif
-struct TraceParams;
-__device__ RT_TILE_INLINE int64_t tile_order(const TraceParams& p, int64_t w);
+__device__ __forceinline__ int64_t tile_order(const TraceParams& p, int64_t w) {
+    if (p.tile_per_row == 0u) return w;
+    const uint32_t t = (uint32_t)w;                         // one image (launch() enables tiles for those only)
+    return (int64_t)tile_map(t, p.tile_per_row, p.tile_w, kTileWLog2);
+}
 
 enum FetchMode { kGeneral = 0, kPacked = 1, kConstant = 2, kGeneral32 = 3, kPinhole = 4 };
 
@@ -118,23 +114,6 @@ __device__ __forceinline__ int64_t ray_offset(const int64_t shape[4], const int6
 // Origin and direction of ray r: strided fetch (reference getRay, shaders.cu:35-63), the fixed direction
 // of contains_points, or a pinhole camera ray generated in registers (reference gen_rays,
 // test/performance_test.py:10-20: d = normalize(x - (w-1)/2, y - (h-1)/2, -f) @ cam_mat^T).
-__device__ RT_TILE_INLINE int64_t tile_order(const TraceParams& p, int64_t w) {
-    if (p.tile_per_row == 0u) return w;
-#if RT_TILE_FRAMES
-    uint32_t frame = 0u;
-    if ((uint64_t)w >= (uint64_t)p.tile_hw) frame = (uint32_t)((uint64_t)w / p.tile_hw);     // batches of several images
-    const uint32_t t = (uint32_t)(w - (int64_t)frame * p.tile_hw);
-#else
-    const uint32_t t = (uint32_t)w;                         // one image (launch() enables tiles for those only)
-#endif
-    const uint32_t q = tile_map(t, p.tile_per_row, p.tile_w, kTileWLog2);
-#if RT_TILE_FRAMES
-    return (int64_t)frame * p.tile_hw + (int64_t)q;
-#else
-    return (int64_t)q;
-#endif
-}
-
 template <int MODE>
 __device__ __forceinline__ void load_ray(const TraceParams& p, int64_t r_local, float& ox, float& oy, float& oz, float& dx,
                                          float& dy, float& dz) {
@@ -198,46 +177,25 @@ struct VisitorOf {
 
 // A warp re-fills its finished lanes from the global ray counter as soon as fewer than
 // `refill_threshold` lanes are still busy (defaults below; TRIRO_REFILL_THRESHOLD overrides).
-constexpr int kRefillThresholdQueued = 28;
-constexpr int kRefillThresholdSlots = 29;             // slot schedule: a lane adopts a prepared ray as soon as 4 lanes are idle
 constexpr int kRefillThresholdCoopIncoherent = 26;   // sweep r: heightfields best at 24-26, soup at 26-28 (profiles/r2_sweeps.md)
 constexpr int kRefillThresholdDirect = 8;
-// Postponed triangle tests: every lane owns a queue of pending triangle record indices in shared
-// memory (s_queue[entry][thread], conflict-free).  Node steps only enqueue; a warp runs a triangle
-// pass (one queued triangle per lane) when at least `tri_threshold` lanes have one pending, when a
-// queue could overflow on the next node (a node yields at most 24 triangles), or when no lane has
-// node work left.  This keeps the ~120-instruction watertight test at high SIMD efficiency instead
-// of running it with the few lanes that happen to hit a leaf in the same step.
-constexpr int kQueueCap = 32;
-constexpr int kQueueHigh = kQueueCap - kNodeMaxTris;   // 8: above this a lane may not take a node step
-constexpr int kTriThreshold = 8;
 // warp-cooperative schedules (rt_trace_coop.cuh): pairs listed before the warp tests them
 constexpr int kPairThresholdCoherent = 16;
 constexpr int kPairThresholdIncoherent = 24;
 constexpr int kPoolWords = 13;   // prepared ray: o, S, o permuted, 1/d, packed (kzf | octinv << 8)
 
-struct LaneQueue {
-    uint32_t (*q)[kTraceThreads];
-    int len;
-    __device__ __forceinline__ void push(uint32_t v) { q[len][threadIdx.x] = v; ++len; }
-    __device__ __forceinline__ uint32_t pop() { --len; return q[len][threadIdx.x]; }
-};
-
-// QUEUED = postpone triangle tests through the per-lane queue (incoherent batches); otherwise the
-// triangles of a hit leaf slot are tested inside the node step (coherent batches: neighbouring
-// lanes reach their leaves in the same step anyway, and the nearest hit shrinks tmax earlier).
+// Per-lane schedule (direct): the triangles of a hit leaf slot are tested inside the node step by the lane that found
+// them.  The host simulation (tests/hostsim) reproduces this kernel node for node.
 #ifndef RT_TRACE_MIN_BLOCKS
 #define RT_TRACE_MIN_BLOCKS 7
 #endif
 #ifndef RT_TRACE_MIN_BLOCKS_LIGHT      // cooperative kernels other than pooled closest-hit: 64 registers, 8 CTAs per SM
 #define RT_TRACE_MIN_BLOCKS_LIGHT 8
 #endif
-template <int MODE, bool STATS, bool QUEUED>
+template <int MODE, bool STATS>
 __global__ void __launch_bounds__(kTraceThreads, RT_TRACE_MIN_BLOCKS) k_trace(const __grid_constant__ TraceParams p) {
     using S = typename std::conditional<STATS, Stats, NoStats>::type;
     using Vis = typename VisitorOf<MODE, S>::type;
-    __shared__ uint32_t s_queue[QUEUED ? kQueueCap : 1][kTraceThreads];
-    __shared__ float s_pool[QUEUED ? kPoolWords : 1][kTraceThreads];   // prepared rays, column = warp * 32 + slot
     init_mask_luts();
     const rt_blob_header* hdr = reinterpret_cast<const rt_blob_header*>(p.blob);
     const uint8_t* tris = p.blob + hdr->tris_offset;
@@ -246,9 +204,6 @@ __global__ void __launch_bounds__(kTraceThreads, RT_TRACE_MIN_BLOCKS) k_trace(co
     const unsigned lt_mask = (1u << lane) - 1u;
     const int64_t nray = p.nray;
     LocalStack stack;
-    LaneQueue queue;
-    queue.q = s_queue;
-    queue.len = 0;
     unsigned long long st_nodes = 0, st_tris = 0, st_rays = 0, st_hits = 0;
     bool any_inside = false, any_broken = false;
 
@@ -261,71 +216,20 @@ __global__ void __launch_bounds__(kTraceThreads, RT_TRACE_MIN_BLOCKS) k_trace(co
     int phase = 0;
     int32_t count_plus = 0;
     trav_init(tv);
-    // per-warp pool of prepared rays (warp-uniform bookkeeping)
-    const int pool_col0 = (int)(threadIdx.x & ~31u);
-    int pool_head = 0, pool_count = 0;
-    int64_t pool_base = 0;
-    // per-warp retire pool (queued closest-hit only; measured slower for coherent batches): finished rays that hit something park
-    // (ray index, triangle record) here; when 32 have gathered the whole warp computes their
-    // attributes at full width (re-fetching the ray, which is cheaper than carrying its set-up)
-    constexpr bool kRetirePool = QUEUED && MODE == kClosest;
-    __shared__ uint32_t s_retire[kRetirePool ? 3 : 1][kTraceThreads];
-    int ret_count = 0;
-    auto flush_retire = [&]() {
-        if (lane < ret_count) {
-            const int col = pool_col0 + lane;
-            const int64_t rr = (int64_t)(((unsigned long long)s_retire[1][col] << 32) | s_retire[0][col]);
-            const uint32_t slot = s_retire[2][col];
-            float ox, oy, oz, dx, dy, dz;
-            load_ray<MODE>(p, rr, ox, oy, oz, dx, dy, dz);
-            Ray t;
-            ray_setup(t, ox, oy, oz, dx, dy, dz);
-            const uint8_t* tp = tris + (size_t)slot * 48u;
-            const U4 a = ldg128(tp), b = ldg128(tp + 16), c = ldg128(tp + 32);
-            const float v0x = as_float(a.x), v0y = as_float(a.y), v0z = as_float(a.z);
-            const float v1x = as_float(b.x), v1y = as_float(b.y), v1z = as_float(b.z);
-            const float v2x = as_float(c.x), v2y = as_float(c.y), v2z = as_float(c.z);
-            TriHit h;
-            tri_test(t, v0x, v0y, v0z, v1x, v1y, v1z, v2x, v2y, v2z, h);
-            const HitAttr at = tri_attr(h, v0x, v0y, v0z, v1x, v1y, v1z, v2x, v2y, v2z);
-            p.hit[rr] = 1; p.front[rr] = tri_front(t, h) ? 1 : 0; p.tri[rr] = (int32_t)a.w;
-            p.loc[3 * rr] = at.lx; p.loc[3 * rr + 1] = at.ly; p.loc[3 * rr + 2] = at.lz;
-            p.uv[2 * rr] = at.uv0; p.uv[2 * rr + 1] = at.uv1;
-        }
-        __syncwarp();
-        ret_count = 0;
-    };
 
     for (;;) {
-        // ---- 1. retire finished rays, re-fill free lanes from the warp's pool of prepared rays
-        const bool finished = active && nodes_done && queue.len == 0;
+        // ---- 1. retire finished rays, re-fill free lanes
+        const bool finished = active && nodes_done;
         const unsigned free_lanes = __ballot_sync(0xffffffffu, !active || finished);
         const int busy = 32 - __popc(free_lanes);
-        if (free_lanes != 0u && busy < ((exhausted && pool_count == 0) ? 1 : p.refill_threshold)) {
-            bool parked = false;
-            if constexpr (kRetirePool) {
-                const bool fin_hit = finished && vis.prim >= 0 && p.hit != nullptr;
-                const unsigned hmask = __ballot_sync(0xffffffffu, fin_hit);
-                if (hmask != 0u) {
-                    const int n_new = __popc(hmask);
-                    if (ret_count + n_new > 32) flush_retire();
-                    if (fin_hit) {
-                        const int col = pool_col0 + ret_count + __popc(hmask & lt_mask);
-                        s_retire[0][col] = (uint32_t)r; s_retire[1][col] = (uint32_t)((unsigned long long)r >> 32);
-                        s_retire[2][col] = vis.slot;
-                        parked = true;
-                    }
-                    __syncwarp();
-                    ret_count += n_new;
-                }
-            }
+        if (free_lanes != 0u && busy < (exhausted ? 1 : p.refill_threshold)) {
             if (finished) {
                 if (STATS) { st_nodes += vis.n_nodes(); st_tris += vis.n_tris(); ++st_rays; }
                 if constexpr (MODE == kClosest || MODE == kFirst) {
                     if (STATS) st_hits += vis.prim >= 0;
                     if (MODE == kFirst) {
                         if (p.tri) p.tri[r] = vis.prim;
-                    } else if (p.hit && !parked) {
+                    } else if (p.hit) {
                         if (vis.prim >= 0) {
                             const uint8_t* tp = tris + (size_t)vis.slot * 48u;
                             const U4 a = ldg128(tp), b = ldg128(tp + 16), c = ldg128(tp + 32);
@@ -381,50 +285,21 @@ __global__ void __launch_bounds__(kTraceThreads, RT_TRACE_MIN_BLOCKS) k_trace(co
                     }
                 }
             }
-            if constexpr (QUEUED) {
-                // incoherent batches re-fill early and often: rays are prepared 32 at a time by the whole
-                // warp (coalesced fetch, full-width set-up) into a shared-memory pool; a lane that frees
-                // up only copies a prepared ray
-                for (;;) {
-                    const unsigned idle = __ballot_sync(0xffffffffu, !active);
-                    if (idle == 0u) break;
-                    if (pool_count == 0) {
-                        if (exhausted) break;
-                        // prepare the next 32 rays with the whole warp: coalesced fetch, full-width set-up
-                        unsigned long long base = 0;
-                        if (lane == 0) base = atomicAdd(p.ray_counter, 32ull);
-                        base = __shfl_sync(0xffffffffu, base, 0);
-                        int64_t n = nray - (int64_t)base;
-                        if (n <= 32) exhausted = true;
-                        if (n <= 0) break;
-                        if (n > 32) n = 32;
-                        if (lane < n) {
-                            float ox, oy, oz, dx, dy, dz;
-                            load_ray<MODE>(p, (int64_t)base + lane, ox, oy, oz, dx, dy, dz);
-                            Ray t;
-                            ray_setup(t, ox, oy, oz, dx, dy, dz);
-                            const int col = pool_col0 + lane;
-                            s_pool[0][col] = t.ox; s_pool[1][col] = t.oy; s_pool[2][col] = t.oz;
-                            s_pool[3][col] = t.Sx; s_pool[4][col] = t.Sy; s_pool[5][col] = t.Sz;
-                            s_pool[6][col] = t.okx; s_pool[7][col] = t.oky; s_pool[8][col] = t.okz;
-                            s_pool[9][col] = t.idx; s_pool[10][col] = t.idy; s_pool[11][col] = t.idz;
-                            s_pool[12][col] = __int_as_float(t.kzf | (int)(t.octinv << 8));
-                        }
-                        __syncwarp();
-                        pool_base = (int64_t)base; pool_head = 0; pool_count = (int)n;
-                    }
-                    const int n_idle = __popc(idle);
-                    const int take = n_idle < pool_count ? n_idle : pool_count;
-                    const int my = __popc(idle & lt_mask);
-                    if (!active && my < take) {
-                        const int col = pool_col0 + pool_head + my;
-                        r = pool_base + pool_head + my;
-                        ray.ox = s_pool[0][col]; ray.oy = s_pool[1][col]; ray.oz = s_pool[2][col];
-                        ray.Sx = s_pool[3][col]; ray.Sy = s_pool[4][col]; ray.Sz = s_pool[5][col];
-                        ray.okx = s_pool[6][col]; ray.oky = s_pool[7][col]; ray.okz = s_pool[8][col];
-                        ray.idx = s_pool[9][col]; ray.idy = s_pool[10][col]; ray.idz = s_pool[11][col];
-                        const int packed = __float_as_int(s_pool[12][col]);
-                        ray.kzf = packed & 0xff; ray.octinv = (uint32_t)packed >> 8;
+            // re-fill late (most lanes at once): fetch and set up in place
+            const unsigned idle = __ballot_sync(0xffffffffu, !active);
+            if (idle != 0u && !exhausted) {
+                const int n_idle = __popc(idle);
+                const int leader = __ffs((int)idle) - 1;
+                unsigned long long base = 0;
+                if (lane == leader) base = atomicAdd(p.ray_counter, (unsigned long long)n_idle);
+                base = __shfl_sync(0xffffffffu, base, leader);
+                if ((int64_t)base + n_idle >= nray) exhausted = true;
+                if (!active) {
+                    r = (int64_t)base + __popc(idle & lt_mask);
+                    if (r < nray) {
+                        float ox, oy, oz, dx, dy, dz;
+                        load_ray<MODE>(p, r, ox, oy, oz, dx, dy, dz);
+                        ray_setup(ray, ox, oy, oz, dx, dy, dz);
                         ray.magic = p.byte_magic;
                         trav_init(tv);
                         vis = Vis(p.tmax);
@@ -434,69 +309,19 @@ __global__ void __launch_bounds__(kTraceThreads, RT_TRACE_MIN_BLOCKS) k_trace(co
                         phase = 0;
                         nodes_done = false;
                         active = true;
-                        if constexpr (MODE == kContains) { if (p.active && !p.active[r]) active = false; }   // masked-out point
-                    }
-                    __syncwarp();
-                    pool_head += take; pool_count -= take;
-                }
-            } else {
-                // coherent batches re-fill late (most lanes at once): fetch and set up in place
-                const unsigned idle = __ballot_sync(0xffffffffu, !active);
-                if (idle != 0u && !exhausted) {
-                    const int n_idle = __popc(idle);
-                    const int leader = __ffs((int)idle) - 1;
-                    unsigned long long base = 0;
-                    if (lane == leader) base = atomicAdd(p.ray_counter, (unsigned long long)n_idle);
-                    base = __shfl_sync(0xffffffffu, base, leader);
-                    if ((int64_t)base + n_idle >= nray) exhausted = true;
-                    if (!active) {
-                        r = (int64_t)base + __popc(idle & lt_mask);
-                        if (r < nray) {
-                            float ox, oy, oz, dx, dy, dz;
-                            load_ray<MODE>(p, r, ox, oy, oz, dx, dy, dz);
-                            ray_setup(ray, ox, oy, oz, dx, dy, dz);
-                            ray.magic = p.byte_magic;
-                            trav_init(tv);
-                            vis = Vis(p.tmax);
-                            if constexpr (MODE == kAllHits) {
-                                vis.max_hits = p.max_hits; vis.out = p.staging + (size_t)r * p.max_hits; vis.tris = tris;
-                            }
-                            phase = 0;
-                            nodes_done = false;
-                            active = true;
-                            if constexpr (MODE == kContains) { if (p.active && !p.active[r]) active = false; }
-                        }
+                        if constexpr (MODE == kContains) { if (p.active && !p.active[r]) active = false; }
                     }
                 }
             }
             if (!__any_sync(0xffffffffu, active)) {
-                if (exhausted && pool_count == 0) break;
+                if (exhausted) break;
                 continue;      // every lane drew a masked-out point (contains with `active`): draw again
             }
         }
 
-        if constexpr (!QUEUED) {
-            // ---- 2'. one wide node per lane including its triangles
-            if (active && !nodes_done) nodes_done = trav_step(nodes, tris, ray, vis, stack, tv);
-            continue;
-        }
-        // ---- 2. node phase: one wide node per lane; hit leaf slots only enqueue their triangles
-        const bool can_node = active && !nodes_done && queue.len <= kQueueHigh;
-        if (can_node) nodes_done = node_step(nodes, ray, vis, stack, tv, queue);
-
-        // ---- 3. triangle phase: one queued triangle per lane, when enough lanes have one
-        const unsigned want = __ballot_sync(0xffffffffu, queue.len > 0);
-        if (want != 0u) {
-            const bool more_nodes = active && !nodes_done && queue.len <= kQueueHigh;
-            const bool force = !__any_sync(0xffffffffu, more_nodes);
-            if (force || __popc(want) >= p.tri_threshold) {
-                if (queue.len > 0) {
-                    if (tri_one(tris, ray, vis, queue.pop())) { nodes_done = true; queue.len = 0; }   // any-hit: done
-                }
-            }
-        }
+        // ---- 2. one wide node per lane including its triangles
+        if (active && !nodes_done) nodes_done = trav_step(nodes, tris, ray, vis, stack, tv);
     }
-    if constexpr (kRetirePool) flush_retire();
     if (MODE == kContains) {
         if (__any_sync(0xffffffffu, any_inside) && lane == 0) atomicOr(&p.flags[0], 1);
         if (__any_sync(0xffffffffu, any_broken) && lane == 0) atomicOr(&p.flags[1], 1);
@@ -533,7 +358,6 @@ __device__ __forceinline__ void release_scratch(const TraceParams& p) {
 
 }  // namespace rt
 #include "rt_trace_coop.cuh"
-#include "rt_trace_slots.cuh"
 namespace rt {
 
 static int fetch_mode(const int64_t shape[4], const int64_t stride[4], int64_t nray);
@@ -577,22 +401,13 @@ constexpr int kMaxDevices = 64;
 constexpr int64_t kShareMaxRaysCoherentClosest = 1 << 20;   // coherent closest hit: launches up to this many rays share work in the tail
 static int g_per_sm[kMaxDevices][5][2][8];
 
-template <int MODE>
-constexpr bool kHasSlots = MODE == kClosest || MODE == kFirst || MODE == kAny || MODE == kCount;
-
 template <int MODE, bool STATS>
 static int occupancy(int sched, int* per_sm) {
     switch (sched) {
-        case RT_SCHED_DIRECT: return (int)cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, k_trace<MODE, STATS, false>, kTraceThreads, 0);
-        case RT_SCHED_QUEUED: return (int)cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, k_trace<MODE, STATS, true>, kTraceThreads, 0);
-        case RT_SCHED_SLOTS:
-            if constexpr (kHasSlots<MODE>)
-                return (int)cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, k_trace_slots<MODE, STATS>, kTraceThreads, 0);
-            return (int)cudaErrorInvalidValue;
-        default:
-            if (sched == RT_SCHED_COOP_COHERENT)
-                return (int)cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, k_trace_coop<MODE, STATS, false, true>, kTraceThreads, 0);
-            return (int)cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, k_trace_coop<MODE, STATS, true, true>, kTraceThreads, 0);
+        case RT_SCHED_DIRECT: return (int)cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, k_trace<MODE, STATS>, kTraceThreads, 0);
+        case RT_SCHED_COOP_COHERENT:
+            return (int)cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, k_trace_coop<MODE, STATS, false, true>, kTraceThreads, 0);
+        default: return (int)cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, k_trace_coop<MODE, STATS, true, true>, kTraceThreads, 0);
     }
 }
 
@@ -638,24 +453,22 @@ static int launch(const char* fn, TraceParams& p, const void* blob, const rt_ray
     p.tile_per_row = 0u;
     if (coherent && !(o.flags & RT_OPT_NO_TILE_ORDER) && o.ray_first == 0 && count == rays->nray) {
         const int64_t h = rays->shape[1], w = rays->shape[2];
-        if (h > 0 && w > 0 && h % kTileH == 0 && w % kTileW == 0 && h * w < ((int64_t)1 << 31) && (RT_TILE_FRAMES ? rays->nray < ((int64_t)1 << 40) : rays->nray == h * w)) {
-            p.tile_per_row = (uint32_t)(w / kTileW); p.tile_w = (uint32_t)w; p.tile_hw = (uint32_t)(h * w);
+        if (h > 0 && w > 0 && h % kTileH == 0 && w % kTileW == 0 && h * w < ((int64_t)1 << 31) && rays->nray == h * w) {
+            p.tile_per_row = (uint32_t)(w / kTileW); p.tile_w = (uint32_t)w;
         }
     }
     int sched = o.schedule;
     RT_REQUIRE(sched >= RT_SCHED_AUTO && sched <= RT_SCHED_SLOTS, RT_ERR_INVALID, "%s: unknown schedule %d", fn, sched);
     if (sched == RT_SCHED_AUTO) sched = coherent ? RT_SCHED_COOP_COHERENT : RT_SCHED_COOP_INCOHERENT;
-    // (all hits on incoherent batches took the per-lane queues until lane sharing and the root-frame test went into the
-    //  cooperative kernel: now soup 13.4 vs 13.8 ms, 4.19 M heightfield 2.22 vs 2.86 ms in its favour)
-    if (sched == RT_SCHED_SLOTS && !kHasSlots<MODE>) sched = RT_SCHED_COOP_INCOHERENT;      // contains / all hits
-    const bool early = sched == RT_SCHED_QUEUED || sched == RT_SCHED_COOP_INCOHERENT || sched == RT_SCHED_SLOTS;
-    const bool coop = sched >= RT_SCHED_COOP_COHERENT;
+    if (sched == RT_SCHED_QUEUED || sched == RT_SCHED_SLOTS) sched = RT_SCHED_COOP_INCOHERENT;   // removed schedules (ABI v2 aliases)
+    const bool coop = sched != RT_SCHED_DIRECT;
     auto clampi = [](int v, int lo, int hi) { return v < lo ? lo : (v > hi ? hi : v); };
     p.refill_threshold = o.refill_threshold > 0 ? clampi(o.refill_threshold, 1, 32)
-                                                : (sched == RT_SCHED_SLOTS ? kRefillThresholdSlots : sched == RT_SCHED_COOP_INCOHERENT ? kRefillThresholdCoopIncoherent
-                                                   : (early ? kRefillThresholdQueued : kRefillThresholdDirect));
-    p.tri_threshold = o.tri_threshold > 0 ? clampi(o.tri_threshold, 1, coop ? kPairCap - 32 : 32)
-                                          : (coop ? (early ? kPairThresholdIncoherent : kPairThresholdCoherent) : kTriThreshold);
+                                                : (sched == RT_SCHED_COOP_INCOHERENT ? kRefillThresholdCoopIncoherent : kRefillThresholdDirect);
+    // the per-lane kernel tests triangles in the node step and does not read tri_threshold
+    p.tri_threshold = !coop ? 0
+                      : o.tri_threshold > 0 ? clampi(o.tri_threshold, 1, kPairCap - 32)
+                                            : (sched == RT_SCHED_COOP_INCOHERENT ? kPairThresholdIncoherent : kPairThresholdCoherent);
     RT_REQUIRE(dev.device >= 0 && dev.device < kMaxDevices, RT_ERR_CUDA, "%s: device index %d not supported", fn, dev.device);
     int& per_sm = g_per_sm[dev.device][sched - 1][STATS ? 1 : 0][MODE];
     if (per_sm == 0) {
@@ -669,11 +482,7 @@ static int launch(const char* fn, TraceParams& p, const void* blob, const rt_ray
     const int64_t need = (count + rays_per_cta - 1) / rays_per_cta;
     if (grid > need) grid = need;
     switch (sched) {
-        case RT_SCHED_DIRECT: k_trace<MODE, STATS, false><<<(unsigned)grid, kTraceThreads, 0, stream>>>(p); break;
-        case RT_SCHED_QUEUED: k_trace<MODE, STATS, true><<<(unsigned)grid, kTraceThreads, 0, stream>>>(p); break;
-        case RT_SCHED_SLOTS:
-            if constexpr (kHasSlots<MODE>) k_trace_slots<MODE, STATS><<<(unsigned)grid, kTraceThreads, 0, stream>>>(p);
-            break;
+        case RT_SCHED_DIRECT: k_trace<MODE, STATS><<<(unsigned)grid, kTraceThreads, 0, stream>>>(p); break;
         default:
             // Work sharing between the lanes of a draining warp (rt_trace_coop.cuh, step 1b) is compiled into every
             // cooperative kernel; coherent closest hit exists a second time without it, for big launches: there the

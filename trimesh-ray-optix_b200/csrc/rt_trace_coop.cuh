@@ -27,7 +27,7 @@
 //
 // ncu of k_trace on config 2 (profiles/r1_ncu_regions_config2_v4.txt): the in-step triangle test was
 // 27.8 % of all warp instructions at 8.17 of 32 active lanes.  Results are bit-identical to k_trace
-// (tests/test_gpu_parity.py::test_all_schedules_give_identical_results).
+// (tests/test_gpu_round2.py::test_all_schedules_give_identical_results).
 #pragma once
 
 namespace rt {
@@ -40,25 +40,12 @@ constexpr int kPairCap = RT_PAIR_CAP;  // pairs a warp can list before it must t
 #define RT_TAIL_LANES 4
 #endif
 constexpr int kTailLanes = RT_TAIL_LANES;          // <= this many lanes with node work: test listed pairs every step
-#ifndef RT_FRONT_IN_KEY
-#define RT_FRONT_IN_KEY 1
-#endif
-#ifndef RT_R_SMEM_CLOSEST
-#define RT_R_SMEM_CLOSEST 0
-#endif
-#ifndef RT_ROOT_AT_FILL
-#define RT_ROOT_AT_FILL 1
-#endif
-#ifndef RT_FILL_INLINE
-#define RT_FILL_INLINE __forceinline__
-#endif
 // Pool fill with the root-frame test (see the call site).  The ORDER inside matters for the whole kernel: with the full
 // ray set-up before the frame test (or with the whole root node tested here) the register peak of this code made ptxas
 // keep traversal state in local memory around every node step (soup -9...-16 %); a __noinline__ call still left one such
-// spill.  Testing on (origin, 1/d) first and setting up only the survivors needs no spill at all (RT_FILL_INLINE is kept
-// for A/B builds).
+// spill.  Testing on (origin, 1/d) first and setting up only the survivors needs no spill at all.
 template <int MODE>
-__device__ RT_FILL_INLINE unsigned fill_pool_frame(const TraceParams& p, int64_t base, int n, float (*s_pool)[kTraceThreads],
+__device__ __forceinline__ unsigned fill_pool_frame(const TraceParams& p, int64_t base, int n, float (*s_pool)[kTraceThreads],
                                                    const RootFrame& s_root, int col0, int lane) {
     // the frame test needs the origin and 1/d only: it runs before the (register-hungry) rest of the set-up
     bool live = false;
@@ -99,9 +86,6 @@ __device__ RT_FILL_INLINE unsigned fill_pool_frame(const TraceParams& p, int64_t
     return alive;
 }
 
-#ifndef RT_SHARE_TAIL
-#define RT_SHARE_TAIL 1
-#endif
 constexpr uint32_t kContainsAnyBit = 0x80000000u;   // contains: s_cnt bit 31 = "this walk only has to find one hit"
 constexpr int kRayWords = 7;           // resident part of a ray in shared memory: S(3), permuted origin(3), kzf
 
@@ -111,22 +95,21 @@ template <int MODE, bool STATS, bool POOL, bool SHARE>
 __global__ void __launch_bounds__(kTraceThreads, (MODE == kClosest && POOL) ? RT_TRACE_MIN_BLOCKS : RT_TRACE_MIN_BLOCKS_LIGHT)
 k_trace_coop(const __grid_constant__ TraceParams p) {
     constexpr bool kKey = MODE == kClosest || MODE == kFirst;
-    constexpr bool kShare = SHARE && RT_SHARE_TAIL;
     __shared__ float s_ray[kRayWords][kTraceThreads];
     // Shared memory is L1 taken away (one 256 KB array per SM, carve-out steps 100 / 132 / 164 KB): the arrays below are
     // sized so that 7 resident CTAs of the pooled closest-hit kernel stay under 132 KB and 8 CTAs of the others under
     // 100 / 132 KB (1 KB per CTA is reserved by the system).
     __shared__ unsigned long long s_best[kKey ? kTraceThreads : 1];      // (t bits << 32) | prim  (closest: prim << 1 | front)
     __shared__ uint32_t s_cnt[kKey ? 1 : kTraceThreads];                 // count / any flag
-    __shared__ float s_attr[MODE == kClosest ? (RT_FRONT_IN_KEY ? 5 : 6) : 1][kTraceThreads];    // loc(3), uv(2) [, front]
+    __shared__ float s_attr[MODE == kClosest ? 5 : 1][kTraceThreads];    // loc(3), uv(2)
     // ray index of the column's ray (all hits: where the owner's records go).  The pooled 64-register kernels keep the
     // lane's ray index here instead of in two registers: their loop sits at the register edge, and a value spilled around
     // every node step costs the L1TEX-bound soup 10 %; it is touched when a ray starts and retires only.  (The pooled
     // closest-hit kernel has 72 registers and keeps it there: measured equal or better.)
-    constexpr bool kRInSmem = POOL && (RT_R_SMEM_CLOSEST || MODE != kClosest);
+    constexpr bool kRInSmem = POOL && MODE != kClosest;
     __shared__ long long s_rayidx[(MODE == kAllHits || kRInSmem) ? kTraceThreads : 1];
     __shared__ uint2 s_pair[kTraceThreads / 32][kPairCap];               // (triangle record, owner lane)
-    constexpr bool kRootFirst = POOL && MODE != kContains && RT_ROOT_AT_FILL;
+    constexpr bool kRootFirst = POOL && MODE != kContains;     // contains fills its pool without the frame test
     __shared__ float s_pool[POOL ? kPoolWords : 1][POOL ? kTraceThreads : 1];
     __shared__ RootFrame s_root;
     __shared__ long long s_pool_base[POOL ? kTraceThreads / 32 : 1];     // ray index of the pool's first ray, per warp (not a register: the loop is at the 64-register edge)
@@ -161,7 +144,7 @@ k_trace_coop(const __grid_constant__ TraceParams p) {
     int my_pend = 0;                  // != 0: some of them belong to this lane's ray
     int pool_head = 0, pool_count = 0;
     uint32_t ty = 0u, tx = 0u, tmask = 0u;      // triangles of this lane's last node step not yet listed
-    // column of the ray this lane walks for: its own, or (work sharing, RT_SHARE_TAIL) a neighbour's - a helper keeps
+    // column of the ray this lane walks for: its own, or (work sharing, SHARE) a neighbour's - a helper keeps
     // ~column in r, which it does not need (no extra register in the loop)
     auto owner_col = [&]() -> int { const int64_t r = ray_index(); return r < 0 ? (int)(~r) : mycol; };
     trav_init(tv);
@@ -196,7 +179,7 @@ k_trace_coop(const __grid_constant__ TraceParams p) {
                         // equal t resolves to the smaller primitive index; closest hit carries the front flag in bit 0
                         // (one word of shared memory per ray less), primitive indices are < 2^31 (int32 outputs)
                         uint32_t low = (uint32_t)a.w;
-                        if constexpr (MODE == kClosest && RT_FRONT_IN_KEY) low = (low << 1) | (tri_front(t, h) ? 1u : 0u);
+                        if constexpr (MODE == kClosest) low = (low << 1) | (tri_front(t, h) ? 1u : 0u);
                         key = ((unsigned long long)__float_as_uint(h.t) << 32) | (unsigned long long)low;
                         if (key < s_best[col]) { atomicMin(&s_best[col], key); won = true; }
                     } else if constexpr (MODE == kAny) {
@@ -223,7 +206,6 @@ k_trace_coop(const __grid_constant__ TraceParams p) {
                     const HitAttr at = tri_attr(h, v0x, v0y, v0z, v1x, v1y, v1z, v2x, v2y, v2z);
                     s_attr[0][col] = at.lx; s_attr[1][col] = at.ly; s_attr[2][col] = at.lz;
                     s_attr[3][col] = at.uv0; s_attr[4][col] = at.uv1;
-                    if constexpr (!RT_FRONT_IN_KEY) s_attr[5][col] = tri_front(t, h) ? 1.0f : 0.0f;
                 }
             }
         }
@@ -297,13 +279,8 @@ k_trace_coop(const __grid_constant__ TraceParams p) {
                     } else if (p.hit) {
                         // miss: reference miss program shaders.cu:128-135
                         p.hit[r] = hit ? 1 : 0;
-                        if constexpr (RT_FRONT_IN_KEY) {
-                            p.front[r] = hit ? (uint8_t)((uint32_t)best & 1u) : 0;
-                            p.tri[r] = hit ? (int32_t)((uint32_t)best >> 1) : -1;
-                        } else {
-                            p.front[r] = hit ? (s_attr[RT_FRONT_IN_KEY ? 0 : 5][mycol] != 0.0f ? 1 : 0) : 0;
-                            p.tri[r] = hit ? (int32_t)(uint32_t)best : -1;
-                        }
+                        p.front[r] = hit ? (uint8_t)((uint32_t)best & 1u) : 0;
+                        p.tri[r] = hit ? (int32_t)((uint32_t)best >> 1) : -1;
                         p.loc[3 * r] = hit ? s_attr[0][mycol] : 0.f; p.loc[3 * r + 1] = hit ? s_attr[1][mycol] : 0.f;
                         p.loc[3 * r + 2] = hit ? s_attr[2][mycol] : 0.f;
                         p.uv[2 * r] = hit ? s_attr[3][mycol] : 0.f; p.uv[2 * r + 1] = hit ? s_attr[4][mycol] : 0.f;
@@ -473,7 +450,7 @@ k_trace_coop(const __grid_constant__ TraceParams p) {
                 }
             }
             if (!__any_sync(0xffffffffu, active)) return (exhausted && pool_count == 0) ? 1 : 0;   // 0: every lane drew a masked-out point, draw again
-            if constexpr (!DRAIN && kShare) { if (exhausted && pool_count == 0 && p.share_lanes) return 2; }
+            if constexpr (!DRAIN && SHARE) { if (exhausted && pool_count == 0 && p.share_lanes) return 2; }
         }
 
         // ---- 1b. work sharing once this warp can draw no more rays: a lane without a ray takes the top stack entry (the
@@ -565,7 +542,7 @@ k_trace_coop(const __grid_constant__ TraceParams p) {
     };
     int rc;
     do { rc = step(std::false_type{}); } while (rc == 0);
-    if constexpr (kShare) {
+    if constexpr (SHARE) {
         if (rc == 2) {
             while (step(std::true_type{}) == 0) {}
         }

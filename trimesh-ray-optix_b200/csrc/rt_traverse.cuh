@@ -81,84 +81,6 @@ RT_HD bool trav_step(const uint8_t* __restrict__ nodes, const uint8_t* __restric
     return false;
 }
 
-// Node half of trav_step for kernels that postpone triangle tests: advances one wide node and
-// hands the record index of every triangle in a hit leaf slot to queue.push(); returns true when
-// the ray has no node work left (its queued triangles may still be pending).
-template <class Visitor, class StackT, class QueueT>
-RT_HD bool node_step(const uint8_t* __restrict__ nodes, const Ray& r, Visitor& vis, StackT& stack, Trav& t,
-                     QueueT& queue) {
-    if (t.gy & 0xff000000u) {
-        const uint32_t hits = t.gy;
-        const int bit = 31 - clz32(hits);
-        t.gy &= ~(1u << bit);
-        if (t.gy & 0xff000000u) { stack.push(t.sp, t.gx, t.gy); ++t.sp; }
-        const uint32_t slot = (uint32_t)(bit - 24) ^ r.octinv;
-        const uint32_t rel = (uint32_t)popc32(hits & ~(0xffffffffu << slot));
-        const uint8_t* np = nodes + (size_t)(t.gx + rel) * 80u;
-        const U4 n0 = ldg128(np), n1 = ldg128(np + 16), n2 = ldg128(np + 32), n3 = ldg128(np + 48),
-                 n4 = ldg128(np + 64);
-        vis.count_node();
-        const uint32_t hm = node_test(r, n0, n1, n2, n3, n4, 0.0f, vis.tmax);
-        t.gx = n1.x;
-        t.gy = (hm & 0xff000000u) | (n0.w >> 24);
-        uint32_t ty = hm & 0x00ffffffu;
-        const uint32_t tx = n1.y, tmask = n1.z;
-        while (ty) {
-            const int b = ffs32(ty) - 1;
-            ty &= ty - 1u;
-            queue.push(tx + (uint32_t)popc32(tmask & ~(0xffffffffu << b)));
-        }
-    }
-    if (!(t.gy & 0xff000000u)) {
-        if (t.sp == 0) return true;
-        --t.sp;
-        stack.pop(t.sp, t.gx, t.gy);
-    }
-    return false;
-}
-
-// Node half for kernels that keep the hit leaf slots of a step as a bit mask: ty = triangle bits of the hit leaf slots
-// (positions of trimask), tx = tri_base, tmask = trimask; triangle record of bit b = tx + popc(tmask & below(b)).
-template <class Visitor, class StackT>
-RT_HD bool node_step_bits(const uint8_t* __restrict__ nodes, const Ray& r, Visitor& vis, StackT& stack, Trav& t,
-                          uint32_t& ty, uint32_t& tx, uint32_t& tmask) {
-    if (t.gy & 0xff000000u) {
-        const uint32_t hits = t.gy;
-        const int bit = 31 - clz32(hits);
-        t.gy &= ~(1u << bit);
-        if (t.gy & 0xff000000u) { stack.push(t.sp, t.gx, t.gy); ++t.sp; }
-        const uint32_t slot = (uint32_t)(bit - 24) ^ r.octinv;
-        const uint32_t rel = (uint32_t)popc32(hits & ~(0xffffffffu << slot));
-        const uint8_t* np = nodes + (size_t)(t.gx + rel) * 80u;
-        const U4 n0 = ldg128(np), n1 = ldg128(np + 16), n2 = ldg128(np + 32), n3 = ldg128(np + 48),
-                 n4 = ldg128(np + 64);
-        vis.count_node();
-        const uint32_t hm = node_test(r, n0, n1, n2, n3, n4, 0.0f, vis.tmax);
-        t.gx = n1.x;
-        t.gy = (hm & 0xff000000u) | (n0.w >> 24);
-        ty = hm & 0x00ffffffu; tx = n1.y; tmask = n1.z;
-    }
-    if (!(t.gy & 0xff000000u)) {
-        if (t.sp == 0) return true;
-        --t.sp;
-        stack.pop(t.sp, t.gx, t.gy);
-    }
-    return false;
-}
-
-// Triangle half: one queued triangle record against the ray; returns true = terminate the ray.
-template <class Visitor>
-RT_HD bool tri_one(const uint8_t* __restrict__ tris, const Ray& r, Visitor& vis, uint32_t slot_t) {
-    const uint8_t* tp = tris + (size_t)slot_t * 48u;
-    const U4 a = ldg128(tp), bb = ldg128(tp + 16), c = ldg128(tp + 32);
-    vis.count_tri();
-    TriHit h;
-    if (tri_test(r, as_float(a.x), as_float(a.y), as_float(a.z), as_float(bb.x), as_float(bb.y), as_float(bb.z),
-                 as_float(c.x), as_float(c.y), as_float(c.z), h))
-        return vis.hit(r, h, (int32_t)a.w, slot_t);
-    return false;
-}
-
 template <class Visitor, class StackT>
 RT_HD void traverse(const uint8_t* __restrict__ nodes, const uint8_t* __restrict__ tris, const Ray& r,
                     Visitor& vis, StackT& stack) {

@@ -54,7 +54,8 @@ class TraceOpts(C.Structure):
                 ("grid_div", C.c_int32), ("reserved", C.c_int32 * 4)]
 
 
-SCHED_AUTO, SCHED_DIRECT, SCHED_QUEUED, SCHED_COOP_COHERENT, SCHED_COOP_INCOHERENT, SCHED_SLOTS = 0, 1, 2, 3, 4, 5
+SCHED_AUTO, SCHED_DIRECT, SCHED_COOP_COHERENT, SCHED_COOP_INCOHERENT = 0, 1, 3, 4
+SCHED_QUEUED, SCHED_SLOTS = 2, 5     # removed schedules: the library runs SCHED_COOP_INCOHERENT for them (ABI v2 aliases)
 OPT_SCRATCH_ZEROED = 1
 OPT_STOP_WHEN_BROKEN = 2
 OPT_NO_LANE_SHARING = 4
