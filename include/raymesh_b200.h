@@ -278,6 +278,33 @@ int rt_closest_point(const void* blob, const rt_ray_desc* points, const rt_trace
                      float* closest, float* distance, int32_t* tri_idx, float* uv, uint64_t* counters_dev,
                      void* scratch, void* stream);
 
+/* ---- Generalized winding number (Jacobson, Kavan, Sorkine-Hornung 2013; libigl's fast_winding_number, Barill et al.
+ *      2018; no counterpart in the reference): w(q) = sum over triangles of the signed solid angle / 4 pi, orientation
+ *      from the face order.  ~1 inside and ~0 outside a closed outward-facing mesh; meaningful for open meshes, soups
+ *      and self-intersecting meshes too (nested shells add up, open surfaces give fractions).
+ *
+ *      rt_winding_moments fills the per-node moment array (64 bytes per node: area-weighted centroid, radius bound,
+ *      sum of area vectors, first-moment tensor) bottom-up from any valid blob: built, re-fitted, broadcast or loaded.
+ *      It is a side array, not part of the blob: recompute it after rt_bvh_refit.  Sizes: rt_winding_moments_sizes
+ *      bounds them from the triangle count (for any leaf size); a caller that knows the blob's node count (header
+ *      n_nodes) may pass exactly n_nodes * 64 moment bytes and a workspace of two 256-byte aligned arrays of
+ *      n_nodes * 4 bytes.  Moments 16-byte and workspace 256-byte aligned.  A blob with more nodes than the buffers
+ *      can hold is left without moments (nothing is written).
+ *
+ *      rt_winding_number: winding[i] for every point of the batch/window (`points` through the origins fields of
+ *      rt_ray_desc, opts for ray_first / ray_count only).  Triangles in leaf slots are summed exactly; an inner child
+ *      whose moment ball is far (|p~ - q| > beta * radius) adds its two-term far-field expansion instead of being
+ *      visited.  beta >= 1 (libigl's default is 2); beta = +inf sums every triangle exactly; beta < 1 or NaN ->
+ *      RT_ERR_INVALID.  A triangle with a non-finite vertex or a zero computed determinant contributes 0; a
+ *      non-finite point gives NaN; an empty mesh gives +0.  The result is a function of (blob, moments, point, beta)
+ *      only.  counters_dev (instrumented kernel when not NULL): [0] BVH8 nodes visited, [1] triangles summed exactly,
+ *      [2] points, [3] far-field terms.  `scratch` is accepted like every trace call's and left untouched. */
+int rt_winding_moments_sizes(int64_t n_faces, size_t* moments_bytes, size_t* workspace_bytes);
+int rt_winding_moments(const void* blob, void* moments, size_t moments_bytes, void* workspace, size_t workspace_bytes,
+                       void* stream);
+int rt_winding_number(const void* blob, const void* moments, const rt_ray_desc* points, const rt_trace_opts* opts,
+                      float beta, float* winding, uint64_t* counters_dev, void* scratch, void* stream);
+
 /* ---- Host-buffer entry points (end-to-end path): rays and results live in (pinned) HOST memory.
  *      Copies ray chunks H2D, traces and copies results D2H on internal streams, overlapping
  *      the three; `dev_work` is caller-provided device memory of rt_host_closest_sizes() bytes.

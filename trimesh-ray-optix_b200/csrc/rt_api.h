@@ -34,6 +34,27 @@ int device_info(DeviceInfo* out);
 
 inline size_t align_up_sz(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
+// blocks for a grid-stride loop over n items: enough to cover them, at most per_sm blocks per SM
+inline int grid_for(int64_t n, int threads, int sm_count, int per_sm) {
+    int64_t b = (n + threads - 1) / threads;
+    const int64_t cap = (int64_t)sm_count * per_sm;
+    if (b > cap) b = cap;
+    if (b < 1) b = 1;
+    return (int)b;
+}
+
+// a point batch (rt_ray_desc origins) that is row-major contiguous [s0, s1, s2, 3]; dimensions of extent 1 may carry
+// any stride
+inline bool points_packed(const int64_t shape[4], const int64_t stride[4]) {
+    if (stride[3] != 1) return false;
+    int64_t expect = 3;
+    for (int i = 2; i >= 0; --i) {
+        if (shape[i] != 1 && stride[i] != expect) return false;
+        expect *= shape[i];
+    }
+    return true;
+}
+
 // Triangles per leaf slot used by the builder: kLeafTrisDefault, or TRIRO_LEAF_TRIS=1..3 (read once per process;
 // sizes, build and refit of one process always agree).
 inline int leaf_tris_setting() {

@@ -354,14 +354,6 @@ __global__ void k_finalize(rt_blob_header* hdr, const BuildState* st, int64_t n,
     }
 }
 
-static int grid_for(int64_t n, int threads, int sm_count, int per_sm) {
-    int64_t b = (n + threads - 1) / threads;
-    const int64_t cap = (int64_t)sm_count * per_sm;
-    if (b > cap) b = cap;
-    if (b < 1) b = 1;
-    return (int)b;
-}
-
 }  // namespace rt
 
 using namespace rt;

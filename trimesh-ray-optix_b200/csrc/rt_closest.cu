@@ -91,17 +91,6 @@ __global__ void __launch_bounds__(kPointThreads) k_closest_point(const __grid_co
     }
 }
 
-static bool points_packed(const int64_t shape[4], const int64_t stride[4]) {
-    // row-major contiguous [s0, s1, s2, 3]; dimensions of extent 1 may carry any stride
-    if (stride[3] != 1) return false;
-    int64_t expect = 3;
-    for (int i = 2; i >= 0; --i) {
-        if (shape[i] != 1 && stride[i] != expect) return false;
-        expect *= shape[i];
-    }
-    return true;
-}
-
 }  // namespace rt
 
 using namespace rt;

@@ -101,6 +101,9 @@ def _declare(lib):
         "rt_contains_parity": (ci, [vp, prd, pto, pf, pf, pf, vp, vp, vp, vp, vp, vp]),
         "rt_trace_stats": (ci, [vp, prd, pto, ci, vp, vp, vp]),
         "rt_closest_point": (ci, [vp, prd, pto, C.c_float, vp, vp, vp, vp, vp, vp, vp]),
+        "rt_winding_moments_sizes": (ci, [i64, psz, psz]),
+        "rt_winding_moments": (ci, [vp, vp, sz, vp, sz, vp]),
+        "rt_winding_number": (ci, [vp, vp, prd, pto, C.c_float, vp, vp, vp, vp]),
         "rt_host_closest_sizes": (ci, [i64, psz]),
         "rt_host_trace_closest": (ci, [vp, i64, vp, ci, vp, pto, vp, vp, vp, vp, vp, vp, sz]),
         "rt_host_trace_closest_compact": (ci, [vp, i64, vp, ci, vp, pto, vp, vp, vp, vp, vp, vp, C.POINTER(C.c_int64), vp, sz]),
@@ -336,6 +339,7 @@ class AccelStructure:
         self.blob: torch.Tensor | None = None
         self.header: dict | None = None
         self.build_ms: float | None = None
+        self.winding_moments: torch.Tensor | None = None   # ops.winding_moments() cache, dropped with the blob's contents
 
     def build(self, vertices: torch.Tensor, faces: torch.Tensor, timing: bool = False):
         lib = get_module()
@@ -375,6 +379,7 @@ class AccelStructure:
         validate_header(hdr, blob.numel())
         self.blob = blob
         self.header = hdr
+        self.winding_moments = None
         return self
 
     def refit(self, vertices: torch.Tensor, faces: torch.Tensor):
@@ -400,6 +405,7 @@ class AccelStructure:
             _check(lib.rt_bvh_refit(_ptr(vertices), vertices.shape[0], _ptr(faces), faces.shape[0], _ptr(ws), ws.numel(),
                                     _ptr(self.blob), self.blob.numel(), _stream(dev)), "rt_bvh_refit")
             self.header = parse_header(self.blob[:BLOB_HEADER_BYTES].cpu().numpy().tobytes())
+        self.winding_moments = None
         return self
 
     def save(self, path: str):
@@ -426,6 +432,7 @@ class AccelStructure:
         validate_header(hdr, blob.numel())
         self.blob = blob
         self.header = hdr
+        self.winding_moments = None
         return self
 
     def used(self) -> torch.Tensor:
@@ -435,6 +442,7 @@ class AccelStructure:
     def free(self):
         self.blob = None
         self.header = None
+        self.winding_moments = None
 
 
 def parse_header(raw: bytes) -> dict:
@@ -813,6 +821,64 @@ def closest_point(accel_structure, points: torch.Tensor, max_distance: float = f
                                              md, _ptr(closest), _ptr(distance), _ptr(tri), _ptr(uv), _ptr(counters),
                                              _ptr(_scratch(dev, st)), st), "rt_closest_point")
     return closest, distance, tri, uv
+
+
+def winding_moments(accel_structure) -> torch.Tensor:
+    """Float32[nodes, 16]: the per-node moments rt_winding_number reads (area-weighted centroid, radius bound, sum of
+    area vectors, first-moment tensor), one row per node of the blob.  Computed on first use and cached on
+    the AccelStructure until its blob changes (build, refit, adopt / load)."""
+    inner = getattr(accel_structure, "_inner", accel_structure)
+    blob = _blob_of(inner)
+    if inner.winding_moments is not None:
+        return inner.winding_moments
+    lib = get_module()
+    # rt_winding_moments_sizes bounds the node count from the triangle count alone (for any leaf size, ~2.7x the
+    # default build's); the header already gives the exact count, and the kernel checks it against the buffers.
+    # Workspace: two 256-byte aligned arrays of one u32 / f32 per node.
+    nn = max(int(inner.header["n_nodes"]), 1)
+    mb, wb = nn * 64, 2 * (-(-nn * 4 // 256) * 256)
+    dev = blob.device
+    with _on_device(dev):
+        moments = torch.empty((nn, 16), dtype=torch.float32, device=dev)
+        ws = torch.empty(wb, dtype=torch.uint8, device=dev)
+        _check(lib.rt_winding_moments(_ptr(blob), _ptr(moments), mb, _ptr(ws), wb, _stream(dev)), "rt_winding_moments")
+    inner.winding_moments = moments
+    return inner.winding_moments
+
+
+def winding_number(accel_structure, points: torch.Tensor, beta: float = 2.0, ray_first: int = 0, ray_count: int = -1,
+                   counters: torch.Tensor | None = None) -> torch.Tensor:
+    """Float32[*b]: generalized winding number of every query point (sum of the triangles' signed solid angles / 4 pi,
+    orientation from the face order): ~1 inside and ~0 outside a closed outward-facing mesh, fractional near holes,
+    additive over nested shells.  Leaf triangles are summed exactly; a BVH subtree farther than `beta` times its radius
+    adds its far-field expansion (Barill et al. 2018).  beta >= 1; beta = inf is exact.  A non-finite point gives NaN,
+    an empty mesh 0.  With a window [ray_first, ray_first + ray_count) of the flattened batch the output is 1-D over the
+    window.  `counters` (Int64[4] on the device, optional) selects the instrumented kernel: nodes visited, triangles
+    summed exactly, points, far-field terms."""
+    tensor_input_check(points)
+    b = float(beta)
+    if not (b >= 1.0):
+        raise ValueError(f"beta must be >= 1 or inf (got {beta})")
+    blob = _blob_of(accel_structure, points.device)
+    rd, batch = make_ray_desc(points, None)
+    if ray_first != 0 or ray_count >= 0:
+        batch = (_window(rd.nray, ray_first, ray_count),)
+    dev = points.device
+    if counters is not None and (counters.dtype != torch.int64 or counters.device != dev or counters.numel() != 4
+                                 or not counters.is_contiguous()):
+        raise ValueError("counters must be a contiguous int64 tensor of 4 elements on the points' device")
+    with _on_device(dev):
+        w = torch.empty(batch, dtype=torch.float32, device=dev)
+        if w.numel() == 0:
+            if counters is not None:
+                counters.zero_()
+            return w
+        moments = winding_moments(accel_structure)
+        st = _stream(dev)
+        _check(get_module().rt_winding_number(_ptr(blob), _ptr(moments), C.byref(rd),
+                                              C.byref(trace_opts(accel_structure, ray_first, ray_count)), b, _ptr(w),
+                                              _ptr(counters), _ptr(_scratch(dev, st)), st), "rt_winding_number")
+    return w
 
 
 def host_closest(accel_structure, origins_host: torch.Tensor, dirs_host: torch.Tensor, out: dict | None = None,

@@ -70,6 +70,10 @@ class RayMeshIntersector:
         c, d, t = self._rmi.closest_point(self._points(points))
         return c.cpu().numpy().astype(np.float64), d.cpu().numpy().astype(np.float64), t.cpu().numpy().astype(np.int64)
 
-    def signed_distance(self, points):
-        """trimesh.proximity.signed_distance -> (n,) float64, positive inside the mesh"""
-        return self._rmi.signed_distance(self._points(points)).cpu().numpy().astype(np.float64)
+    def signed_distance(self, points, sign="contains"):
+        """trimesh.proximity.signed_distance -> (n,) float64, positive inside the mesh (sign: see the torch class)"""
+        return self._rmi.signed_distance(self._points(points), sign=sign).cpu().numpy().astype(np.float64)
+
+    def winding_number(self, points, beta=2.0):
+        """generalized winding number -> (n,) float64"""
+        return self._rmi.winding_number(self._points(points), beta).cpu().numpy().astype(np.float64)

@@ -152,12 +152,28 @@ class RayMeshIntersector:
             return closest, distance, tri, uv
         return closest, distance, tri
 
-    def signed_distance(self, points: torch.Tensor) -> torch.Tensor:
+    def signed_distance(self, points: torch.Tensor, sign: str = "contains") -> torch.Tensor:
         """Float32[*b] — distance to the surface, positive inside and negative outside (trimesh.proximity.signed_distance).
-        The sign is `contains_points` (with its documented decision procedure); an exact 0 is returned as +0.0."""
+        sign="contains": the sign is `contains_points` (with its documented decision procedure), meaningful for closed
+        meshes that do not intersect themselves.  sign="winding": inside where the generalized winding number
+        (`winding_number`, beta 2) exceeds 0.5, the robust choice for open, overlapping or soup meshes.  An exact 0 is
+        returned as +0.0 either way."""
+        if sign not in ("contains", "winding"):
+            raise ValueError(f"sign must be 'contains' or 'winding' (got {sign!r})")
         _, d, _ = self.closest_point(points)
-        inside = self.contains_points(points.reshape(-1, 3)).reshape(d.shape)
+        if sign == "winding":
+            inside = self.winding_number(points) > 0.5
+        else:
+            inside = self.contains_points(points.reshape(-1, 3)).reshape(d.shape)
         return torch.where(inside | (d == 0), d, -d)
+
+    def winding_number(self, points: torch.Tensor, beta: float = 2.0) -> torch.Tensor:
+        """Float32[*b] — generalized winding number of every point (Jacobson et al. 2013): the sum of the triangles'
+        signed solid angles over 4 pi, orientation from the face order.  ~1 inside and ~0 outside a closed
+        outward-facing mesh; nested shells add up and holes give fractions, so it answers "inside?" for scans, soups
+        and self-intersecting meshes too.  Distant BVH subtrees use the far-field expansion of Barill et al. 2018
+        (libigl's fast_winding_number) when they are farther than `beta` times their radius; beta = inf is exact."""
+        return hops.winding_number(self.as_wrapper, points, beta)
 
     DEFAULT_CHECK_DIRECTION = (0.4395064455, 0.617598629942, 0.652231566745)   # reference :245-247
 
