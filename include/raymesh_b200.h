@@ -305,6 +305,33 @@ int rt_winding_moments(const void* blob, void* moments, size_t moments_bytes, vo
 int rt_winding_number(const void* blob, const void* moments, const rt_ray_desc* points, const rt_trace_opts* opts,
                       float beta, float* winding, uint64_t* counters_dev, void* scratch, void* stream);
 
+/* ---- Pseudo-normal signed distance (Baerentzen & Aanaes 2005, "Signed distance computation using the angle weighted
+ *      pseudonormal"; no counterpart in the reference): the sign of the closest point's feature normal, exact for a
+ *      closed, manifold, consistently oriented mesh, with one closest-point walk per point.
+ *
+ *      rt_pseudonormals fills the side array of 96 bytes per triangle record (6 x f32x4: the angle-weighted normals of
+ *      vertices a, b, c and the normals of edges ab, ac, bc) from any valid blob: built, re-fitted, broadcast or loaded.
+ *      Corners are welded by exact equality of their coordinates (-0 = +0), not by the face indices, so an unwelded
+ *      soup of a closed surface gets the normals of the welded mesh; a triangle with a non-finite vertex takes part in
+ *      nothing.  It is a side array, not part of the blob: recompute it after rt_bvh_refit.  normals_bytes / 96 is the
+ *      capacity in triangles (at most 2^30 / 3, else RT_ERR_INVALID); a blob with more triangles than that is left
+ *      without normals.  Normals 16-byte and workspace 256-byte aligned; rt_pseudonormals_sizes gives both sizes for
+ *      n_faces triangles.  edge_counts_dev (u64[3], zeroed by the call): [0] boundary edges (one face), [1]
+ *      non-manifold edges (more than two faces), [2] inconsistent edges (two faces that traverse it the same way), on
+ *      the welded surface.  The sign below is an inside/outside answer when all three are 0.
+ *
+ *      rt_signed_distance: signed_distance[i] for every point of the batch/window (`points` through the origins fields
+ *      of rt_ray_desc, opts for ray_first / ray_count only).  |signed_distance| is bit for bit the distance of
+ *      rt_closest_point (max_distance = +inf) and the closest triangle is the one it picks; the value is +d when
+ *      (p - c) . n < 0 for the pseudo-normal n of the Voronoi region of c (face, edge or vertex), else -d; an exact
+ *      d = 0 gives +0; a non-finite point or an empty mesh gives -inf.  A function of (blob, normals, point) only.
+ *      counters_dev: NULL or u64[4] as for rt_closest_point.  `scratch` is accepted and left untouched. */
+int rt_pseudonormals_sizes(int64_t n_faces, size_t* normals_bytes, size_t* workspace_bytes);
+int rt_pseudonormals(const void* blob, void* normals, size_t normals_bytes, void* workspace, size_t workspace_bytes,
+                     uint64_t* edge_counts_dev, void* stream);
+int rt_signed_distance(const void* blob, const void* normals, const rt_ray_desc* points, const rt_trace_opts* opts,
+                       float* signed_distance, uint64_t* counters_dev, void* scratch, void* stream);
+
 /* ---- Host-buffer entry points (end-to-end path): rays and results live in (pinned) HOST memory.
  *      Copies ray chunks H2D, traces and copies results D2H on internal streams, overlapping
  *      the three; `dev_work` is caller-provided device memory of rt_host_closest_sizes() bytes.

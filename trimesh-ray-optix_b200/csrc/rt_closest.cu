@@ -1,5 +1,6 @@
 // rt_closest.cu — closest point on the mesh for a batch of query points (rt_closest_point), the counterpart of
-// trimesh.proximity.closest_point on the BVH8 blob the ray queries use.
+// trimesh.proximity.closest_point on the BVH8 blob the ray queries use, and the pseudo-normal signed distance
+// (rt_signed_distance) that ends the same walk with one read of the rt_pseudonormals side array.
 //
 // One thread per point: stack-based traversal of the BVH8 (point_step, rt_point.cuh), children nearest first by
 // their lower bound, subtrees dropped when their bound exceeds the best squared distance found so far.  The answer is
@@ -7,7 +8,7 @@
 // geometry: the host simulator under tests/pointquery/ and a brute-force loop give the same bits.
 #include <type_traits>
 #include "rt_api.h"
-#include "rt_point.cuh"
+#include "rt_pseudonormal.cuh"
 
 namespace rt {
 
@@ -25,6 +26,8 @@ struct PointParams {
     int32_t* tri;
     float* uv;
     unsigned long long* counters;
+    const uint8_t* normals;      // rt_signed_distance: the rt_pseudonormals rows
+    float* signed_distance;
 };
 
 struct PointStack {
@@ -42,8 +45,10 @@ __device__ __forceinline__ int64_t point_offset(const PointParams& p, int64_t r)
     return i0 * p.stride[0] + i1 * p.stride[1] + i2 * p.stride[2];
 }
 
-template <bool STATS>
-__global__ void __launch_bounds__(kPointThreads) k_closest_point(const __grid_constant__ PointParams p) {
+// The body of both kernels: SIGNED ends the walk with the pseudo-normal sign (DESIGN.md §4.8) instead of writing the
+// closest point, so |signed distance| is bit for bit the distance rt_closest_point returns.
+template <bool STATS, bool SIGNED>
+__device__ __forceinline__ void point_query(const PointParams& p) {
     using S = typename std::conditional<STATS, Stats, NoStats>::type;
     const rt_blob_header* hdr = reinterpret_cast<const rt_blob_header*>(p.blob);
     const uint8_t* tris = p.blob + hdr->tris_offset;
@@ -64,10 +69,18 @@ __global__ void __launch_bounds__(kPointThreads) k_closest_point(const __grid_co
             const U4 a = ldg128(tp), b = ldg128(tp + 16), c = ldg128(tp + 32);
             const PointHit h = point_tri(t.x, t.y, t.z, as_float(a.x), as_float(a.y), as_float(a.z), as_float(b.x),
                                          as_float(b.y), as_float(b.z), as_float(c.x), as_float(c.y), as_float(c.z));
-            p.closest[3 * i] = h.cx; p.closest[3 * i + 1] = h.cy; p.closest[3 * i + 2] = h.cz;
-            p.distance[i] = fsqrt(t.best);
-            p.tri[i] = t.prim;
-            p.uv[2 * i] = h.w0; p.uv[2 * i + 1] = h.w1;
+            if (SIGNED) {
+                const float v[9] = {as_float(a.x), as_float(a.y), as_float(a.z), as_float(b.x), as_float(b.y),
+                                    as_float(b.z), as_float(c.x), as_float(c.y), as_float(c.z)};
+                p.signed_distance[i] = pseudonormal_sign(p.normals, t.slot, h, t.x, t.y, t.z, v, fsqrt(t.best));
+            } else {
+                p.closest[3 * i] = h.cx; p.closest[3 * i + 1] = h.cy; p.closest[3 * i + 2] = h.cz;
+                p.distance[i] = fsqrt(t.best);
+                p.tri[i] = t.prim;
+                p.uv[2 * i] = h.w0; p.uv[2 * i + 1] = h.w1;
+            }
+        } else if (SIGNED) {
+            p.signed_distance[i] = as_float(0xff800000u);
         } else {
             p.closest[3 * i] = 0.0f; p.closest[3 * i + 1] = 0.0f; p.closest[3 * i + 2] = 0.0f;
             p.distance[i] = as_float(0x7f800000u);
@@ -91,19 +104,26 @@ __global__ void __launch_bounds__(kPointThreads) k_closest_point(const __grid_co
     }
 }
 
+template <bool STATS>
+__global__ void __launch_bounds__(kPointThreads) k_closest_point(const __grid_constant__ PointParams p) {
+    point_query<STATS, false>(p);
+}
+
+template <bool STATS>
+__global__ void __launch_bounds__(kPointThreads) k_signed_distance(const __grid_constant__ PointParams p) {
+    point_query<STATS, true>(p);
+}
+
 }  // namespace rt
 
 using namespace rt;
 
-extern "C" int rt_closest_point(const void* blob, const rt_ray_desc* points, const rt_trace_opts* opts, float max_distance,
-                                float* closest, float* distance, int32_t* tri_idx, float* uv, uint64_t* counters_dev,
-                                void* scratch, void* stream) {
-    (void)scratch;   // one thread per point: no work counter, the scratch is left as it was
-    const char* fn = "rt_closest_point";
+// Checks shared by both entry points and the batch part of the launch parameters; *count = points in the window (0:
+// nothing to launch, the counters are already zeroed).
+static int point_params(const char* fn, const void* blob, const rt_ray_desc* points, const rt_trace_opts* opts,
+                        uint64_t* counters_dev, void* stream, PointParams& p, int64_t* count) {
     RT_REQUIRE(blob != nullptr && ((uintptr_t)blob & 15) == 0, RT_ERR_INVALID, "%s: blob null or not 16-byte aligned", fn);
     RT_REQUIRE(points != nullptr, RT_ERR_INVALID, "%s: null point descriptor", fn);
-    RT_REQUIRE(!(max_distance != max_distance) && max_distance >= 0.0f, RT_ERR_INVALID,
-               "%s: max_distance must be >= 0 or +inf (got %g)", fn, (double)max_distance);
     RT_REQUIRE(points->nray >= 0 && points->shape[3] == 3, RT_ERR_INVALID, "%s: point batch must be [*b, 3]", fn);
     RT_REQUIRE(points->shape[0] >= 0 && points->shape[1] >= 0 && points->shape[2] >= 0 &&
                    points->shape[0] * points->shape[1] * points->shape[2] == points->nray,
@@ -112,30 +132,68 @@ extern "C" int rt_closest_point(const void* blob, const rt_ray_desc* points, con
     const rt_trace_opts& o = opts ? *opts : kDefaults;
     RT_REQUIRE(o.ray_first >= 0 && o.ray_first <= points->nray, RT_ERR_INVALID, "%s: ray_first %lld outside [0, %lld]", fn,
                (long long)o.ray_first, (long long)points->nray);
-    const int64_t count = o.ray_count <= 0 ? points->nray - o.ray_first : o.ray_count;
-    RT_REQUIRE(count <= points->nray - o.ray_first, RT_ERR_INVALID, "%s: window [%lld, +%lld) exceeds the batch of %lld", fn,
-               (long long)o.ray_first, (long long)count, (long long)points->nray);
+    const int64_t n = o.ray_count <= 0 ? points->nray - o.ray_first : o.ray_count;
+    RT_REQUIRE(n <= points->nray - o.ray_first, RT_ERR_INVALID, "%s: window [%lld, +%lld) exceeds the batch of %lld", fn,
+               (long long)o.ray_first, (long long)n, (long long)points->nray);
     if (counters_dev) RT_CUDA_TRY(cudaMemsetAsync(counters_dev, 0, 4 * sizeof(uint64_t), (cudaStream_t)stream));
-    if (count == 0) return RT_OK;
+    *count = n;
+    if (n == 0) return RT_OK;
     RT_REQUIRE(points->origins != nullptr, RT_ERR_INVALID, "%s: null points", fn);
-    RT_REQUIRE(closest && distance && tri_idx && uv, RT_ERR_INVALID, "%s: null output", fn);
-    PointParams p = {};
+    RT_REQUIRE((n + kPointThreads - 1) / kPointThreads < ((int64_t)1 << 31), RT_ERR_INVALID,
+               "%s: batch of %lld points too large for one launch", fn, (long long)n);
+    p = PointParams{};
     p.blob = reinterpret_cast<const uint8_t*>(blob);
     p.origins = points->origins;
     for (int a = 0; a < 4; ++a) { p.shape[a] = points->shape[a]; p.stride[a] = points->o_stride[a]; }
     p.packed = points_packed(points->shape, points->o_stride) ? 1 : 0;
     p.first = o.ray_first;
-    p.n = count;
+    p.n = n;
+    p.counters = reinterpret_cast<unsigned long long*>(counters_dev);
+    return RT_OK;
+}
+
+extern "C" int rt_closest_point(const void* blob, const rt_ray_desc* points, const rt_trace_opts* opts, float max_distance,
+                                float* closest, float* distance, int32_t* tri_idx, float* uv, uint64_t* counters_dev,
+                                void* scratch, void* stream) {
+    (void)scratch;   // one thread per point: no work counter, the scratch is left as it was
+    const char* fn = "rt_closest_point";
+    RT_REQUIRE(!(max_distance != max_distance) && max_distance >= 0.0f, RT_ERR_INVALID,
+               "%s: max_distance must be >= 0 or +inf (got %g)", fn, (double)max_distance);
+    PointParams p;
+    int64_t count = 0;
+    const int rc = point_params(fn, blob, points, opts, counters_dev, stream, p, &count);
+    if (rc != RT_OK || count == 0) return rc;
+    RT_REQUIRE(closest && distance && tri_idx && uv, RT_ERR_INVALID, "%s: null output", fn);
     p.max_distance = max_distance;
     p.closest = closest; p.distance = distance; p.tri = tri_idx; p.uv = uv;
-    p.counters = reinterpret_cast<unsigned long long*>(counters_dev);
-    const int64_t grid = (count + kPointThreads - 1) / kPointThreads;
-    RT_REQUIRE(grid < ((int64_t)1 << 31), RT_ERR_INVALID, "%s: batch of %lld points too large for one launch", fn,
-               (long long)count);
+    const unsigned grid = (unsigned)((count + kPointThreads - 1) / kPointThreads);
     if (counters_dev)
-        k_closest_point<true><<<(unsigned)grid, kPointThreads, 0, (cudaStream_t)stream>>>(p);
+        k_closest_point<true><<<grid, kPointThreads, 0, (cudaStream_t)stream>>>(p);
     else
-        k_closest_point<false><<<(unsigned)grid, kPointThreads, 0, (cudaStream_t)stream>>>(p);
+        k_closest_point<false><<<grid, kPointThreads, 0, (cudaStream_t)stream>>>(p);
+    RT_CUDA_TRY(cudaGetLastError());
+    return RT_OK;
+}
+
+extern "C" int rt_signed_distance(const void* blob, const void* normals, const rt_ray_desc* points, const rt_trace_opts* opts,
+                                  float* signed_distance, uint64_t* counters_dev, void* scratch, void* stream) {
+    (void)scratch;
+    const char* fn = "rt_signed_distance";
+    RT_REQUIRE(normals != nullptr && ((uintptr_t)normals & 15) == 0, RT_ERR_INVALID,
+               "%s: normals null or not 16-byte aligned", fn);
+    PointParams p;
+    int64_t count = 0;
+    const int rc = point_params(fn, blob, points, opts, counters_dev, stream, p, &count);
+    if (rc != RT_OK || count == 0) return rc;
+    RT_REQUIRE(signed_distance != nullptr, RT_ERR_INVALID, "%s: null output", fn);
+    p.max_distance = as_float(0x7f800000u);
+    p.normals = reinterpret_cast<const uint8_t*>(normals);
+    p.signed_distance = signed_distance;
+    const unsigned grid = (unsigned)((count + kPointThreads - 1) / kPointThreads);
+    if (counters_dev)
+        k_signed_distance<true><<<grid, kPointThreads, 0, (cudaStream_t)stream>>>(p);
+    else
+        k_signed_distance<false><<<grid, kPointThreads, 0, (cudaStream_t)stream>>>(p);
     RT_CUDA_TRY(cudaGetLastError());
     return RT_OK;
 }

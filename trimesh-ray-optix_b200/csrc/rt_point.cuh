@@ -28,7 +28,14 @@ RT_HD uint32_t as_uint(float f) { union { float f; uint32_t u; } c; c.f = f; ret
 //     clamped at 0): the computed c is a convex combination of the vertices up to rounding (the margin of
 //     slot_lower_bounds relies on that).  Finite vertices: no division by zero, no NaN;
 //   * a NaN coordinate anywhere gives d2 = NaN, which no comparison accepts: such a triangle is never selected.
-struct PointHit { float cx, cy, cz, d2, w0, w1; };
+// `region` is the Voronoi region of the branch that produced c (kRegion*, DESIGN.md §4.8): in the zero-area branch the
+// chosen segment's edge, or the vertex at its end when t = 0 or t = 1.  The signed-distance kernel takes the
+// pseudo-normal of that feature.
+enum : uint32_t { kRegionFace = 0, kRegionA = 1, kRegionB = 2, kRegionC = 3, kRegionAB = 4, kRegionAC = 5, kRegionBC = 6 };
+struct PointHit { float cx, cy, cz, d2, w0, w1; uint32_t region; };
+
+// the region of a point at parameter t on the segment from vertex region `v0` to `v1` along edge region `e`
+RT_HD uint32_t seg_region(float t, uint32_t v0, uint32_t v1, uint32_t e) { return t == 0.0f ? v0 : (t == 1.0f ? v1 : e); }
 
 RT_HD float dot3f(float ax, float ay, float az, float bx, float by, float bz) {
     return fadd(fadd(fmul(ax, bx), fmul(ay, by)), fmul(az, bz));
@@ -48,7 +55,7 @@ RT_HD PointHit point_tri(float px, float py, float pz, float ax, float ay, float
     const bool nan_vertex = ax != ax || ay != ay || az != az || bx != bx || by != by || bz != bz || cx != cx ||
                             cy != cy || cz != cz;
     if (nan_vertex) {
-        r.cx = r.cy = r.cz = 0.0f; r.w0 = r.w1 = 0.0f; r.d2 = as_float(0x7fc00000u);
+        r.cx = r.cy = r.cz = 0.0f; r.w0 = r.w1 = 0.0f; r.d2 = as_float(0x7fc00000u); r.region = kRegionFace;
         return r;
     }
     const float abx = fsub(bx, ax), aby = fsub(by, ay), abz = fsub(bz, az);
@@ -76,33 +83,36 @@ RT_HD PointHit point_tri(float px, float py, float pz, float ax, float ay, float
         const float e2 = dot3f(fsub(px, qx2), fsub(py, qy2), fsub(pz, qz2), fsub(px, qx2), fsub(py, qy2), fsub(pz, qz2));
         if (e0 <= e1 && e0 <= e2) {
             r.cx = qx0; r.cy = qy0; r.cz = qz0; r.w0 = fsub(1.0f, t0); r.w1 = t0;
+            r.region = seg_region(t0, kRegionA, kRegionB, kRegionAB);
         } else if (e1 <= e2) {
             r.cx = qx1; r.cy = qy1; r.cz = qz1; r.w0 = fsub(1.0f, t1); r.w1 = 0.0f;
+            r.region = seg_region(t1, kRegionA, kRegionC, kRegionAC);
         } else {
             r.cx = qx2; r.cy = qy2; r.cz = qz2; r.w0 = 0.0f; r.w1 = fsub(1.0f, t2);
+            r.region = seg_region(t2, kRegionB, kRegionC, kRegionBC);
         }
     } else if (d1 <= 0.0f && d2 <= 0.0f) {                            // vertex a
-        r.cx = ax; r.cy = ay; r.cz = az; r.w0 = 1.0f; r.w1 = 0.0f;
+        r.cx = ax; r.cy = ay; r.cz = az; r.w0 = 1.0f; r.w1 = 0.0f; r.region = kRegionA;
     } else if (d3 >= 0.0f && d4 <= d3) {                              // vertex b
-        r.cx = bx; r.cy = by; r.cz = bz; r.w0 = 0.0f; r.w1 = 1.0f;
+        r.cx = bx; r.cy = by; r.cz = bz; r.w0 = 0.0f; r.w1 = 1.0f; r.region = kRegionB;
     } else if (vc <= 0.0f && d1 >= 0.0f && d3 <= 0.0f) {              // edge ab
         const float den = fsub(d1, d3);
         const float t = den > 0.0f ? fdiv(d1, den) : 0.0f;
         r.cx = fadd(ax, fmul(t, abx)); r.cy = fadd(ay, fmul(t, aby)); r.cz = fadd(az, fmul(t, abz));
-        r.w0 = fsub(1.0f, t); r.w1 = t;
+        r.w0 = fsub(1.0f, t); r.w1 = t; r.region = kRegionAB;
     } else if (d6 >= 0.0f && d5 <= d6) {                              // vertex c
-        r.cx = cx; r.cy = cy; r.cz = cz; r.w0 = 0.0f; r.w1 = 0.0f;
+        r.cx = cx; r.cy = cy; r.cz = cz; r.w0 = 0.0f; r.w1 = 0.0f; r.region = kRegionC;
     } else if (vb <= 0.0f && d2 >= 0.0f && d6 <= 0.0f) {              // edge ac
         const float den = fsub(d2, d6);
         const float t = den > 0.0f ? fdiv(d2, den) : 0.0f;
         r.cx = fadd(ax, fmul(t, acx)); r.cy = fadd(ay, fmul(t, acy)); r.cz = fadd(az, fmul(t, acz));
-        r.w0 = fsub(1.0f, t); r.w1 = 0.0f;
+        r.w0 = fsub(1.0f, t); r.w1 = 0.0f; r.region = kRegionAC;
     } else if (va <= 0.0f && fsub(d4, d3) >= 0.0f && fsub(d5, d6) >= 0.0f) {   // edge bc
         const float num = fsub(d4, d3);
         const float den = fadd(num, fsub(d5, d6));
         const float t = den > 0.0f ? fdiv(num, den) : 0.0f;
         r.cx = fadd(bx, fmul(t, fsub(cx, bx))); r.cy = fadd(by, fmul(t, fsub(cy, by))); r.cz = fadd(bz, fmul(t, fsub(cz, bz)));
-        r.w0 = 0.0f; r.w1 = fsub(1.0f, t);
+        r.w0 = 0.0f; r.w1 = fsub(1.0f, t); r.region = kRegionBC;
     } else {                                                          // face
         // va, vb, vc >= 0 here in exact arithmetic; v, w >= 0 and v + w <= 1 are enforced so that rounding on a sliver
         // cannot move the point off the triangle
@@ -111,7 +121,7 @@ RT_HD PointHit point_tri(float px, float py, float pz, float ax, float ay, float
         r.cx = fadd(fadd(ax, fmul(v, abx)), fmul(w, acx));
         r.cy = fadd(fadd(ay, fmul(v, aby)), fmul(w, acy));
         r.cz = fadd(fadd(az, fmul(v, abz)), fmul(w, acz));
-        r.w0 = fsub(fsub(1.0f, v), w); r.w1 = v;
+        r.w0 = fsub(fsub(1.0f, v), w); r.w1 = v; r.region = kRegionFace;
     }
     const float dx = fsub(px, r.cx), dy = fsub(py, r.cy), dz = fsub(pz, r.cz);
     r.d2 = dot3f(dx, dy, dz, dx, dy, dz);

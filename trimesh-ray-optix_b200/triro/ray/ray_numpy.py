@@ -77,3 +77,13 @@ class RayMeshIntersector:
     def winding_number(self, points, beta=2.0):
         """generalized winding number -> (n,) float64"""
         return self._rmi.winding_number(self._points(points), beta).cpu().numpy().astype(np.float64)
+
+    @property
+    def is_watertight(self):
+        """every edge of the welded surface has exactly two faces (see the torch class)"""
+        return self._rmi.is_watertight
+
+    @property
+    def is_winding_consistent(self):
+        """every two-face edge is traversed in opposite directions (see the torch class)"""
+        return self._rmi.is_winding_consistent

@@ -156,16 +156,36 @@ class RayMeshIntersector:
         """Float32[*b] — distance to the surface, positive inside and negative outside (trimesh.proximity.signed_distance).
         sign="contains": the sign is `contains_points` (with its documented decision procedure), meaningful for closed
         meshes that do not intersect themselves.  sign="winding": inside where the generalized winding number
-        (`winding_number`, beta 2) exceeds 0.5, the robust choice for open, overlapping or soup meshes.  An exact 0 is
-        returned as +0.0 either way."""
-        if sign not in ("contains", "winding"):
-            raise ValueError(f"sign must be 'contains' or 'winding' (got {sign!r})")
+        (`winding_number`, beta 2) exceeds 0.5, the robust choice for open, overlapping or soup meshes.
+        sign="pseudonormal": inside where (p - c) . n < 0 for the angle-weighted pseudo-normal n of the face, edge or
+        vertex on which the closest point c lies (Baerentzen & Aanaes 2005) — one closest-point walk per point and no
+        host sync once the pseudo-normals are cached, the usual choice for SDF samples of watertight meshes.  It is
+        exact when the welded mesh is closed, manifold and consistently oriented (`is_watertight` and
+        `is_winding_consistent`); elsewhere the result is still fully defined but is the side of the local
+        orientation (on an open heightfield: above or below it), not inside/outside.  An exact 0 is returned as +0.0
+        in every mode."""
+        if sign not in ("contains", "winding", "pseudonormal"):
+            raise ValueError(f"sign must be 'contains', 'winding' or 'pseudonormal' (got {sign!r})")
+        if sign == "pseudonormal":
+            return hops.signed_distance_pseudonormal(self.as_wrapper, points)
         _, d, _ = self.closest_point(points)
         if sign == "winding":
             inside = self.winding_number(points) > 0.5
         else:
             inside = self.contains_points(points.reshape(-1, 3)).reshape(d.shape)
         return torch.where(inside | (d == 0), d, -d)
+
+    @property
+    def is_watertight(self) -> bool:
+        """Every edge of the welded surface (corners joined by equal coordinates) has exactly two faces, as in
+        trimesh.  Reads the edge counts of the cached pseudo-normals: one host sync."""
+        boundary, non_manifold, _ = hops.edge_counts(self.as_wrapper)
+        return self.as_wrapper.header["n_tris"] > 0 and boundary == 0 and non_manifold == 0
+
+    @property
+    def is_winding_consistent(self) -> bool:
+        """Every edge of the welded surface with two faces is traversed in opposite directions by them, as in trimesh."""
+        return self.as_wrapper.header["n_tris"] > 0 and hops.edge_counts(self.as_wrapper)[2] == 0
 
     def winding_number(self, points: torch.Tensor, beta: float = 2.0) -> torch.Tensor:
         """Float32[*b] — generalized winding number of every point (Jacobson et al. 2013): the sum of the triangles'
