@@ -331,6 +331,33 @@ int rt_pseudonormals(const void* blob, void* normals, size_t normals_bytes, void
                      uint64_t* edge_counts_dev, void* stream);
 int rt_signed_distance(const void* blob, const void* normals, const rt_ray_desc* points, const rt_trace_opts* opts,
                        float* signed_distance, uint64_t* counters_dev, void* scratch, void* stream);
+/*      rt_signed_distance_closest: rt_signed_distance (the same signed_distance bits) that also writes closest [n,3],
+ *      tri_idx [n] and uv [n,2] exactly as rt_closest_point does (tri -1, closest 0, uv 0 where there is no
+ *      triangle).  All three outputs are required. */
+int rt_signed_distance_closest(const void* blob, const void* normals, const rt_ray_desc* points, const rt_trace_opts* opts,
+                               float* signed_distance, float* closest, int32_t* tri_idx, float* uv, uint64_t* counters_dev,
+                               void* scratch, void* stream);
+
+/* ---- Gradient of the distance (DESIGN.md §4.9): the backward of rt_closest_point's distance and of the signed
+ *      distances, from the forward's outputs alone (no BVH walk).  With g = grad_out[i], s = -1 when value[i] has its
+ *      sign bit set else +1, c = closest[i], (w0, w1, w2) = (uv0, uv1, 1 - uv0 - uv1):
+ *        grad_points[i]              = g * s * (p - c) / |value|                      (= q_i)
+ *        grad_vertices[faces[t][k]] += -w_k * q_i       for k = 0, 1, 2, t = tri_idx[i]
+ *      A point with value +-0, +-inf or NaN, tri_idx outside [0, n_faces), or a vertex index outside [0, n_verts)
+ *      contributes 0 (its grad_points row is +0).  `points`, opts (ray_first / ray_count) and the outputs of the
+ *      forward are laid out as in rt_closest_point: value, closest, tri_idx and uv indexed by the position in the
+ *      window, faces int32 [n_faces, 3].  grad_points (dense [n,3]) and grad_vertices ([n_verts,3], overwritten) may
+ *      each be NULL.  Deterministic: the vertex sums are stably sorted by vertex and reduced in a fixed tree over
+ *      each vertex's contributions in point order (groups of 32, left to right, then groups of 32 of those sums),
+ *      independent of the launch.  The batch runs as consecutive point windows of the size that fits
+ *      workspace_bytes (at most 2^30 / 3 points); grad_vertices starts at +0 and each window's sums are added in
+ *      window order.  rt_distance_grad_sizes: workspace for one window of n_points (the whole batch when it fits one
+ *      window); none is needed when grad_vertices is NULL.  Workspace 256-byte aligned. */
+int rt_distance_grad_sizes(int64_t n_points, int64_t n_verts, size_t* workspace_bytes);
+int rt_distance_grad(const rt_ray_desc* points, const rt_trace_opts* opts, const float* grad_out, const float* value,
+                     const float* closest, const int32_t* tri_idx, const float* uv, const int32_t* faces, int64_t n_faces,
+                     int64_t n_verts, float* grad_points, float* grad_vertices, void* workspace, size_t workspace_bytes,
+                     void* stream);
 
 /* ---- Host-buffer entry points (end-to-end path): rays and results live in (pinned) HOST memory.
  *      Copies ray chunks H2D, traces and copies results D2H on internal streams, overlapping

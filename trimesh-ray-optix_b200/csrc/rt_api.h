@@ -32,6 +32,10 @@ struct DeviceInfo { int device; int sm_count; };
 // cached per device; sm_count == 0 when there is no usable device
 int device_info(DeviceInfo* out);
 
+// rt_build.cu: the builder's onesweep sort on the low 8 * passes key bits (sorted pairs at *keys_out / *vals_out)
+int sort_pairs_low(uint64_t* keys, uint32_t* vals, int64_t n, void* workspace, int passes, uint64_t** keys_out,
+                   uint32_t** vals_out, cudaStream_t stream);
+
 inline size_t align_up_sz(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 // blocks for a grid-stride loop over n items: enough to cover them, at most per_sm blocks per SM

@@ -531,6 +531,18 @@ extern "C" int rt_bvh_refit(const float* vertices, int64_t n_verts, const int32_
     return RT_OK;
 }
 
+namespace rt {
+// The onesweep sort on the low 8 * passes key bits for other units (the caller guarantees the rest is zero); the
+// sorted pairs are at *keys_out / *vals_out (the workspace's alternate buffers after an odd number of passes).
+int sort_pairs_low(uint64_t* keys, uint32_t* vals, int64_t n, void* workspace, int passes, uint64_t** keys_out,
+                   uint32_t** vals_out, cudaStream_t stream) {
+    DeviceInfo dev;
+    RT_REQUIRE(device_info(&dev) == RT_OK && dev.sm_count > 0, RT_ERR_CUDA, "sort: no CUDA device");
+    RT_CUDA_TRY(sort::sort_pairs(keys, vals, n, workspace, dev.sm_count, stream, passes, keys_out, vals_out));
+    return RT_OK;
+}
+}  // namespace rt
+
 extern "C" int rt_sort_sizes(int64_t n, size_t* workspace_bytes) {
     RT_REQUIRE(n >= 0 && n <= (int64_t)1 << 30 && workspace_bytes, RT_ERR_INVALID, "rt_sort_sizes: bad arguments");
     *workspace_bytes = sort::workspace_bytes(n);

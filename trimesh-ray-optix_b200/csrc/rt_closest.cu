@@ -1,6 +1,7 @@
 // rt_closest.cu — closest point on the mesh for a batch of query points (rt_closest_point), the counterpart of
 // trimesh.proximity.closest_point on the BVH8 blob the ray queries use, and the pseudo-normal signed distance
-// (rt_signed_distance) that ends the same walk with one read of the rt_pseudonormals side array.
+// (rt_signed_distance) that ends the same walk with one read of the rt_pseudonormals side array;
+// rt_signed_distance_closest also writes the closest point, triangle and weights the gradient (rt_distgrad.cu) needs.
 //
 // One thread per point: stack-based traversal of the BVH8 (point_step, rt_point.cuh), children nearest first by
 // their lower bound, subtrees dropped when their bound exceeds the best squared distance found so far.  The answer is
@@ -45,9 +46,10 @@ __device__ __forceinline__ int64_t point_offset(const PointParams& p, int64_t r)
     return i0 * p.stride[0] + i1 * p.stride[1] + i2 * p.stride[2];
 }
 
-// The body of both kernels: SIGNED ends the walk with the pseudo-normal sign (DESIGN.md §4.8) instead of writing the
-// closest point, so |signed distance| is bit for bit the distance rt_closest_point returns.
-template <bool STATS, bool SIGNED>
+// The body of the three kernels: SIGNED ends the walk with the pseudo-normal sign (DESIGN.md §4.8) instead of writing
+// the closest point, so |signed distance| is bit for bit the distance rt_closest_point returns; SIGNED_CLOSEST does
+// both (closest, tri and uv as rt_closest_point writes them, no distance).
+template <bool STATS, bool SIGNED, bool SIGNED_CLOSEST = false>
 __device__ __forceinline__ void point_query(const PointParams& p) {
     using S = typename std::conditional<STATS, Stats, NoStats>::type;
     const rt_blob_header* hdr = reinterpret_cast<const rt_blob_header*>(p.blob);
@@ -73,6 +75,11 @@ __device__ __forceinline__ void point_query(const PointParams& p) {
                 const float v[9] = {as_float(a.x), as_float(a.y), as_float(a.z), as_float(b.x), as_float(b.y),
                                     as_float(b.z), as_float(c.x), as_float(c.y), as_float(c.z)};
                 p.signed_distance[i] = pseudonormal_sign(p.normals, t.slot, h, t.x, t.y, t.z, v, fsqrt(t.best));
+                if (SIGNED_CLOSEST) {
+                    p.closest[3 * i] = h.cx; p.closest[3 * i + 1] = h.cy; p.closest[3 * i + 2] = h.cz;
+                    p.tri[i] = t.prim;
+                    p.uv[2 * i] = h.w0; p.uv[2 * i + 1] = h.w1;
+                }
             } else {
                 p.closest[3 * i] = h.cx; p.closest[3 * i + 1] = h.cy; p.closest[3 * i + 2] = h.cz;
                 p.distance[i] = fsqrt(t.best);
@@ -81,6 +88,11 @@ __device__ __forceinline__ void point_query(const PointParams& p) {
             }
         } else if (SIGNED) {
             p.signed_distance[i] = as_float(0xff800000u);
+            if (SIGNED_CLOSEST) {
+                p.closest[3 * i] = 0.0f; p.closest[3 * i + 1] = 0.0f; p.closest[3 * i + 2] = 0.0f;
+                p.tri[i] = -1;
+                p.uv[2 * i] = 0.0f; p.uv[2 * i + 1] = 0.0f;
+            }
         } else {
             p.closest[3 * i] = 0.0f; p.closest[3 * i + 1] = 0.0f; p.closest[3 * i + 2] = 0.0f;
             p.distance[i] = as_float(0x7f800000u);
@@ -112,6 +124,11 @@ __global__ void __launch_bounds__(kPointThreads) k_closest_point(const __grid_co
 template <bool STATS>
 __global__ void __launch_bounds__(kPointThreads) k_signed_distance(const __grid_constant__ PointParams p) {
     point_query<STATS, true>(p);
+}
+
+template <bool STATS>
+__global__ void __launch_bounds__(kPointThreads) k_signed_distance_closest(const __grid_constant__ PointParams p) {
+    point_query<STATS, true, true>(p);
 }
 
 }  // namespace rt
@@ -175,10 +192,10 @@ extern "C" int rt_closest_point(const void* blob, const rt_ray_desc* points, con
     return RT_OK;
 }
 
-extern "C" int rt_signed_distance(const void* blob, const void* normals, const rt_ray_desc* points, const rt_trace_opts* opts,
-                                  float* signed_distance, uint64_t* counters_dev, void* scratch, void* stream) {
-    (void)scratch;
-    const char* fn = "rt_signed_distance";
+// Both signed-distance entry points; closest, tri_idx and uv are all null (rt_signed_distance) or all set.
+static int signed_distance_launch(const char* fn, const void* blob, const void* normals, const rt_ray_desc* points,
+                                  const rt_trace_opts* opts, float* signed_distance, float* closest, int32_t* tri_idx, float* uv,
+                                  uint64_t* counters_dev, void* stream) {
     RT_REQUIRE(normals != nullptr && ((uintptr_t)normals & 15) == 0, RT_ERR_INVALID,
                "%s: normals null or not 16-byte aligned", fn);
     PointParams p;
@@ -189,11 +206,33 @@ extern "C" int rt_signed_distance(const void* blob, const void* normals, const r
     p.max_distance = as_float(0x7f800000u);
     p.normals = reinterpret_cast<const uint8_t*>(normals);
     p.signed_distance = signed_distance;
+    p.closest = closest; p.tri = tri_idx; p.uv = uv;
     const unsigned grid = (unsigned)((count + kPointThreads - 1) / kPointThreads);
-    if (counters_dev)
+    if (closest && counters_dev)
+        k_signed_distance_closest<true><<<grid, kPointThreads, 0, (cudaStream_t)stream>>>(p);
+    else if (closest)
+        k_signed_distance_closest<false><<<grid, kPointThreads, 0, (cudaStream_t)stream>>>(p);
+    else if (counters_dev)
         k_signed_distance<true><<<grid, kPointThreads, 0, (cudaStream_t)stream>>>(p);
     else
         k_signed_distance<false><<<grid, kPointThreads, 0, (cudaStream_t)stream>>>(p);
     RT_CUDA_TRY(cudaGetLastError());
     return RT_OK;
+}
+
+extern "C" int rt_signed_distance(const void* blob, const void* normals, const rt_ray_desc* points, const rt_trace_opts* opts,
+                                  float* signed_distance, uint64_t* counters_dev, void* scratch, void* stream) {
+    (void)scratch;
+    return signed_distance_launch("rt_signed_distance", blob, normals, points, opts, signed_distance, nullptr, nullptr, nullptr,
+                                  counters_dev, stream);
+}
+
+extern "C" int rt_signed_distance_closest(const void* blob, const void* normals, const rt_ray_desc* points,
+                                          const rt_trace_opts* opts, float* signed_distance, float* closest,
+                                          int32_t* tri_idx, float* uv, uint64_t* counters_dev, void* scratch,
+                                          void* stream) {
+    (void)scratch;
+    const char* fn = "rt_signed_distance_closest";
+    RT_REQUIRE(closest && tri_idx && uv, RT_ERR_INVALID, "%s: null output", fn);
+    return signed_distance_launch(fn, blob, normals, points, opts, signed_distance, closest, tri_idx, uv, counters_dev, stream);
 }

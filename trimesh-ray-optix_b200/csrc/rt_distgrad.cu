@@ -1,0 +1,232 @@
+// rt_distgrad.cu — the gradient of the point-to-mesh distance with respect to the query points and the mesh vertices
+// (rt_distance_grad, DESIGN.md §4.9), from the outputs of rt_closest_point or rt_signed_distance_closest alone.
+//
+// Per point window, with the arithmetic of rt_distgrad.cuh:
+//   1. one thread per point: grad_points and, when the vertex gradient is wanted, q (12 B) and three
+//      (key = vertex, value = pair index 3 i + k) pairs;
+//   2. the builder's stable onesweep sort of the pairs on the low bits of the key (ceil(log2(n_verts + 1)) bits,
+//      at most 4 passes): each vertex's pairs become one run, in ascending pair order;
+//   3. the run starts, then the tree reduction: level 0 sums groups of kDgGroup pairs of a run, every further level
+//      groups of kDgGroup sums of the level below; a run that fits one group is added to grad_vertices.
+// Nothing is atomic and every sum has one fixed order, so the result does not depend on the launch.
+#include "rt_api.h"
+#include "rt_distgrad.cuh"
+
+namespace rt {
+
+constexpr int kDgThreads = 256;
+
+struct DgPointParams {
+    const float* points;
+    int64_t shape[4], stride[4];
+    int packed;
+    int64_t first;               // batch index of window position 0
+    int64_t n;                   // points in this launch, window positions [base, base + n)
+    int64_t base;
+    const float* grad_out;
+    const float* value;
+    const float* closest;
+    const int32_t* tri;
+    const int32_t* faces;
+    int64_t n_faces, n_verts;
+    float* grad_points;          // [window, 3] or null
+    float* q;                    // [n, 3] or null (no vertex gradient)
+    uint64_t* keys;              // [3 n]
+    uint32_t* vals;              // [3 n]
+};
+
+__global__ void __launch_bounds__(kDgThreads) k_dg_points(const __grid_constant__ DgPointParams p) {
+    const int64_t i = (int64_t)blockIdx.x * kDgThreads + threadIdx.x;
+    if (i >= p.n) return;
+    const int64_t w = p.base + i;              // position in the caller's window
+    const int64_t r = p.first + w;             // index in the batch
+    int64_t o;
+    if (p.packed) {
+        o = 3 * r;
+    } else {
+        const int64_t i2 = r % p.shape[2], qq = r / p.shape[2];
+        o = (qq / p.shape[1]) * p.stride[0] + (qq % p.shape[1]) * p.stride[1] + i2 * p.stride[2];
+    }
+    const int64_t os = p.stride[3];
+    const int32_t t = p.tri[w];
+    float q[3];
+    const bool live = dg_point_q(p.points[o], p.points[o + os], p.points[o + 2 * os], p.grad_out[w], p.value[w],
+                                 p.closest[3 * w], p.closest[3 * w + 1], p.closest[3 * w + 2], t, p.n_faces, q);
+    if (p.grad_points) {
+        p.grad_points[3 * w] = q[0]; p.grad_points[3 * w + 1] = q[1]; p.grad_points[3 * w + 2] = q[2];
+    }
+    if (p.q) {
+        p.q[3 * i] = q[0]; p.q[3 * i + 1] = q[1]; p.q[3 * i + 2] = q[2];
+#pragma unroll
+        for (uint32_t k = 0; k < 3; ++k) {
+            p.keys[3 * i + k] = dg_key(live, p.faces, t, k, p.n_verts);
+            p.vals[3 * i + k] = (uint32_t)(3 * i + k);
+        }
+    }
+}
+
+__global__ void __launch_bounds__(kDgThreads) k_dg_run_start(const uint64_t* keys, int64_t m, uint64_t n_verts,
+                                                             uint32_t* start) {
+    const int64_t stride = (int64_t)gridDim.x * kDgThreads;
+    for (int64_t j = (int64_t)blockIdx.x * kDgThreads + threadIdx.x; j < m; j += stride)
+        dg_run_start((uint64_t)j, keys, n_verts, start);
+}
+
+__global__ void __launch_bounds__(kDgThreads) k_dg_level0(const uint64_t* keys, const uint32_t* vals, int64_t m,
+                                                          const uint32_t* start, uint64_t n_verts, const float* q,
+                                                          const float* uv, float* grad_vertices, DgLevel next) {
+    const int64_t stride = (int64_t)gridDim.x * kDgThreads;
+    for (int64_t j = (int64_t)blockIdx.x * kDgThreads + threadIdx.x; j < m; j += stride)
+        dg_level0_at((uint64_t)j, (uint64_t)m, keys, vals, start, n_verts, q, uv, grad_vertices, next);
+}
+
+__global__ void __launch_bounds__(kDgThreads) k_dg_level(DgLevel cur, int64_t size, float* grad_vertices, DgLevel next) {
+    const int64_t stride = (int64_t)gridDim.x * kDgThreads;
+    for (int64_t j = (int64_t)blockIdx.x * kDgThreads + threadIdx.x; j < size; j += stride)
+        dg_level_at((uint64_t)j, (uint64_t)size, cur, grad_vertices, next);
+}
+
+// Workspace of a window of w points: q, keys, values, sort workspace, run starts, two level buffers.
+struct DgWorkspace {
+    float* q;
+    uint64_t* keys;
+    uint32_t* vals;
+    void* sort_ws;
+    uint32_t* start;
+    DgLevel lv[2];
+    size_t total;
+};
+static DgWorkspace carve_dg(void* base, int64_t w, int64_t n_verts) {
+    const int64_t m = 3 * w;
+    const uint64_t slots = dg_next_size((uint64_t)m);
+    size_t sb = 0;
+    rt_sort_sizes(m, &sb);
+    const size_t sizes[10] = {(size_t)w * 12u, (size_t)m * 8u, (size_t)m * 4u, sb, (size_t)n_verts * 4u,
+                              slots * 4u, slots * 4u, slots * 12u, slots * 4u, slots * 4u};
+    size_t off[11];
+    off[0] = 0;
+    for (int i = 0; i < 10; ++i) off[i + 1] = off[i] + align_up_sz(sizes[i], 256);
+    // the last level buffer's values follow its idx array
+    const size_t total = off[10] + align_up_sz(slots * 12u, 256);
+    uint8_t* p = reinterpret_cast<uint8_t*>(base);
+    auto at = [&](size_t o) { return p ? p + o : nullptr; };
+    DgWorkspace ws;
+    ws.q = reinterpret_cast<float*>(at(off[0]));
+    ws.keys = reinterpret_cast<uint64_t*>(at(off[1]));
+    ws.vals = reinterpret_cast<uint32_t*>(at(off[2]));
+    ws.sort_ws = at(off[3]);
+    ws.start = reinterpret_cast<uint32_t*>(at(off[4]));
+    ws.lv[0] = DgLevel{reinterpret_cast<uint32_t*>(at(off[5])), reinterpret_cast<uint32_t*>(at(off[6])),
+                       reinterpret_cast<float*>(at(off[7]))};
+    ws.lv[1] = DgLevel{reinterpret_cast<uint32_t*>(at(off[8])), reinterpret_cast<uint32_t*>(at(off[9])),
+                       reinterpret_cast<float*>(at(off[10]))};
+    ws.total = total;
+    return ws;
+}
+
+constexpr int64_t kDgMaxVerts = 0xffffffffll;     // vertex ids and the sentinel n_verts fit 32 bits
+
+}  // namespace rt
+
+using namespace rt;
+
+extern "C" int rt_distance_grad_sizes(int64_t n_points, int64_t n_verts, size_t* workspace_bytes) {
+    RT_REQUIRE(n_points >= 0 && n_verts >= 0 && n_verts < kDgMaxVerts && workspace_bytes, RT_ERR_INVALID,
+               "rt_distance_grad_sizes: bad arguments (at most %lld vertices)", (long long)(kDgMaxVerts - 1));
+    *workspace_bytes = carve_dg(nullptr, n_points < kDgMaxPoints ? n_points : kDgMaxPoints, n_verts).total;
+    return RT_OK;
+}
+
+extern "C" int rt_distance_grad(const rt_ray_desc* points, const rt_trace_opts* opts, const float* grad_out,
+                                const float* value, const float* closest, const int32_t* tri_idx, const float* uv,
+                                const int32_t* faces, int64_t n_faces, int64_t n_verts, float* grad_points,
+                                float* grad_vertices, void* workspace, size_t workspace_bytes, void* stream_) {
+    const char* fn = "rt_distance_grad";
+    cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+    RT_REQUIRE(points != nullptr, RT_ERR_INVALID, "%s: null point descriptor", fn);
+    RT_REQUIRE(points->nray >= 0 && points->shape[3] == 3, RT_ERR_INVALID, "%s: point batch must be [*b, 3]", fn);
+    RT_REQUIRE(points->shape[0] >= 0 && points->shape[1] >= 0 && points->shape[2] >= 0 &&
+                   points->shape[0] * points->shape[1] * points->shape[2] == points->nray,
+               RT_ERR_INVALID, "%s: nray %lld does not match shape", fn, (long long)points->nray);
+    RT_REQUIRE(n_faces >= 0 && n_verts >= 0 && n_verts < kDgMaxVerts, RT_ERR_INVALID,
+               "%s: bad mesh size (%lld faces, %lld vertices)", fn, (long long)n_faces, (long long)n_verts);
+    static const rt_trace_opts kDefaults = {};
+    const rt_trace_opts& o = opts ? *opts : kDefaults;
+    RT_REQUIRE(o.ray_first >= 0 && o.ray_first <= points->nray, RT_ERR_INVALID, "%s: ray_first %lld outside [0, %lld]", fn,
+               (long long)o.ray_first, (long long)points->nray);
+    const int64_t n = o.ray_count <= 0 ? points->nray - o.ray_first : o.ray_count;
+    RT_REQUIRE(n <= points->nray - o.ray_first, RT_ERR_INVALID, "%s: window [%lld, +%lld) exceeds the batch of %lld", fn,
+               (long long)o.ray_first, (long long)n, (long long)points->nray);
+    if (grad_vertices) RT_CUDA_TRY(cudaMemsetAsync(grad_vertices, 0, (size_t)n_verts * 12u, stream));
+    if (n == 0 || (!grad_points && !grad_vertices)) return RT_OK;
+    RT_REQUIRE(points->origins && grad_out && value && closest && tri_idx && uv, RT_ERR_INVALID, "%s: null input", fn);
+    RT_REQUIRE(!grad_vertices || faces || n_faces == 0, RT_ERR_INVALID, "%s: null faces", fn);
+
+    DgPointParams p{};
+    p.points = points->origins;
+    for (int a = 0; a < 4; ++a) { p.shape[a] = points->shape[a]; p.stride[a] = points->o_stride[a]; }
+    p.packed = points_packed(points->shape, points->o_stride) ? 1 : 0;
+    p.first = o.ray_first;
+    p.grad_out = grad_out; p.value = value; p.closest = closest; p.tri = tri_idx; p.faces = faces;
+    p.n_faces = n_faces; p.n_verts = n_verts;
+    p.grad_points = grad_points;
+
+    if (!grad_vertices) {   // one pass, no sort
+        RT_REQUIRE((n + kDgThreads - 1) / kDgThreads < ((int64_t)1 << 31), RT_ERR_INVALID,
+                   "%s: batch of %lld points too large for one launch", fn, (long long)n);
+        p.n = n; p.base = 0;
+        k_dg_points<<<(unsigned)((n + kDgThreads - 1) / kDgThreads), kDgThreads, 0, stream>>>(p);
+        RT_CUDA_TRY(cudaGetLastError());
+        return RT_OK;
+    }
+
+    // the largest window whose workspace fits
+    RT_REQUIRE(workspace != nullptr && ((uintptr_t)workspace & 255) == 0, RT_ERR_INVALID,
+               "%s: workspace null or not 256-byte aligned", fn);
+    int64_t win = n < kDgMaxPoints ? n : kDgMaxPoints;
+    if (carve_dg(nullptr, win, n_verts).total > workspace_bytes) {
+        int64_t lo = 0, hi = win;                       // fits(lo), !fits(hi)
+        while (hi - lo > 1) {
+            const int64_t mid = lo + (hi - lo) / 2;
+            (carve_dg(nullptr, mid, n_verts).total <= workspace_bytes ? lo : hi) = mid;
+        }
+        win = lo;
+    }
+    RT_REQUIRE(win > 0, RT_ERR_SIZE, "%s: workspace %zu < %zu (one point)", fn, workspace_bytes,
+               carve_dg(nullptr, 1, n_verts).total);
+    const DgWorkspace w = carve_dg(workspace, win, n_verts);
+    DeviceInfo dev;
+    RT_REQUIRE(device_info(&dev) == RT_OK && dev.sm_count > 0, RT_ERR_CUDA, "%s: no CUDA device", fn);
+    const int passes = dg_sort_passes(n_verts);
+    p.q = w.q; p.keys = w.keys; p.vals = w.vals;
+    for (int64_t base = 0; base < n; base += win) {
+        const int64_t nw = n - base < win ? n - base : win;
+        const int64_t m = 3 * nw;
+        p.n = nw; p.base = base;
+        k_dg_points<<<(unsigned)((nw + kDgThreads - 1) / kDgThreads), kDgThreads, 0, stream>>>(p);
+        RT_CUDA_TRY(cudaGetLastError());
+        uint64_t* keys = nullptr;
+        uint32_t* vals = nullptr;
+        const int rc = sort_pairs_low(w.keys, w.vals, m, w.sort_ws, passes, &keys, &vals, stream);
+        if (rc != RT_OK) return rc;
+        const int grid = grid_for(m, kDgThreads, dev.sm_count, 8);
+        k_dg_run_start<<<grid, kDgThreads, 0, stream>>>(keys, m, (uint64_t)n_verts, w.start);
+        // level l holds `size` slots; runs at most `len` long; it forwards into the next level while len > kDgGroup
+        uint64_t size = (uint64_t)m, len = (uint64_t)m;
+        int cur = 0;
+        if (len > kDgGroup) RT_CUDA_TRY(cudaMemsetAsync(w.lv[0].key, 0xff, dg_next_size(size) * 4u, stream));
+        k_dg_level0<<<grid, kDgThreads, 0, stream>>>(keys, vals, m, w.start, (uint64_t)n_verts, w.q, uv + 2 * base,
+                                                     grad_vertices, w.lv[0]);
+        RT_CUDA_TRY(cudaGetLastError());
+        while (len > kDgGroup) {
+            size = dg_next_size(size);
+            len = (len + kDgGroup - 1) / kDgGroup;
+            if (len > kDgGroup) RT_CUDA_TRY(cudaMemsetAsync(w.lv[cur ^ 1].key, 0xff, dg_next_size(size) * 4u, stream));
+            k_dg_level<<<grid_for((int64_t)size, kDgThreads, dev.sm_count, 8), kDgThreads, 0, stream>>>(
+                w.lv[cur], (int64_t)size, grad_vertices, w.lv[cur ^ 1]);
+            RT_CUDA_TRY(cudaGetLastError());
+            cur ^= 1;
+        }
+    }
+    return RT_OK;
+}

@@ -107,6 +107,9 @@ def _declare(lib):
         "rt_pseudonormals_sizes": (ci, [i64, psz, psz]),
         "rt_pseudonormals": (ci, [vp, vp, sz, vp, sz, vp, vp]),
         "rt_signed_distance": (ci, [vp, vp, prd, pto, vp, vp, vp, vp]),
+        "rt_signed_distance_closest": (ci, [vp, vp, prd, pto, vp, vp, vp, vp, vp, vp, vp]),
+        "rt_distance_grad_sizes": (ci, [i64, i64, psz]),
+        "rt_distance_grad": (ci, [prd, pto, vp, vp, vp, vp, vp, vp, i64, i64, vp, vp, vp, sz, vp]),
         "rt_host_closest_sizes": (ci, [i64, psz]),
         "rt_host_trace_closest": (ci, [vp, i64, vp, ci, vp, pto, vp, vp, vp, vp, vp, vp, sz]),
         "rt_host_trace_closest_compact": (ci, [vp, i64, vp, ci, vp, pto, vp, vp, vp, vp, vp, vp, C.POINTER(C.c_int64), vp, sz]),
@@ -914,11 +917,12 @@ def pseudo_normals(accel_structure) -> tuple[torch.Tensor, torch.Tensor]:
 
 
 def signed_distance_pseudonormal(accel_structure, points: torch.Tensor, ray_first: int = 0, ray_count: int = -1,
-                                 counters: torch.Tensor | None = None) -> torch.Tensor:
+                                 counters: torch.Tensor | None = None, return_closest: bool = False):
     """Float32[*b]: distance to the surface, positive inside, with the sign of the angle-weighted pseudo-normal of the
     closest feature (Baerentzen & Aanaes 2005): one closest-point walk per point, no host sync once pseudo_normals()
     is cached.  |result| is bit for bit closest_point's distance; an exact 0 is +0; a non-finite point or an empty
-    mesh gives -inf.  Batch, window and counters as closest_point."""
+    mesh gives -inf.  Batch, window and counters as closest_point.  return_closest=True returns
+    (signed distance, closest, tri, uv) from the same walk, the last three exactly as closest_point's."""
     tensor_input_check(points)
     blob = _blob_of(accel_structure, points.device)
     rd, batch = make_ray_desc(points, None)
@@ -930,18 +934,70 @@ def signed_distance_pseudonormal(accel_structure, points: torch.Tensor, ray_firs
         raise ValueError("counters must be a contiguous int64 tensor of 4 elements on the points' device")
     with _on_device(dev):
         sd = torch.empty(batch, dtype=torch.float32, device=dev)
+        if return_closest:
+            closest = torch.empty((*batch, 3), dtype=torch.float32, device=dev)
+            tri = torch.empty(batch, dtype=torch.int32, device=dev)
+            uv = torch.empty((*batch, 2), dtype=torch.float32, device=dev)
         if sd.numel() == 0:
             if counters is not None:
                 counters.zero_()
-            return sd
+            return (sd, closest, tri, uv) if return_closest else sd
         normals, _ = pseudo_normals(accel_structure)
         # an empty mesh has an empty (null) normals tensor: the kernel finds no triangle and reads no row
         nptr = _ptr(normals) if normals.numel() else _ptr(blob)
         st = _stream(dev)
-        _check(get_module().rt_signed_distance(_ptr(blob), nptr, C.byref(rd),
-                                               C.byref(trace_opts(accel_structure, ray_first, ray_count)), _ptr(sd),
-                                               _ptr(counters), _ptr(_scratch(dev, st)), st), "rt_signed_distance")
+        opts = C.byref(trace_opts(accel_structure, ray_first, ray_count))
+        if return_closest:
+            _check(get_module().rt_signed_distance_closest(_ptr(blob), nptr, C.byref(rd), opts, _ptr(sd), _ptr(closest),
+                                                           _ptr(tri), _ptr(uv), _ptr(counters), _ptr(_scratch(dev, st)),
+                                                           st), "rt_signed_distance_closest")
+            return sd, closest, tri, uv
+        _check(get_module().rt_signed_distance(_ptr(blob), nptr, C.byref(rd), opts, _ptr(sd), _ptr(counters),
+                                               _ptr(_scratch(dev, st)), st), "rt_signed_distance")
     return sd
+
+
+def distance_grad_workspace_bytes(n_points: int, n_verts: int) -> int:
+    """Workspace rt_distance_grad needs to run a batch of n_points as one window."""
+    wb = C.c_size_t()
+    _check(get_module().rt_distance_grad_sizes(int(n_points), int(n_verts), C.byref(wb)), "rt_distance_grad_sizes")
+    return wb.value
+
+
+def distance_grad(points: torch.Tensor, grad_out: torch.Tensor, value: torch.Tensor, closest: torch.Tensor,
+                  tri: torch.Tensor, uv: torch.Tensor, faces: torch.Tensor, n_verts: int, points_grad: bool = True,
+                  vertices_grad: bool = True, workspace_bytes: int | None = None):
+    """Backward of a distance (closest_point's) or signed distance (any sign mode) from the forward's outputs, with
+    no BVH walk: (grad_points Float32[*b,3] or None, grad_vertices Float32[n_verts,3] or None).  With g = grad_out,
+    s = the sign of value (+1 for +0), grad_points = g s (p - c) / |value| and every point adds -w_k times that to
+    vertex faces[tri][k], w = (uv0, uv1, 1 - uv0 - uv1).  A point with value +-0, +-inf or NaN, or tri -1, gives 0.
+    The vertex sums are a sort and a fixed-order tree (DESIGN.md §4.9): the same inputs give the same bits on every
+    run.  `workspace_bytes` bounds the workspace (default: one window for the whole batch); a smaller one runs the
+    batch as several point windows, whose sums are added in window order."""
+    tensor_input_check(points)
+    rd, batch = make_ray_desc(points, None)
+    dev = points.device
+    n = rd.nray
+    for name, t, shape, dt in (("grad_out", grad_out, batch, torch.float32), ("value", value, batch, torch.float32),
+                               ("closest", closest, (*batch, 3), torch.float32), ("tri", tri, batch, torch.int32),
+                               ("uv", uv, (*batch, 2), torch.float32)):
+        if tuple(t.shape) != tuple(shape) or t.dtype != dt or t.device != dev:
+            raise ValueError(f"{name} must be {dt} {tuple(shape)} on {dev}, got {t.dtype} {tuple(t.shape)} on {t.device}")
+    if faces.dtype != torch.int32 or faces.dim() != 2 or faces.shape[1] != 3 or faces.device != dev:
+        raise ValueError("faces must be int32 [f, 3] on the points' device")
+    grad_out, value, closest, tri, uv, faces = (t.contiguous() for t in (grad_out, value, closest, tri, uv, faces))
+    with _on_device(dev):
+        gp = torch.empty((*batch, 3), dtype=torch.float32, device=dev) if points_grad else None
+        gv = torch.empty((int(n_verts), 3), dtype=torch.float32, device=dev) if vertices_grad else None
+        wb = 0
+        if gv is not None:
+            wb = distance_grad_workspace_bytes(n, n_verts) if workspace_bytes is None else int(workspace_bytes)
+        ws = torch.empty(max(wb, 256), dtype=torch.uint8, device=dev) if gv is not None else None
+        _check(get_module().rt_distance_grad(C.byref(rd), C.byref(trace_opts()), _ptr(grad_out), _ptr(value),
+                                             _ptr(closest), _ptr(tri), _ptr(uv), _ptr(faces), faces.shape[0],
+                                             int(n_verts), _ptr(gp), _ptr(gv), _ptr(ws), wb, _stream(dev)),
+               "rt_distance_grad")
+    return gp, gv
 
 
 def edge_counts(accel_structure) -> tuple[int, int, int]:

@@ -14,6 +14,7 @@ from typing import Optional, Tuple
 import torch
 
 import triro.backend.ops as hops
+from torch.autograd.function import once_differentiable
 
 
 class RayMeshIntersector:
@@ -145,12 +146,26 @@ class RayMeshIntersector:
         every query point, in the order of trimesh.proximity.closest_point.  Triangles farther than `max_distance`
         (None = unbounded) are ignored; a point with no triangle in reach gets triangle_id -1, distance inf and
         closest 0.  Equal distances go to the smaller triangle index.  uv are the weights of the triangle's vertices
-        0 and 1 like intersects_closest's, so `interpolate(attr, triangle_id, uv)` transfers attributes."""
+        0 and 1 like intersects_closest's, so `interpolate(attr, triangle_id, uv)` transfers attributes.
+
+        `distance` is differentiable with respect to `points` and to `mesh_vertices` (the tensor made from what was
+        last given to the constructor, `update_raw` or `refit`, so gradients reach the caller's tensor): d(distance)/dp
+        = (p - closest) / distance and vertex k of the triangle gets -w_k times that.  It is 0 where the distance is
+        0 or inf.  `closest`, `triangle_id` and `uv` are not differentiable: write losses in terms of `distance`
+        (a loss on |p - closest| would give no vertex gradient).  The BVH does not follow the vertices: call
+        `refit(vertices)` after each optimiser step.  Nothing of this runs unless grad mode is on and `points` or
+        `mesh_vertices` requires grad; the gradients are deterministic to the bit."""
         md = float("inf") if max_distance is None else float(max_distance)
-        closest, distance, tri, uv = hops.closest_point(self.as_wrapper, points, md)
+        if self._tracks_grad(points):
+            closest, distance, tri, uv = _ClosestPointFn.apply(points, self.mesh_vertices, self, md)
+        else:
+            closest, distance, tri, uv = hops.closest_point(self.as_wrapper, points, md)
         if return_uv:
             return closest, distance, tri, uv
         return closest, distance, tri
+
+    def _tracks_grad(self, points: torch.Tensor) -> bool:
+        return torch.is_grad_enabled() and (points.requires_grad or self.mesh_vertices.requires_grad)
 
     def signed_distance(self, points: torch.Tensor, sign: str = "contains") -> torch.Tensor:
         """Float32[*b] — distance to the surface, positive inside and negative outside (trimesh.proximity.signed_distance).
@@ -163,10 +178,13 @@ class RayMeshIntersector:
         exact when the welded mesh is closed, manifold and consistently oriented (`is_watertight` and
         `is_winding_consistent`); elsewhere the result is still fully defined but is the side of the local
         orientation (on an open heightfield: above or below it), not inside/outside.  An exact 0 is returned as +0.0
-        in every mode."""
+        in every mode.  Differentiable in every mode with respect to `points` and `mesh_vertices`, like
+        `closest_point`'s distance (the sign is piecewise constant); call `refit(vertices)` after each optimiser step."""
         if sign not in ("contains", "winding", "pseudonormal"):
             raise ValueError(f"sign must be 'contains', 'winding' or 'pseudonormal' (got {sign!r})")
         if sign == "pseudonormal":
+            if self._tracks_grad(points):
+                return _PseudonormalSDFFn.apply(points, self.mesh_vertices, self)
             return hops.signed_distance_pseudonormal(self.as_wrapper, points)
         _, d, _ = self.closest_point(points)
         if sign == "winding":
@@ -249,6 +267,48 @@ def contains_points_flow(parity, points: torch.Tensor, check_direction, reduce_f
     if not sub_inside or sub_broken:
         contain.logical_and_(was_broken.logical_not_())      # contains[broken] = False, as two elementwise kernels
     return contain
+
+
+def _distance_backward(ctx, grad_value):
+    points, value, closest, tri, uv = ctx.saved_tensors
+    r = ctx.intersector
+    return hops.distance_grad(points, grad_value, value, closest, tri, uv, r.mesh_faces, r.mesh_vertices.shape[0],
+                              points_grad=ctx.needs_input_grad[0], vertices_grad=ctx.needs_input_grad[1])
+
+
+class _ClosestPointFn(torch.autograd.Function):
+    """closest_point with a differentiable distance (DESIGN.md §4.9); `vertices` is only the autograd handle of
+    mesh_vertices, the forward walks the BVH."""
+
+    @staticmethod
+    def forward(ctx, points, vertices, intersector, max_distance):
+        closest, distance, tri, uv = hops.closest_point(intersector.as_wrapper, points.detach(), max_distance)
+        ctx.mark_non_differentiable(closest, tri, uv)
+        ctx.save_for_backward(points, distance, closest, tri, uv)
+        ctx.intersector = intersector
+        return closest, distance, tri, uv
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_closest, grad_distance, grad_tri, grad_uv):
+        return (*_distance_backward(ctx, grad_distance), None, None)
+
+
+class _PseudonormalSDFFn(torch.autograd.Function):
+    """signed_distance(sign="pseudonormal") with its gradient: one walk gives the sign and the closest feature."""
+
+    @staticmethod
+    def forward(ctx, points, vertices, intersector):
+        sd, closest, tri, uv = hops.signed_distance_pseudonormal(intersector.as_wrapper, points.detach(),
+                                                                 return_closest=True)
+        ctx.save_for_backward(points, sd, closest, tri, uv)
+        ctx.intersector = intersector
+        return sd
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_sd):
+        return (*_distance_backward(ctx, grad_sd), None)
 
 
 class OptixAccelStructureWrapper:
