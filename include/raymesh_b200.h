@@ -359,6 +359,35 @@ int rt_distance_grad(const rt_ray_desc* points, const rt_trace_opts* opts, const
                      int64_t n_verts, float* grad_points, float* grad_vertices, void* workspace, size_t workspace_bytes,
                      void* stream);
 
+/* ---- Gradient of the hit locations and barycentrics (DESIGN.md §4.10): the backward of rt_trace_closest's loc and uv
+ *      (dense or compacted) and of the all-hits loc, with respect to the rays and the mesh vertices, without a BVH
+ *      walk.  Row i is the hit of triangle t = tri_idx[i] by ray r = row_ray[i] of the window (row_ray NULL: r = i,
+ *      and n_rows must equal the window's ray count unless it is 0); g_L = grad_loc[i] (NULL: 0) and
+ *      g_U = grad_uv[i] (NULL: 0).
+ *      With v0, v1, v2 = vertices[faces[t]], e1 = v1 - v0, e2 = v2 - v0, the hit is recomputed in binary32 with one
+ *      fixed Moeller-Trumbore sequence:
+ *        s = o - v0, p = d x e2, det = e1.p, b1 = s.p / det, r = s x e1, b2 = d.r / det, t = e2.r / det
+ *        gb1 = g_L.e1 - g_U0 + g_U1, gb2 = g_L.e2 - g_U0, lambda = (gb1 p + gb2 (e1 x d)) / det
+ *        grad_origins[r] += lambda, grad_directions[r] += t lambda,
+ *        grad_vertices[faces[t][k]] += -w_k (lambda - g_L),   w = (1 - b1 - b2, b1, 1 - w0 - w1)
+ *      A row whose triangle is outside [0, n_faces), with a vertex index outside [0, n_verts), a row_ray outside
+ *      the window, det = 0, or any non-finite value among lambda, t lambda, lambda - g_L and w contributes 0.  The
+ *      rows of one ray must be contiguous (row_ray non-decreasing, as rt_compact_scatter and rt_allhits_scatter
+ *      write it); each ray's sums run over its rows left to right from +0, and rays without rows get +0 (with
+ *      n_rows = 0 every ray and vertex does, whatever row_ray is).  The vertex sums are those of rt_distance_grad: a
+ *      stable sort by vertex and the fixed 32-ary tree per vertex, in row windows of the size that fits
+ *      workspace_bytes (at most 2^30 / 3 rows), added in window order.  The zero rules are per row: finite rows can
+ *      still overflow in a product or a sum, as in rt_distance_grad.
+ *      `rays` and opts (ray_first / ray_count only) are those of the forward; vertices float32 [n_verts, 3], faces
+ *      int32 [n_faces, 3].  grad_origins and grad_directions (dense [window, 3]) and grad_vertices ([n_verts, 3],
+ *      overwritten) may each be NULL.  rt_ray_grad_sizes: workspace for one window of n_rows (the whole batch when it
+ *      fits one window); none is needed when grad_vertices is NULL.  Workspace 256-byte aligned. */
+int rt_ray_grad_sizes(int64_t n_rows, int64_t n_verts, size_t* workspace_bytes);
+int rt_ray_grad(const rt_ray_desc* rays, const rt_trace_opts* opts, int64_t n_rows, const int32_t* row_ray,
+                const int32_t* tri_idx, const float* grad_loc, const float* grad_uv, const float* vertices, int64_t n_verts,
+                const int32_t* faces, int64_t n_faces, float* grad_origins, float* grad_directions, float* grad_vertices,
+                void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- Host-buffer entry points (end-to-end path): rays and results live in (pinned) HOST memory.
  *      Copies ray chunks H2D, traces and copies results D2H on internal streams, overlapping
  *      the three; `dev_work` is caller-provided device memory of rt_host_closest_sizes() bytes.

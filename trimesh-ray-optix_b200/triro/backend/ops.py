@@ -110,6 +110,8 @@ def _declare(lib):
         "rt_signed_distance_closest": (ci, [vp, vp, prd, pto, vp, vp, vp, vp, vp, vp, vp]),
         "rt_distance_grad_sizes": (ci, [i64, i64, psz]),
         "rt_distance_grad": (ci, [prd, pto, vp, vp, vp, vp, vp, vp, i64, i64, vp, vp, vp, sz, vp]),
+        "rt_ray_grad_sizes": (ci, [i64, i64, psz]),
+        "rt_ray_grad": (ci, [prd, pto, i64, vp, vp, vp, vp, vp, i64, vp, i64, vp, vp, vp, vp, sz, vp]),
         "rt_host_closest_sizes": (ci, [i64, psz]),
         "rt_host_trace_closest": (ci, [vp, i64, vp, ci, vp, pto, vp, vp, vp, vp, vp, vp, sz]),
         "rt_host_trace_closest_compact": (ci, [vp, i64, vp, ci, vp, pto, vp, vp, vp, vp, vp, vp, C.POINTER(C.c_int64), vp, sz]),
@@ -998,6 +1000,57 @@ def distance_grad(points: torch.Tensor, grad_out: torch.Tensor, value: torch.Ten
                                              int(n_verts), _ptr(gp), _ptr(gv), _ptr(ws), wb, _stream(dev)),
                "rt_distance_grad")
     return gp, gv
+
+
+def ray_grad_workspace_bytes(n_rows: int, n_verts: int) -> int:
+    """Workspace rt_ray_grad needs to run n_rows hit rows as one window."""
+    wb = C.c_size_t()
+    _check(get_module().rt_ray_grad_sizes(int(n_rows), int(n_verts), C.byref(wb)), "rt_ray_grad_sizes")
+    return wb.value
+
+
+def ray_grad(origins: torch.Tensor, dirs: torch.Tensor, tri: torch.Tensor, grad_loc: torch.Tensor | None,
+             grad_uv: torch.Tensor | None, vertices: torch.Tensor, faces: torch.Tensor,
+             ray_idx: torch.Tensor | None = None, origins_grad: bool = True, directions_grad: bool = True,
+             vertices_grad: bool = True, workspace_bytes: int | None = None):
+    """Backward of the hit locations (and barycentrics) of intersects_closest, compact_closest or intersects_location,
+    with no BVH walk: (grad_origins Float32[*b,3] or None, grad_directions Float32[*b,3] or None, grad_vertices
+    Float32[n_verts,3] or None).  Row i is the hit of triangle tri[i] by ray ray_idx[i] (None: ray i, one row per
+    ray) of the flattened batch; grad_loc Float32[h,3] and grad_uv Float32[h,2] are the incoming gradients (None: 0).
+    Each row recomputes its hit with the Moeller-Trumbore sequence of DESIGN.md §4.10 from `vertices` and `faces`;
+    the rows of one ray must be contiguous.  A row with no triangle, a degenerate triangle or a non-finite value
+    gives 0.  Deterministic to the bit: per-ray sums in row order, vertex sums through the sort and fixed tree of
+    distance_grad.  `workspace_bytes` bounds the workspace (default: one window for all rows); a smaller one runs
+    the rows as several windows, whose vertex sums are added in window order."""
+    tensor_input_check(origins, dirs, vertices)
+    rd, batch = make_ray_desc(origins, dirs)
+    dev = origins.device
+    h = tri.shape[0] if tri.dim() == 1 else -1
+    if ray_idx is None and h != rd.nray:
+        raise ValueError(f"tri must have one row per ray ({rd.nray}) without ray_idx, got {tuple(tri.shape)}")
+    for name, t, shape, dt in (("tri", tri, (h,), torch.int32), ("grad_loc", grad_loc, (h, 3), torch.float32),
+                               ("grad_uv", grad_uv, (h, 2), torch.float32), ("ray_idx", ray_idx, (h,), torch.int32)):
+        if t is not None and (tuple(t.shape) != shape or t.dtype != dt or t.device != dev):
+            raise ValueError(f"{name} must be {dt} {shape} on {dev}, got {t.dtype} {tuple(t.shape)} on {t.device}")
+    if vertices.dim() != 2 or vertices.shape[1] != 3 or vertices.device != dev:
+        raise ValueError("vertices must be float32 [n, 3] on the rays' device")
+    if faces.dtype != torch.int32 or faces.dim() != 2 or faces.shape[1] != 3 or faces.device != dev:
+        raise ValueError("faces must be int32 [f, 3] on the rays' device")
+    tri, grad_loc, grad_uv, ray_idx, vertices, faces = (None if t is None else t.contiguous() for t in
+                                                        (tri, grad_loc, grad_uv, ray_idx, vertices, faces))
+    n_verts = vertices.shape[0]
+    with _on_device(dev):
+        go = torch.empty((*batch, 3), dtype=torch.float32, device=dev) if origins_grad else None
+        gd = torch.empty((*batch, 3), dtype=torch.float32, device=dev) if directions_grad else None
+        gv = torch.empty((n_verts, 3), dtype=torch.float32, device=dev) if vertices_grad else None
+        wb = 0
+        if gv is not None:
+            wb = ray_grad_workspace_bytes(h, n_verts) if workspace_bytes is None else int(workspace_bytes)
+        ws = torch.empty(max(wb, 256), dtype=torch.uint8, device=dev) if gv is not None else None
+        _check(get_module().rt_ray_grad(C.byref(rd), C.byref(trace_opts()), h, _ptr(ray_idx), _ptr(tri), _ptr(grad_loc),
+                                        _ptr(grad_uv), _ptr(vertices), n_verts, _ptr(faces), faces.shape[0], _ptr(go),
+                                        _ptr(gd), _ptr(gv), _ptr(ws), wb, _stream(dev)), "rt_ray_grad")
+    return go, gd, gv
 
 
 def edge_counts(accel_structure) -> tuple[int, int, int]:

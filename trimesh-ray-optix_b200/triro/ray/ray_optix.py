@@ -92,7 +92,20 @@ class RayMeshIntersector:
         stream_compaction=False -> (hit[*b], front[*b], tri_idx[*b], loc[*b,3], uv[*b,2])
         stream_compaction=True  -> (hit[*b], front[h], ray_idx[h], tri_idx[h], loc[h,3], uv[h,2])
         with ray_idx the flattened row-major ray index in ascending order (int32).
+
+        `loc` and `uv` are differentiable with respect to `origins`, `directions` and `mesh_vertices` (the tensor
+        made from what was last given to the constructor, `update_raw` or `refit`, so gradients reach the caller's
+        tensor): the gradient of the hit inside the visible triangle, recomputed from the vertices as of this call
+        (DESIGN.md §4.10).  Visibility changes contribute nothing: a silhouette, an occlusion boundary or a hit that
+        would move to another triangle has no gradient (no edge sampling).  Misses and degenerate triangles give 0.
+        `hit`, `front`, `tri_idx` and `ray_idx` are not differentiable.  `interpolate(attr, tri_idx, uv)` is
+        differentiable through `uv`.  The BVH does not follow the vertices: call `refit(vertices)` after each
+        optimiser step.  Nothing of this runs unless grad mode is on and one of the three requires grad; the
+        gradients are deterministic to the bit.
         """
+        if self._tracks_grad(origins, directions):
+            return _ClosestHitFn.apply(origins, directions, self.mesh_vertices, self.mesh_faces, self.as_wrapper,
+                                       stream_compaction)
         hit, front, tri_idx, loc, uv = hops.intersects_closest(self.as_wrapper, origins, directions)
         if stream_compaction:
             front_c, ray_idx, tri_c, loc_c, uv_c = hops.compact_closest(hit, front, tri_idx, loc, uv)
@@ -103,7 +116,8 @@ class RayMeshIntersector:
                                    stream_compaction: bool = False):
         """Extension (SURVEY §8f): `intersects_closest` for the pinhole camera of the reference's benchmark
         (`gen_rays`, test/performance_test.py:10-20) with the rays generated inside the kernel.  Same tuples as
-        `intersects_closest`, batch shape [height, width]."""
+        `intersects_closest`, batch shape [height, width].  Not differentiable: the rays are made inside the kernel;
+        pass explicit rays to `intersects_closest` for gradients."""
         hit, front, tri_idx, loc, uv = hops.intersects_closest_pinhole(self.as_wrapper, cam_mat, cam_origin, width, height, focal)
         if stream_compaction:
             front_c, ray_idx, tri_c, loc_c, uv_c = hops.compact_closest(hit, front, tri_idx, loc, uv)
@@ -119,7 +133,13 @@ class RayMeshIntersector:
 
     def intersects_location(self, origins: torch.Tensor, directions: torch.Tensor
                             ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
-        """(loc[h,3], ray_idx[h], tri_idx[h]) for every hit, at most 8 per ray (reference :157-164)."""
+        """(loc[h,3], ray_idx[h], tri_idx[h]) for every hit, at most 8 per ray (reference :157-164).  `loc` is
+        differentiable like `intersects_closest`'s, each hit inside its own triangle.  The gradients are a function
+        of the rows: a ray's hits come in traversal order, which may differ between runs, and a different order sums
+        the ray's and the vertices' terms in a different order."""
+        if self._tracks_grad(origins, directions):
+            return _AllHitsFn.apply(origins, directions, self.mesh_vertices, self.mesh_faces, self.as_wrapper,
+                                    getattr(self, "max_hits", hops.MAX_ANYHIT_SIZE))
         return hops.intersects_location(self.as_wrapper, origins, directions, getattr(self, "max_hits", hops.MAX_ANYHIT_SIZE))
 
     def intersects_count(self, origins: torch.Tensor, directions: torch.Tensor) -> torch.Tensor:
@@ -128,7 +148,14 @@ class RayMeshIntersector:
 
     def intersects_id(self, origins: torch.Tensor, directions: torch.Tensor, return_locations: bool = False,
                       multiple_hits: bool = True):
-        """(tri_idx[h], ray_idx[h][, loc[h,3]]) (reference :191-223)."""
+        """(tri_idx[h], ray_idx[h][, loc[h,3]]) (reference :191-223).  `loc` is differentiable like
+        `intersects_closest`'s."""
+        if return_locations and self._tracks_grad(origins, directions):
+            if multiple_hits:
+                loc, ray_idx, tri_idx = self.intersects_location(origins, directions)
+                return tri_idx, ray_idx, loc
+            _, _, ray_idx, tri_c, loc_c, _ = self.intersects_closest(origins, directions, stream_compaction=True)
+            return tri_c, ray_idx, loc_c
         if multiple_hits:
             loc, ray_idx, tri_idx = hops.intersects_location(self.as_wrapper, origins, directions,
                                                              getattr(self, "max_hits", hops.MAX_ANYHIT_SIZE))
@@ -164,8 +191,8 @@ class RayMeshIntersector:
             return closest, distance, tri, uv
         return closest, distance, tri
 
-    def _tracks_grad(self, points: torch.Tensor) -> bool:
-        return torch.is_grad_enabled() and (points.requires_grad or self.mesh_vertices.requires_grad)
+    def _tracks_grad(self, *tensors: torch.Tensor) -> bool:
+        return torch.is_grad_enabled() and (self.mesh_vertices.requires_grad or any(t.requires_grad for t in tensors))
 
     def signed_distance(self, points: torch.Tensor, sign: str = "contains") -> torch.Tensor:
         """Float32[*b] — distance to the surface, positive inside and negative outside (trimesh.proximity.signed_distance).
@@ -309,6 +336,54 @@ class _PseudonormalSDFFn(torch.autograd.Function):
     @once_differentiable
     def backward(ctx, grad_sd):
         return (*_distance_backward(ctx, grad_sd), None)
+
+
+def _hit_backward(ctx, grad_loc, grad_uv):
+    origins, dirs, vertices, faces, tri, ray_idx = ctx.saved_tensors
+    h = tri.numel()
+    go, gd, gv = hops.ray_grad(origins.detach(), dirs.detach(), tri.reshape(h), grad_loc.reshape(h, 3),
+                               None if grad_uv is None else grad_uv.reshape(h, 2), vertices.detach(), faces,
+                               ray_idx=ray_idx, origins_grad=ctx.needs_input_grad[0],
+                               directions_grad=ctx.needs_input_grad[1], vertices_grad=ctx.needs_input_grad[2])
+    return go, gd, gv
+
+
+class _ClosestHitFn(torch.autograd.Function):
+    """intersects_closest with differentiable loc and uv (DESIGN.md §4.10).  `vertices` and `faces` are the mesh as of
+    the forward, saved for the backward (refit and update_raw replace the intersector's tensors)."""
+
+    @staticmethod
+    def forward(ctx, origins, dirs, vertices, faces, wrapper, compaction):
+        hit, front, tri, loc, uv = hops.intersects_closest(wrapper, origins.detach(), dirs.detach())
+        ray_idx = None
+        if compaction:
+            front, ray_idx, tri, loc, uv = hops.compact_closest(hit, front, tri, loc, uv)
+        ctx.mark_non_differentiable(*(t for t in (hit, front, ray_idx, tri) if t is not None))
+        ctx.save_for_backward(origins, dirs, vertices, faces, tri, ray_idx)
+        if compaction:
+            return hit, front, ray_idx, tri, loc, uv
+        return hit, front, tri, loc, uv
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, *grads):
+        return (*_hit_backward(ctx, grads[-2], grads[-1]), None, None, None)
+
+
+class _AllHitsFn(torch.autograd.Function):
+    """intersects_location with a differentiable loc (DESIGN.md §4.10), the mesh saved as for _ClosestHitFn."""
+
+    @staticmethod
+    def forward(ctx, origins, dirs, vertices, faces, wrapper, max_hits):
+        loc, ray_idx, tri = hops.intersects_location(wrapper, origins.detach(), dirs.detach(), max_hits)
+        ctx.mark_non_differentiable(ray_idx, tri)
+        ctx.save_for_backward(origins, dirs, vertices, faces, tri, ray_idx)
+        return loc, ray_idx, tri
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_loc, grad_ray_idx, grad_tri):
+        return (*_hit_backward(ctx, grad_loc, None), None, None, None)
 
 
 class OptixAccelStructureWrapper:
