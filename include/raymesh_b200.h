@@ -388,6 +388,41 @@ int rt_ray_grad(const rt_ray_desc* rays, const rt_trace_opts* opts, int64_t n_ro
                 const int32_t* faces, int64_t n_faces, float* grad_origins, float* grad_directions, float* grad_vertices,
                 void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- Instanced scenes (DESIGN.md §4.11; the reference's OptiX instance acceleration structures were never exposed):
+ *      M meshes (BVH8 blobs from rt_bvh_build) and I instances, instance i = (mesh m_i, affine object->world transform
+ *      (A_i | b_i) as a row-major binary32 3x4).  The world ray (o, d) meets instance i as o' = A_i^-1 (o - b_i),
+ *      d' = A_i^-1 d, with the same t.
+ *
+ *      rt_scene_prepare_sizes: bytes of the scene table (256-byte aligned device memory) for M meshes and I instances.
+ *      rt_scene_prepare: `blobs` (HOST array of M device addresses, each a blob of the current device), `inst_mesh`
+ *      (HOST int32 [I]) and `transforms` (HOST f32 [I,3,4]) are checked on the host: a mesh index outside [0, M), a
+ *      non-finite transform, det(A) = 0 in binary64, or an inverse that overflows binary32 -> RT_ERR_INVALID, and
+ *      nothing is written.  Then one kernel reads each mesh's header box from the device, computes A^-1 and the
+ *      object-space offset -A^-1 b in binary64, rounds them to binary32 once, and writes the instance table plus the
+ *      top-level geometry: tlas_vertices f32 [2I,3] = the padded world boxes (lo_i, hi_i), tlas_faces i32 [I,3] =
+ *      (2i, 2i+1, 2i).  Build the top-level tree from those with rt_bvh_build (its records' prim is the instance).  An
+ *      instance of a mesh without triangles gets a point box and is never entered.  Asynchronous on `stream`; the
+ *      host arrays may be released when it returns.  Rebuilding or re-fitting a member blob makes the table stale:
+ *      prepare again.
+ *
+ *      rt_scene_trace: one query for the batch/window (rays, opts: tmax, ray_first / ray_count) against the table and
+ *      the top-level blob.  mode RT_SCENE_CLOSEST: the hit minimising (t, inst, prim) over every instance in
+ *      (0, tmax); hit u8, front u8 (object-space front face XOR det(A) < 0), inst_idx i32, tri_idx i32 (row of the
+ *      instance's mesh faces), loc f32x3 (the world point A loc_obj + b), uv f32x2 (object-space weights of v0, v1);
+ *      a miss gives inst_idx = tri_idx = -1 and 0 elsewhere.  RT_SCENE_ANY: hit.  RT_SCENE_COUNT: count i32 = the sum
+ *      over instances of the crossings in (0, tmax).  Outputs the mode does not write may be NULL.  One identity
+ *      instance gives the bits of rt_trace_closest / _any / _count on its mesh. */
+#define RT_SCENE_CLOSEST 0
+#define RT_SCENE_ANY 1
+#define RT_SCENE_COUNT 2
+int rt_scene_prepare_sizes(int64_t n_meshes, int64_t n_inst, size_t* table_bytes);
+int rt_scene_prepare(int64_t n_meshes, const void* const* blobs, int64_t n_inst, const int32_t* inst_mesh,
+                     const float* transforms, void* table, size_t table_bytes, float* tlas_vertices, int32_t* tlas_faces,
+                     void* stream);
+int rt_scene_trace(const void* table, const void* tlas_blob, const rt_ray_desc* rays, const rt_trace_opts* opts, int mode,
+                   uint8_t* hit, uint8_t* front, int32_t* inst_idx, int32_t* tri_idx, float* loc, float* uv, int32_t* count,
+                   void* stream);
+
 /* ---- Host-buffer entry points (end-to-end path): rays and results live in (pinned) HOST memory.
  *      Copies ray chunks H2D, traces and copies results D2H on internal streams, overlapping
  *      the three; `dev_work` is caller-provided device memory of rt_host_closest_sizes() bytes.

@@ -112,6 +112,9 @@ def _declare(lib):
         "rt_distance_grad": (ci, [prd, pto, vp, vp, vp, vp, vp, vp, i64, i64, vp, vp, vp, sz, vp]),
         "rt_ray_grad_sizes": (ci, [i64, i64, psz]),
         "rt_ray_grad": (ci, [prd, pto, i64, vp, vp, vp, vp, vp, i64, vp, i64, vp, vp, vp, vp, sz, vp]),
+        "rt_scene_prepare_sizes": (ci, [i64, i64, psz]),
+        "rt_scene_prepare": (ci, [i64, vp, i64, vp, vp, vp, sz, vp, vp, vp]),
+        "rt_scene_trace": (ci, [vp, vp, prd, pto, ci, vp, vp, vp, vp, vp, vp, vp, vp]),
         "rt_host_closest_sizes": (ci, [i64, psz]),
         "rt_host_trace_closest": (ci, [vp, i64, vp, ci, vp, pto, vp, vp, vp, vp, vp, vp, sz]),
         "rt_host_trace_closest_compact": (ci, [vp, i64, vp, ci, vp, pto, vp, vp, vp, vp, vp, vp, C.POINTER(C.c_int64), vp, sz]),
@@ -349,6 +352,7 @@ class AccelStructure:
         self.build_ms: float | None = None
         self.winding_moments: torch.Tensor | None = None   # ops.winding_moments() cache, dropped with the blob's contents
         self.pseudo_normals: tuple | None = None           # ops.pseudo_normals() cache, likewise
+        self.generation: int = 0                           # counts build() and refit(): scenes detect stale members
 
     def build(self, vertices: torch.Tensor, faces: torch.Tensor, timing: bool = False):
         lib = get_module()
@@ -390,6 +394,7 @@ class AccelStructure:
         self.header = hdr
         self.winding_moments = None
         self.pseudo_normals = None
+        self.generation += 1
         return self
 
     def refit(self, vertices: torch.Tensor, faces: torch.Tensor):
@@ -417,6 +422,7 @@ class AccelStructure:
             self.header = parse_header(self.blob[:BLOB_HEADER_BYTES].cpu().numpy().tobytes())
         self.winding_moments = None
         self.pseudo_normals = None
+        self.generation += 1
         return self
 
     def save(self, path: str):
@@ -1132,3 +1138,66 @@ def sort_pairs_u64(keys: torch.Tensor, vals: torch.Tensor):
         ws = torch.empty(max(wb.value, 256), dtype=torch.uint8, device=dev)
         _check(lib.rt_sort_pairs_u64(_ptr(keys), _ptr(vals), n, _ptr(ws), ws.numel(), _stream(dev)), "rt_sort_pairs_u64")
     return keys, vals
+
+
+# ------------------------------------------------------------------ instanced scenes (DESIGN.md §4.11)
+SCENE_CLOSEST, SCENE_ANY, SCENE_COUNT = 0, 1, 2
+
+
+def scene_prepare(blobs: list, inst_mesh: torch.Tensor, transforms: torch.Tensor, device) -> tuple[torch.Tensor, AccelStructure]:
+    """rt_scene_prepare + rt_bvh_build: (scene table, top-level AccelStructure) for the member blobs (device uint8
+    tensors), the host int32 [I] mesh indices and the host float32 [I,3,4] object->world transforms.  Raises ValueError
+    for a mesh index out of range, a non-finite or singular transform, or a blob on another device."""
+    lib = get_module()
+    dev = torch.device(device)
+    for b in blobs:
+        if not b.is_cuda or b.device != dev:
+            raise ValueError(f"every mesh of a scene must live on {dev} (one is on {b.device})")
+    inst_mesh = inst_mesh.to(torch.int32).contiguous()
+    transforms = transforms.to(torch.float32).contiguous()
+    n_inst, n_meshes = inst_mesh.numel(), len(blobs)
+    tb = C.c_size_t()
+    _check(lib.rt_scene_prepare_sizes(n_meshes, n_inst, C.byref(tb)), "rt_scene_prepare_sizes")
+    addrs = (C.c_void_p * max(n_meshes, 1))(*[b.data_ptr() for b in blobs])
+    with torch.cuda.device(dev):
+        table = torch.empty(tb.value, dtype=torch.uint8, device=dev)
+        tv = torch.empty((2 * n_inst, 3), dtype=torch.float32, device=dev)
+        tf = torch.empty((n_inst, 3), dtype=torch.int32, device=dev)
+        _check(lib.rt_scene_prepare(n_meshes, addrs, n_inst, C.c_void_p(inst_mesh.data_ptr()),
+                                    C.c_void_p(transforms.data_ptr()), _ptr(table), table.numel(), _ptr(tv), _ptr(tf),
+                                    _stream(dev)), "rt_scene_prepare")
+        tlas = AccelStructure().build(tv, tf)
+    return table, tlas
+
+
+def scene_trace(table: torch.Tensor, tlas: AccelStructure, origins: torch.Tensor, dirs: torch.Tensor, mode: int,
+                tmax: float = TMAX_DEFAULT, ray_first: int = 0, ray_count: int = -1):
+    """rt_scene_trace.  closest: (hit, front, inst, tri, loc, uv); any: hit; count: count — shaped like the batch, or
+    1-D over the window [ray_first, ray_first + ray_count)."""
+    tensor_input_check(origins, dirs)
+    if table.device != origins.device:
+        raise ValueError(f"the scene lives on {table.device} but the rays are on {origins.device}")
+    rd, batch = make_ray_desc(origins, dirs)
+    if ray_first != 0 or ray_count >= 0:
+        batch = (_window(rd.nray, ray_first, ray_count),)
+    dev = origins.device
+    opts = TraceOpts()
+    opts.tmax = float(tmax)
+    opts.ray_first, opts.ray_count = int(ray_first), max(int(ray_count), 0)
+    with _on_device(dev):
+        e = lambda shape, dt: torch.empty(shape, dtype=dt, device=dev)   # noqa: E731
+        if mode == SCENE_CLOSEST:
+            out = (e(batch, torch.bool), e(batch, torch.bool), e(batch, torch.int32), e(batch, torch.int32),
+                   e((*batch, 3), torch.float32), e((*batch, 2), torch.float32))
+            ptrs = (out[0], out[1], out[2], out[3], out[4], out[5], None)
+        elif mode == SCENE_ANY:
+            out = e(batch, torch.bool)
+            ptrs = (out, None, None, None, None, None, None)
+        else:
+            out = e(batch, torch.int32)
+            ptrs = (None, None, None, None, None, None, out)
+        n = ptrs[0].numel() if ptrs[0] is not None else ptrs[6].numel()
+        if n > 0:
+            _check(get_module().rt_scene_trace(_ptr(table), _ptr(tlas.blob), C.byref(rd), C.byref(opts), int(mode),
+                                               *[_ptr(p) for p in ptrs], _stream(dev)), "rt_scene_trace")
+    return out
