@@ -423,6 +423,39 @@ int rt_scene_trace(const void* table, const void* tlas_blob, const rt_ray_desc* 
                    uint8_t* hit, uint8_t* front, int32_t* inst_idx, int32_t* tri_idx, float* loc, float* uv, int32_t* count,
                    void* stream);
 
+/* ---- Point queries on instanced scenes (DESIGN.md §4.12), on a table and top-level blob from rt_scene_prepare.
+ *      The world triangle t of instance i has the vertices W_k = affine_row(A_i row, b_i (0 as -0), v_k) in binary32,
+ *      the sequence rt_scene_trace uses for loc.
+ *
+ *      rt_scene_point_sizes: bytes of the side array (16-byte aligned device memory) for I instances.
+ *      rt_scene_point_prepare: one kernel writes the side array (per instance a lower bound on the smallest singular
+ *      value of A_i and the margins of the instance walk's bound) from the table and its meshes' header boxes.  A
+ *      function of those alone; prepare again after rt_scene_prepare.  Asynchronous on `stream`.
+ *
+ *      rt_scene_closest_point: for each point of the batch/window (points, opts: ray_first / ray_count) the (inst, prim)
+ *      minimising the key (d2, inst, prim) over every non-empty instance and triangle with d2 <= fl(max_distance^2),
+ *      d2 = the single-mesh point/triangle distance of rt_closest_point on the world triangle.  closest f32x3 (world),
+ *      distance f32 = sqrt(d2), inst_idx i32, tri_idx i32 (row of the instance's mesh faces), uv f32x2 (weights of
+ *      v0, v1).  A point with none (nothing in reach, non-finite point, empty scene): inst = tri = -1, distance +inf,
+ *      closest and uv 0.  max_distance must be >= 0 or +inf (NaN or negative -> RT_ERR_INVALID).  The result equals
+ *      rt_closest_point on the mesh of every instance's affine_row world vertices, faces in instance order, bit for bit.
+ *
+ *      rt_scene_signed_distance: the same walk with max_distance +inf, then the pseudo-normal sign of rt_signed_distance
+ *      with the normal carried to world space as A^-T n (from the stored binary32 inverse): +d when (p - c) . n_w < 0,
+ *      -d otherwise, +0 for d = 0, -inf for a point without answer.  `normals_table`: DEVICE array of M addresses, the
+ *      rt_pseudonormals rows of each mesh (any 16-byte aligned address for a mesh without triangles); NULL or misaligned
+ *      -> RT_ERR_INVALID.  closest, inst_idx, tri_idx and uv are all NULL or all set (then written as by
+ *      rt_scene_closest_point).  The sign is that of inside/outside when every mesh is closed, manifold and consistently
+ *      oriented, every A_i is a similarity (mirrors allowed) and the instances do not overlap. */
+int rt_scene_point_sizes(int64_t n_inst, size_t* side_bytes);
+int rt_scene_point_prepare(const void* table, int64_t n_inst, void* side, size_t side_bytes, void* stream);
+int rt_scene_closest_point(const void* table, const void* tlas_blob, const void* side, const rt_ray_desc* points,
+                           const rt_trace_opts* opts, float max_distance, float* closest, float* distance, int32_t* inst_idx,
+                           int32_t* tri_idx, float* uv, void* stream);
+int rt_scene_signed_distance(const void* table, const void* tlas_blob, const void* side, const void* normals_table,
+                             const rt_ray_desc* points, const rt_trace_opts* opts, float* signed_distance, float* closest,
+                             int32_t* inst_idx, int32_t* tri_idx, float* uv, void* stream);
+
 /* ---- Host-buffer entry points (end-to-end path): rays and results live in (pinned) HOST memory.
  *      Copies ray chunks H2D, traces and copies results D2H on internal streams, overlapping
  *      the three; `dev_work` is caller-provided device memory of rt_host_closest_sizes() bytes.

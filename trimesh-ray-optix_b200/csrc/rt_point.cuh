@@ -196,16 +196,31 @@ RT_HD void point_init(PointTrav& t, float x, float y, float z, float max_d2) {
 // >= +0, so the bit pattern orders like the value, and clearing 3 bits only lowers it (still a lower bound).
 RT_HD void cswap_lo(uint32_t& a, uint32_t& b) { const uint32_t lo = a < b ? a : b, hi = a < b ? b : a; a = lo; b = hi; }
 
+// The space a walk runs in: how a node's slot bounds are formed and how a leaf record is tested.  MeshSpace is the
+// single mesh (the point and the triangles in one space); the instanced scene (rt_scene.cuh) adds a world-space walk of
+// one instance's tree and the top-level walk whose records are instances.  leaf() may lower t.best and sets the answer.
+struct MeshSpace {
+    RT_HD void bounds(const PointTrav& t, const U4& n0, const U4& n2, const U4& n3, const U4& n4, float lb[8]) const {
+        slot_lower_bounds(t.x, t.y, t.z, n0, n2, n3, n4, lb);
+    }
+    RT_HD void leaf(PointTrav& t, uint32_t rec, const U4& a, const U4& b, const U4& c) const {
+        const PointHit h = point_tri(t.x, t.y, t.z, as_float(a.x), as_float(a.y), as_float(a.z), as_float(b.x),
+                                     as_float(b.y), as_float(b.z), as_float(c.x), as_float(c.y), as_float(c.z));
+        const int32_t prim = (int32_t)a.w;
+        if (h.d2 < t.best || (h.d2 == t.best && prim < t.prim)) { t.best = h.d2; t.prim = prim; t.slot = rec; }
+    }
+};
+
 // One node visit or one pop; returns true when the point is finished.  Visitor: count_node(), count_tri().
-template <class S, class StackT>
+template <class S, class StackT, class Space>
 RT_HD bool point_step(const uint8_t* __restrict__ nodes, const uint8_t* __restrict__ tris, PointTrav& t, S& st,
-                      StackT& stack) {
+                      StackT& stack, Space& space) {
     if (t.node != kNoNode) {
         const uint8_t* np = nodes + (size_t)t.node * 80u;
         const U4 n0 = ldg128(np), n1 = ldg128(np + 16), n2 = ldg128(np + 32), n3 = ldg128(np + 48), n4 = ldg128(np + 64);
         st.count_node();
         float lb[8];
-        slot_lower_bounds(t.x, t.y, t.z, n0, n2, n3, n4, lb);
+        space.bounds(t, n0, n2, n3, n4, lb);
         const uint32_t imask = n0.w >> 24, tbase = n1.y, tmask = n1.z;
         // leaves first: their triangles can only lower `best`, which prunes the inner slots below
         for (int s = 0; s < 8; ++s) {
@@ -217,10 +232,7 @@ RT_HD bool point_step(const uint8_t* __restrict__ nodes, const uint8_t* __restri
                 const uint8_t* tp = tris + (size_t)rec * 48u;
                 const U4 a = ldg128(tp), b = ldg128(tp + 16), c = ldg128(tp + 32);
                 st.count_tri();
-                const PointHit h = point_tri(t.x, t.y, t.z, as_float(a.x), as_float(a.y), as_float(a.z), as_float(b.x),
-                                             as_float(b.y), as_float(b.z), as_float(c.x), as_float(c.y), as_float(c.z));
-                const int32_t prim = (int32_t)a.w;
-                if (h.d2 < t.best || (h.d2 == t.best && prim < t.prim)) { t.best = h.d2; t.prim = prim; t.slot = rec; }
+                space.leaf(t, rec, a, b, c);
             }
         }
         // inner children within reach, nearest first (sorting network on 8 keys; absent ones sort last as ~0)
@@ -273,6 +285,13 @@ RT_HD bool point_step(const uint8_t* __restrict__ nodes, const uint8_t* __restri
         return false;
     }
     return true;
+}
+
+template <class S, class StackT>
+RT_HD bool point_step(const uint8_t* __restrict__ nodes, const uint8_t* __restrict__ tris, PointTrav& t, S& st,
+                      StackT& stack) {
+    MeshSpace space;
+    return point_step(nodes, tris, t, st, stack, space);
 }
 
 }  // namespace rt

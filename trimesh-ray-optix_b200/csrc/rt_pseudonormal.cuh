@@ -154,15 +154,20 @@ RT_HD uint32_t edge_class(const EdgeRun& e) {   // 0 boundary, 1 non-manifold, 2
 // ------------------------------------------------------------------ the sign
 // +d when (p - c) . n < 0 (inside), -d otherwise; an exact d = 0 gives +0.  n is the pseudo-normal of the region of c:
 // the unit face normal for the face, the record's row for a vertex or an edge.
+RT_HD void region_normal(const uint8_t* normals, uint32_t rec, uint32_t region, const float v[9], float& nx, float& ny,
+                         float& nz) {
+    if (region == kRegionFace) {
+        face_unit_normal(v, nx, ny, nz);
+    } else {
+        const U4 q = ldg128(normals + (size_t)rec * kPnRowBytes + (size_t)(region - 1u) * 16u);
+        nx = as_float(q.x); ny = as_float(q.y); nz = as_float(q.z);
+    }
+}
+
 RT_HD float pseudonormal_sign(const uint8_t* normals, uint32_t rec, const PointHit& h, float px, float py, float pz,
                               const float v[9], float d) {
     float nx, ny, nz;
-    if (h.region == kRegionFace) {
-        face_unit_normal(v, nx, ny, nz);
-    } else {
-        const U4 q = ldg128(normals + (size_t)rec * kPnRowBytes + (size_t)(h.region - 1u) * 16u);
-        nx = as_float(q.x); ny = as_float(q.y); nz = as_float(q.z);
-    }
+    region_normal(normals, rec, h.region, v, nx, ny, nz);
     const float s = dot3f(fsub(px, h.cx), fsub(py, h.cy), fsub(pz, h.cz), nx, ny, nz);
     return (s < 0.0f || d == 0.0f) ? d : -d;
 }

@@ -47,14 +47,6 @@ struct SceneStack {
     __device__ __forceinline__ void pop(int sp, uint32_t& x, uint32_t& y) { const uint2 v = e[sp]; x = v.x; y = v.y; }
 };
 
-__device__ __forceinline__ int64_t scene_offset(const int64_t shape[4], const int64_t stride[4], int64_t r) {
-    const int64_t i2 = r % shape[2];
-    const int64_t q = r / shape[2];
-    const int64_t i1 = q % shape[1];
-    const int64_t i0 = q / shape[1];
-    return i0 * stride[0] + i1 * stride[1] + i2 * stride[2];
-}
-
 template <int MODE>   // 0 closest, 1 any, 2 count
 __global__ void __launch_bounds__(kSceneThreads) k_scene_trace(const __grid_constant__ SceneParams p) {
     const int64_t i = (int64_t)blockIdx.x * kSceneThreads + threadIdx.x;

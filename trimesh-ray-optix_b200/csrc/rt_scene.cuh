@@ -6,16 +6,18 @@
 // (lo_i, hi_i, lo_i) whose box is exactly the padded world box [lo_i, hi_i], and its record's prim is i.
 #pragma once
 #include "../../include/raymesh_b200.h"
-#include "rt_traverse.cuh"
+#include "rt_pseudonormal.cuh"
 
 namespace rt {
 
 #if defined(__CUDA_ARCH__)
 RT_HD double dadd(double a, double b) { return __dadd_rn(a, b); }
 RT_HD double ddiv(double a, double b) { return __ddiv_rn(a, b); }
+RT_HD double dsqrt(double a) { return __dsqrt_rn(a); }
 #else
 RT_HD double dadd(double a, double b) { return a + b; }
 RT_HD double ddiv(double a, double b) { return a / b; }
+RT_HD double dsqrt(double a) { return sqrt(a); }
 #endif
 
 // Scene table (one device buffer): [SceneHeader][instance records, 128 B each][BLAS blob addresses, 8 B each].
@@ -180,6 +182,15 @@ RT_HD bool box_hit(const Ray& r, const float lo[3], const float hi[3], float tma
     return tn <= tf;
 }
 
+// Element offset of row r of a [*b, 3] batch flattened to shape[0..2] with element strides stride[0..2].
+RT_HD int64_t scene_offset(const int64_t shape[4], const int64_t stride[4], int64_t r) {
+    const int64_t i2 = r % shape[2];
+    const int64_t q = r / shape[2];
+    const int64_t i1 = q % shape[1];
+    const int64_t i0 = q / shape[1];
+    return i0 * stride[0] + i1 * stride[1] + i2 * stride[2];
+}
+
 struct SceneView {
     const SceneInst* inst;
     const uint64_t* blobs;      // BLAS blob address of each mesh
@@ -330,6 +341,245 @@ RT_HD SceneHitOut scene_hit_attr(const SceneView& sv, int32_t inst, uint32_t slo
     out.uv[0] = at.uv0;
     out.uv[1] = at.uv1;
     return out;
+}
+
+// ---------------------------------------------------------------- point queries (DESIGN.md §4.12)
+// Closest point and pseudo-normal signed distance over the instances: the minimum of the key (d2, inst, prim) over
+// every non-empty instance and triangle with d2 <= max_d2, d2 = point_tri(p, W0, W1, W2).d2 of the WORLD triangle
+// Wk = affine_row(fwd row, zero_as_negative(b), vk).  That is exactly the key (d2, f) of the mesh flattened with the
+// same affine_row, faces concatenated in instance order, so the answer equals rt_closest_point on that mesh.
+
+// Side array of the point queries, one entry per instance (rt_scene_point_prepare): sigma <= the smallest singular
+// value of A, and the world margin mu(p) = alpha + beta |p|inf of the instance walk's bound (scene_world_bound).
+struct alignas(16) ScenePointSide { float sigma, alpha, beta, reserved; };
+static_assert(sizeof(ScenePointSide) == 16, "ScenePointSide must be 16 bytes");
+
+// A rigorous lower bound on the smallest eigenvalue of the symmetric 3x3 matrix g (binary64, row-major): eight cyclic
+// Jacobi sweeps, then Gershgorin's lower end on the rotated matrix, less a Weyl margin of 2^-40 * `scale` for the
+// rounding of the rotations (backward stable: each is an exact orthogonal similarity of a matrix within a few
+// 2^-53 ||g|| of the computed one).  `scale` >= ||g||F.  Every operation is fixed, so the host repeats the bits.
+RT_HD double sym3_min_eig_lower(const double g_in[9], double scale) {
+    double g[9];
+    for (int k = 0; k < 9; ++k) g[k] = g_in[k];
+    for (int sweep = 0; sweep < 8; ++sweep) {
+        for (int pr = 0; pr < 3; ++pr) {
+            const int p = pr == 2 ? 1 : 0, q = pr == 0 ? 1 : 2, r = 3 - p - q;
+            const double apq = g[3 * p + q];
+            if (apq == 0.0) continue;
+            const double theta = ddiv(dsub(g[3 * q + q], g[3 * p + p]), dmul(2.0, apq));
+            const double t0 = ddiv(1.0, dadd(fabs(theta), dsqrt(dadd(dmul(theta, theta), 1.0))));
+            const double t = theta < 0.0 ? -t0 : t0;
+            const double c = ddiv(1.0, dsqrt(dadd(dmul(t, t), 1.0)));
+            const double sn = dmul(t, c);
+            const double arp = g[3 * r + p], arq = g[3 * r + q];
+            g[3 * p + p] = dsub(g[3 * p + p], dmul(t, apq));
+            g[3 * q + q] = dadd(g[3 * q + q], dmul(t, apq));
+            g[3 * p + q] = g[3 * q + p] = 0.0;
+            g[3 * r + p] = g[3 * p + r] = dsub(dmul(c, arp), dmul(sn, arq));
+            g[3 * r + q] = g[3 * q + r] = dadd(dmul(sn, arp), dmul(c, arq));
+        }
+    }
+    double lo = INFINITY;
+    for (int k = 0; k < 3; ++k) {
+        const double off = dadd(fabs(g[3 * k + (k + 1) % 3]), fabs(g[3 * k + (k + 2) % 3]));
+        const double e = dsub(g[4 * k], off);
+        lo = e < lo ? e : lo;
+    }
+    return dsub(lo, dmul(9.094947017729282e-13, scale));   // 2^-40
+}
+
+// The side entry of one instance, from its record and its mesh's header box (binary64, rounded once).  With u = 2^-24,
+// M | c the stored inverse, E = A M - I and g = A c + b (both from binary32 values, so their binary64 residuals are
+// bounded below), S = ||b||inf + ||A||inf R as in prepare_instance:
+//   alpha = sigma 2^-21 ||c||inf + 1.75 ||g||inf + 2^-18 S,   beta = sigma 2^-21 ||M||inf + 1.75 ||E||inf,
+// each inflated by 2^-16 and rounded up; DESIGN.md §4.12 derives them.  An empty instance gets zeros (never read).
+RT_HD ScenePointSide prepare_point_side(const uint8_t* blob, const SceneInst& s) {
+    ScenePointSide out = {0.0f, 0.0f, 0.0f, 0.0f};
+    if (s.flags & kInstEmpty) return out;
+    const rt_blob_header* h = reinterpret_cast<const rt_blob_header*>(blob);
+    double R = 0.0;
+    for (int a = 0; a < 3; ++a) {
+        const double lo = fabs((double)h->aabb_lo[a]), hi = fabs((double)h->aabb_hi[a]);
+        const double m = lo > hi ? lo : hi;
+        R = m > R ? m : R;
+    }
+    double g[9], fro = 0.0, na = 0.0, nb = 0.0, nm = 0.0, nc = 0.0, ne = 0.0, ng = 0.0;
+    const double ulp53 = 1.1102230246251565e-16;   // 2^-53
+    for (int k = 0; k < 3; ++k) {
+        double ra = 0.0, rm = 0.0, re = 0.0;
+        for (int j = 0; j < 3; ++j) {
+            double gkj = 0.0, ekj = 0.0, abs_e = 0.0;
+            for (int l = 0; l < 3; ++l) {
+                gkj = dadd(gkj, dmul((double)s.fwd[4 * l + k], (double)s.fwd[4 * l + j]));
+                ekj = dadd(ekj, dmul((double)s.fwd[4 * k + l], (double)s.inv[4 * l + j]));
+                abs_e = dadd(abs_e, fabs(dmul((double)s.fwd[4 * k + l], (double)s.inv[4 * l + j])));
+            }
+            g[3 * k + j] = gkj;
+            ekj = dsub(ekj, k == j ? 1.0 : 0.0);
+            re = dadd(re, dadd(fabs(ekj), dmul(4.0 * ulp53, dadd(abs_e, 1.0))));
+            ra = dadd(ra, fabs((double)s.fwd[4 * k + j]));
+            rm = dadd(rm, fabs((double)s.inv[4 * k + j]));
+            fro = dadd(fro, dmul((double)s.fwd[4 * k + j], (double)s.fwd[4 * k + j]));
+        }
+        double gk = (double)s.fwd[4 * k + 3], abs_g = fabs((double)s.fwd[4 * k + 3]);
+        for (int l = 0; l < 3; ++l) {
+            gk = dadd(gk, dmul((double)s.fwd[4 * k + l], (double)s.inv[4 * l + 3]));
+            abs_g = dadd(abs_g, fabs(dmul((double)s.fwd[4 * k + l], (double)s.inv[4 * l + 3])));
+        }
+        const double gb = dadd(fabs(gk), dmul(4.0 * ulp53, abs_g));
+        na = ra > na ? ra : na;
+        nm = rm > nm ? rm : nm;
+        ne = re > ne ? re : ne;
+        ng = gb > ng ? gb : ng;
+        const double bk = fabs((double)s.fwd[4 * k + 3]), ck = fabs((double)s.inv[4 * k + 3]);
+        nb = bk > nb ? bk : nb;
+        nc = ck > nc ? ck : nc;
+    }
+    const double lam = sym3_min_eig_lower(g, fro);
+    const double sigma = lam > 0.0 ? dmul(dsqrt(lam), 1.0 - 3.552713678800501e-15) : 0.0;   // 1 - 2^-48
+    out.sigma = round_down(sigma);
+    const double sd = (double)out.sigma, k21 = 4.76837158203125e-07, k18 = 3.814697265625e-06, inf16 = 1.0 + 1.52587890625e-05;
+    const double S = dadd(nb, dmul(na, R));
+    const double alpha = dadd(dadd(dmul(dmul(sd, k21), nc), dmul(1.75, ng)), dmul(k18, S));
+    const double beta = dadd(dmul(dmul(sd, k21), nm), dmul(1.75, ne));
+    out.alpha = round_up(dmul(alpha, inf16));
+    out.beta = round_up(dmul(beta, inf16));
+    return out;
+}
+
+// Squared distance from (x, y, z) to the box [lo, hi], rounded so that it never exceeds the exact value times 1 - 5u
+// (the factor 1 - 2^-20 covers the roundings of the gaps and the sum): the top-level leaf bound.
+RT_HD float box_point_lower(float x, float y, float z, const float lo[3], const float hi[3]) {
+    const float gx = fmaxf(fmaxf(fsub(lo[0], x), fsub(x, hi[0])), 0.0f);
+    const float gy = fmaxf(fmaxf(fsub(lo[1], y), fsub(y, hi[1])), 0.0f);
+    const float gz = fmaxf(fmaxf(fsub(lo[2], z), fsub(z, hi[2])), 0.0f);
+    return fmul(dot3f(gx, gy, gz, gx, gy, gz), 0.999999046325684f);   // 1 - 2^-20
+}
+
+// World vertices of an object-space triangle record: Wk = affine_row(fwd row, zero_as_negative(b), vk).
+RT_HD void world_tri(const float fwd[12], const U4& a, const U4& b, const U4& c, float w[9]) {
+    const float v[9] = {as_float(a.x), as_float(a.y), as_float(a.z), as_float(b.x), as_float(b.y), as_float(b.z),
+                        as_float(c.x), as_float(c.y), as_float(c.z)};
+    for (int k = 0; k < 3; ++k) {
+        const float* m = fwd + 4 * k;
+        const float bk = zero_as_negative(m[3]);
+        for (int j = 0; j < 3; ++j) w[3 * j + k] = affine_row(m[0], m[1], m[2], bk, v[3 * j], v[3 * j + 1], v[3 * j + 2]);
+    }
+}
+
+// World lower bound of an instance-walk slot from its object-space bound lb = slot_lower_bounds(p'):
+// (sigma sqrt(lb) - mu)+^2 (1 - 2^-20) <= the d2 point_tri computes for every world triangle below the slot.
+RT_HD float scene_world_bound(float lb, float sigma, float mu) {
+    const float h = fmaxf(fsub(fmul(sigma, fsqrt(lb)), mu), 0.0f);
+    return fmul(fmul(h, h), 0.999999046325684f);
+}
+
+// The walk of one instance's own tree: slot bounds from the object point p' mapped to world bounds, leaves tested as
+// world triangles against the world point (t.x, t.y, t.z).
+struct InstanceSpace {
+    float fwd[12];
+    float ox, oy, oz;          // p' = affine_row(inv rows, p)
+    float sigma, mu;
+    RT_HD void bounds(const PointTrav& t, const U4& n0, const U4& n2, const U4& n3, const U4& n4, float lb[8]) const {
+        (void)t;
+        slot_lower_bounds(ox, oy, oz, n0, n2, n3, n4, lb);
+#pragma unroll
+        for (int s = 0; s < 8; ++s) lb[s] = scene_world_bound(lb[s], sigma, mu);
+    }
+    RT_HD void leaf(PointTrav& t, uint32_t rec, const U4& a, const U4& b, const U4& c) const {
+        float w[9];
+        world_tri(fwd, a, b, c, w);
+        const PointHit h = point_tri(t.x, t.y, t.z, w[0], w[1], w[2], w[3], w[4], w[5], w[6], w[7], w[8]);
+        const int32_t prim = (int32_t)a.w;
+        if (h.d2 < t.best || (h.d2 == t.best && prim < t.prim)) { t.best = h.d2; t.prim = prim; t.slot = rec; }
+    }
+};
+
+// Walks instance i with the world best t.best.  The seed extends the single-mesh tie rule to (d2, inst, prim): when
+// no instance has an answer yet or i precedes the best one an equal d2 wins (seed kNoPrim), otherwise it loses
+// (seed -1).  Returns the prim found, or the seed when nothing beat the best; lowers t.best and sets *slot on a find.
+template <class StackT>
+RT_HD int32_t scene_point_instance(const SceneView& sv, const ScenePointSide* side, int32_t i, int32_t best_inst,
+                                   PointTrav& t, uint32_t* slot, StackT& stack) {
+    const int32_t seed = (best_inst < 0 || i < best_inst) ? kNoPrim : -1;
+    const SceneInst& s = sv.inst[i];
+    if (s.flags & kInstEmpty) return seed;
+    const uint8_t* blob = reinterpret_cast<const uint8_t*>(sv.blobs[s.mesh]);
+    const rt_blob_header* h = reinterpret_cast<const rt_blob_header*>(blob);
+    InstanceSpace sp;
+    for (int k = 0; k < 12; ++k) sp.fwd[k] = s.fwd[k];
+    sp.ox = affine_row(s.inv[0], s.inv[1], s.inv[2], s.inv[3], t.x, t.y, t.z);
+    sp.oy = affine_row(s.inv[4], s.inv[5], s.inv[6], s.inv[7], t.x, t.y, t.z);
+    sp.oz = affine_row(s.inv[8], s.inv[9], s.inv[10], s.inv[11], t.x, t.y, t.z);
+    const ScenePointSide e = side[i];
+    const float pmax = fmaxf(fmaxf(fabsf(t.x), fabsf(t.y)), fabsf(t.z));
+    sp.sigma = e.sigma;
+    sp.mu = fadd(e.alpha, fmul(e.beta, pmax));
+    PointTrav it;
+    it.x = t.x; it.y = t.y; it.z = t.z; it.best = t.best; it.prim = seed; it.slot = 0u; it.node = 0u; it.sp = 0;
+    NoStats st;
+    while (!point_step(blob + h->nodes_offset, blob + h->tris_offset, it, st, stack, sp)) {}
+    if (it.prim != seed) { t.best = it.best; *slot = it.slot; }
+    return it.prim;
+}
+
+// The top-level walk: world slot bounds (the slot boxes contain the padded instance boxes), and a leaf record is an
+// instance, entered when the squared distance to its padded world box is within the best.
+template <class StackT>
+struct SceneTopSpace {
+    SceneView sv;
+    const ScenePointSide* side;
+    StackT* stack;
+    int32_t inst = -1, prim = -1;
+    uint32_t slot = 0;
+    RT_HD void bounds(const PointTrav& t, const U4& n0, const U4& n2, const U4& n3, const U4& n4, float lb[8]) const {
+        slot_lower_bounds(t.x, t.y, t.z, n0, n2, n3, n4, lb);
+    }
+    RT_HD void leaf(PointTrav& t, uint32_t rec, const U4& a, const U4& b, const U4& c) {
+        (void)rec; (void)c;
+        const float lo[3] = {as_float(a.x), as_float(a.y), as_float(a.z)};
+        const float hi[3] = {as_float(b.x), as_float(b.y), as_float(b.z)};
+        if (!(box_point_lower(t.x, t.y, t.z, lo, hi) <= t.best)) return;
+        visit(t, (int32_t)a.w);
+    }
+    RT_HD void visit(PointTrav& t, int32_t i) {
+        uint32_t sl = 0u;
+        const int32_t seed = (inst < 0 || i < inst) ? kNoPrim : -1;
+        const int32_t pr = scene_point_instance(sv, side, i, inst, t, &sl, *stack);
+        if (pr != seed) { inst = i; prim = pr; slot = sl; }
+    }
+};
+
+// Outputs of the answer (inst, slot) for the world point p: point_tri on the world triangle (c, d2, w0, w1, region)
+// and the object-space vertices v (for the face normal of the sign).
+RT_HD PointHit scene_point_attr(const SceneView& sv, int32_t inst, uint32_t slot, float px, float py, float pz, float v[9]) {
+    const SceneInst& s = sv.inst[inst];
+    const uint8_t* blob = reinterpret_cast<const uint8_t*>(sv.blobs[s.mesh]);
+    const rt_blob_header* h = reinterpret_cast<const rt_blob_header*>(blob);
+    const uint8_t* tp = blob + h->tris_offset + (size_t)slot * 48u;
+    const U4 a = ldg128(tp), b = ldg128(tp + 16), c = ldg128(tp + 32);
+    v[0] = as_float(a.x); v[1] = as_float(a.y); v[2] = as_float(a.z);
+    v[3] = as_float(b.x); v[4] = as_float(b.y); v[5] = as_float(b.z);
+    v[6] = as_float(c.x); v[7] = as_float(c.y); v[8] = as_float(c.z);
+    float w[9];
+    world_tri(s.fwd, a, b, c, w);
+    return point_tri(px, py, pz, w[0], w[1], w[2], w[3], w[4], w[5], w[6], w[7], w[8]);
+}
+
+// Pseudo-normal sign of a scene answer: n = the mesh's row (or object face normal) of the region of c, carried to
+// world as n_w = A^-T n (column k of the stored inverse, affine_row with offset -0: the identity keeps n), then
+// +d when (p - c) . n_w < 0, else -d; d = 0 gives +0.  A^-T maps outward normals to outward normals for every
+// invertible A, mirrors included.
+RT_HD float scene_pseudonormal_sign(const SceneInst& s, const uint8_t* normals, uint32_t slot, const PointHit& h, float px,
+                                    float py, float pz, const float v[9], float d) {
+    float nx, ny, nz;
+    region_normal(normals, slot, h.region, v, nx, ny, nz);
+    const float nz0 = as_float(0x80000000u);
+    const float wx = affine_row(s.inv[0], s.inv[4], s.inv[8], nz0, nx, ny, nz);
+    const float wy = affine_row(s.inv[1], s.inv[5], s.inv[9], nz0, nx, ny, nz);
+    const float wz = affine_row(s.inv[2], s.inv[6], s.inv[10], nz0, nx, ny, nz);
+    const float sg = dot3f(fsub(px, h.cx), fsub(py, h.cy), fsub(pz, h.cz), wx, wy, wz);
+    return (sg < 0.0f || d == 0.0f) ? d : -d;
 }
 
 }  // namespace rt

@@ -115,6 +115,10 @@ def _declare(lib):
         "rt_scene_prepare_sizes": (ci, [i64, i64, psz]),
         "rt_scene_prepare": (ci, [i64, vp, i64, vp, vp, vp, sz, vp, vp, vp]),
         "rt_scene_trace": (ci, [vp, vp, prd, pto, ci, vp, vp, vp, vp, vp, vp, vp, vp]),
+        "rt_scene_point_sizes": (ci, [i64, psz]),
+        "rt_scene_point_prepare": (ci, [vp, i64, vp, sz, vp]),
+        "rt_scene_closest_point": (ci, [vp, vp, vp, prd, pto, C.c_float, vp, vp, vp, vp, vp, vp]),
+        "rt_scene_signed_distance": (ci, [vp, vp, vp, vp, prd, pto, vp, vp, vp, vp, vp, vp]),
         "rt_host_closest_sizes": (ci, [i64, psz]),
         "rt_host_trace_closest": (ci, [vp, i64, vp, ci, vp, pto, vp, vp, vp, vp, vp, vp, sz]),
         "rt_host_trace_closest_compact": (ci, [vp, i64, vp, ci, vp, pto, vp, vp, vp, vp, vp, vp, C.POINTER(C.c_int64), vp, sz]),
@@ -1201,3 +1205,88 @@ def scene_trace(table: torch.Tensor, tlas: AccelStructure, origins: torch.Tensor
             _check(get_module().rt_scene_trace(_ptr(table), _ptr(tlas.blob), C.byref(rd), C.byref(opts), int(mode),
                                                *[_ptr(p) for p in ptrs], _stream(dev)), "rt_scene_trace")
     return out
+
+
+# ------------------------------------------------------------------ point queries on instanced scenes (DESIGN.md §4.12)
+def scene_point_prepare(table: torch.Tensor, n_inst: int) -> torch.Tensor:
+    """rt_scene_point_prepare: the side array (uint8 on the table's device) of the point queries: per instance a lower
+    bound on the smallest singular value of its A and the margins of the instance walk's world bound."""
+    lib = get_module()
+    sb = C.c_size_t()
+    _check(lib.rt_scene_point_sizes(int(n_inst), C.byref(sb)), "rt_scene_point_sizes")
+    dev = table.device
+    with _on_device(dev):
+        side = torch.zeros(sb.value, dtype=torch.uint8, device=dev)
+        _check(lib.rt_scene_point_prepare(_ptr(table), int(n_inst), _ptr(side), side.numel(), _stream(dev)),
+               "rt_scene_point_prepare")
+    return side
+
+
+def _scene_points(table: torch.Tensor, points: torch.Tensor, ray_first: int, ray_count: int):
+    tensor_input_check(points)
+    if table.device != points.device:
+        raise ValueError(f"the scene lives on {table.device} but the points are on {points.device}")
+    rd, batch = make_ray_desc(points, None)
+    if ray_first != 0 or ray_count >= 0:
+        batch = (_window(rd.nray, ray_first, ray_count),)
+    opts = TraceOpts()
+    opts.ray_first, opts.ray_count = int(ray_first), max(int(ray_count), 0)
+    return rd, batch, opts
+
+
+def scene_closest_point(table: torch.Tensor, tlas: AccelStructure, side: torch.Tensor, points: torch.Tensor,
+                        max_distance: float = float("inf"), ray_first: int = 0, ray_count: int = -1):
+    """rt_scene_closest_point: (closest Float32[*b,3], distance Float32[*b], inst Int32[*b], tri Int32[*b],
+    uv Float32[*b,2]) over every instance, the key (d2, inst, tri) minimised; misses give inst = tri = -1, distance
+    inf, closest and uv 0.  1-D over the window [ray_first, ray_first + ray_count) when one is given."""
+    md = float(max_distance)
+    if md != md or md < 0.0:
+        raise ValueError(f"max_distance must be >= 0 or inf (got {max_distance})")
+    rd, batch, opts = _scene_points(table, points, ray_first, ray_count)
+    dev = points.device
+    with _on_device(dev):
+        e = lambda shape, dt: torch.empty(shape, dtype=dt, device=dev)   # noqa: E731
+        out = (e((*batch, 3), torch.float32), e(batch, torch.float32), e(batch, torch.int32), e(batch, torch.int32),
+               e((*batch, 2), torch.float32))
+        if out[1].numel() > 0:
+            _check(get_module().rt_scene_closest_point(_ptr(table), _ptr(tlas.blob), _ptr(side), C.byref(rd),
+                                                       C.byref(opts), md, *[_ptr(t) for t in out], _stream(dev)),
+                   "rt_scene_closest_point")
+    return out
+
+
+def scene_signed_distance(table: torch.Tensor, tlas: AccelStructure, side: torch.Tensor, normals_table: torch.Tensor,
+                          points: torch.Tensor, ray_first: int = 0, ray_count: int = -1, return_closest: bool = False):
+    """rt_scene_signed_distance: Float32[*b], positive inside by the world pseudo-normal of the closest feature, -inf
+    for a point without answer; return_closest=True returns (signed distance, closest, inst, tri, uv) from the same
+    walk.  `normals_table`: int64 device tensor of each mesh's pseudo-normal rows address."""
+    rd, batch, opts = _scene_points(table, points, ray_first, ray_count)
+    dev = points.device
+    with _on_device(dev):
+        e = lambda shape, dt: torch.empty(shape, dtype=dt, device=dev)   # noqa: E731
+        sd = e(batch, torch.float32)
+        extra = ((e((*batch, 3), torch.float32), e(batch, torch.int32), e(batch, torch.int32),
+                  e((*batch, 2), torch.float32)) if return_closest else (None, None, None, None))
+        if sd.numel() > 0:
+            _check(get_module().rt_scene_signed_distance(_ptr(table), _ptr(tlas.blob), _ptr(side), _ptr(normals_table),
+                                                         C.byref(rd), C.byref(opts), _ptr(sd),
+                                                         *[_ptr(t) for t in extra], _stream(dev)),
+                   "rt_scene_signed_distance")
+    return (sd, *extra) if return_closest else sd
+
+
+def scene_distance_grad(points: torch.Tensor, grad_out: torch.Tensor, value: torch.Tensor, closest: torch.Tensor,
+                        tri: torch.Tensor, uv: torch.Tensor, n_faces: int) -> torch.Tensor:
+    """grad_points of a scene distance or signed distance: rt_distance_grad without vertex gradient, g s (p - c) /
+    |value| per point, 0 where value is +-0, +-inf or NaN or tri is outside [0, n_faces)."""
+    tensor_input_check(points)
+    rd, batch = make_ray_desc(points, None)
+    dev = points.device
+    grad_out, value, closest, tri, uv = (t.contiguous() for t in (grad_out, value, closest, tri, uv))
+    with _on_device(dev):
+        gp = torch.empty((*batch, 3), dtype=torch.float32, device=dev)
+        if gp.numel() > 0:
+            _check(get_module().rt_distance_grad(C.byref(rd), C.byref(trace_opts()), _ptr(grad_out), _ptr(value),
+                                                 _ptr(closest), _ptr(tri), _ptr(uv), None, int(n_faces), 0, _ptr(gp),
+                                                 None, None, 0, _stream(dev)), "rt_distance_grad")
+    return gp
