@@ -13,12 +13,6 @@
 using namespace rt;
 
 namespace {
-struct HostPointStack {
-    PointStackEntry e[kMaxDepth];
-    void push(int sp, const PointStackEntry& v) { e[sp] = v; }
-    void pop(int sp, PointStackEntry& v) { v = e[sp]; }
-};
-
 std::vector<uint32_t> stable_order(const std::vector<uint64_t>& keys, std::vector<uint32_t> order) {
     std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return keys[a] < keys[b]; });
     return order;
@@ -71,7 +65,7 @@ extern "C" int pn_signed_distance(const uint8_t* blob, const uint8_t* normals, i
     for (int64_t i = 0; i < n; ++i) {
         PointTrav t;
         point_init(t, pts[3 * i], pts[3 * i + 1], pts[3 * i + 2], INFINITY);
-        HostPointStack stack;
+        ArrayStack<PointStackEntry> stack;
         Stats st;
         while (!point_step(nodes, tris, t, st, stack)) {}
         sn += st.nodes; stt += st.tris;

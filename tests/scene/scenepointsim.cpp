@@ -9,14 +9,6 @@
 
 using namespace rt;
 
-namespace {
-struct HostPointStack {
-    PointStackEntry e[kMaxDepth];
-    void push(int sp, const PointStackEntry& v) { e[sp] = v; }
-    void pop(int sp, PointStackEntry& v) { v = e[sp]; }
-};
-}  // namespace
-
 // rt_scene_point_prepare: side = n_inst x 16 bytes
 extern "C" void ss_point_prepare(const uint8_t* table, ScenePointSide* side) {
     const SceneView sv = scene_view(table);
@@ -36,8 +28,8 @@ extern "C" int ss_point_query(const uint8_t* table, const uint8_t* tlas, const S
     const int32_t n_inst = (int32_t)reinterpret_cast<const SceneHeader*>(table)->n_inst;
     const float max_d2 = normals ? INFINITY : fmul(max_distance, max_distance);
     for (int64_t r = 0; r < n; ++r) {
-        HostPointStack top, below;
-        SceneTopSpace<HostPointStack> sp{sv, side, &below};
+        ArrayStack<PointStackEntry> top, below;
+        SceneTopSpace<ArrayStack<PointStackEntry>> sp{sv, side, &below};
         PointTrav t;
         point_init(t, pts[3 * r], pts[3 * r + 1], pts[3 * r + 2], max_d2);
         NoStats st;

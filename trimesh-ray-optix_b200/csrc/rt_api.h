@@ -47,9 +47,9 @@ inline int grid_for(int64_t n, int threads, int sm_count, int per_sm) {
     return (int)b;
 }
 
-// a point batch (rt_ray_desc origins) that is row-major contiguous [s0, s1, s2, 3]; dimensions of extent 1 may carry
-// any stride
-inline bool points_packed(const int64_t shape[4], const int64_t stride[4]) {
+// a batch (rt_ray_desc origins or directions) that is row-major contiguous [s0, s1, s2, 3]: row r starts at element
+// 3 r (batch_offset); dimensions of extent 1 may carry any stride
+inline bool batch_packed(const int64_t shape[4], const int64_t stride[4]) {
     if (stride[3] != 1) return false;
     int64_t expect = 3;
     for (int i = 2; i >= 0; --i) {
@@ -57,6 +57,26 @@ inline bool points_packed(const int64_t shape[4], const int64_t stride[4]) {
         expect *= shape[i];
     }
     return true;
+}
+
+// Checks the descriptor of a [*b, 3] batch and resolves the window [*first, *first + *n) that opts selects: all of
+// the batch when opts is NULL, to its end when ray_count <= 0.  The data pointers are left to the caller: which ones a
+// query reads, and whether it reads them for an empty window, differ between entry points.
+inline int batch_window(const char* fn, const rt_ray_desc* d, const rt_trace_opts* opts, int64_t* first, int64_t* n) {
+    RT_REQUIRE(d != nullptr, RT_ERR_INVALID, "%s: null batch descriptor", fn);
+    RT_REQUIRE(d->nray >= 0 && d->shape[3] == 3, RT_ERR_INVALID, "%s: batch must be [*b, 3] (nray %lld, last dimension %lld)",
+               fn, (long long)d->nray, (long long)d->shape[3]);
+    RT_REQUIRE(d->shape[0] >= 0 && d->shape[1] >= 0 && d->shape[2] >= 0 && d->shape[0] * d->shape[1] * d->shape[2] == d->nray,
+               RT_ERR_INVALID, "%s: nray %lld does not match shape", fn, (long long)d->nray);
+    const int64_t f = opts ? opts->ray_first : 0, c = opts ? opts->ray_count : 0;
+    RT_REQUIRE(f >= 0 && f <= d->nray, RT_ERR_INVALID, "%s: ray_first %lld outside [0, %lld]", fn, (long long)f,
+               (long long)d->nray);
+    const int64_t m = c <= 0 ? d->nray - f : c;
+    RT_REQUIRE(m <= d->nray - f, RT_ERR_INVALID, "%s: window [%lld, +%lld) exceeds the batch of %lld", fn, (long long)f,
+               (long long)m, (long long)d->nray);
+    *first = f;
+    *n = m;
+    return RT_OK;
 }
 
 // Triangles per leaf slot used by the builder: kLeafTrisDefault, or TRIRO_LEAF_TRIS=1..3 (read once per process;

@@ -31,21 +31,6 @@ struct PointParams {
     float* signed_distance;
 };
 
-struct PointStack {
-    PointStackEntry e[kMaxDepth];
-    __device__ __forceinline__ void push(int sp, const PointStackEntry& v) { e[sp] = v; }
-    __device__ __forceinline__ void pop(int sp, PointStackEntry& v) { v = e[sp]; }
-};
-
-__device__ __forceinline__ int64_t point_offset(const PointParams& p, int64_t r) {
-    if (p.packed) return 3 * r;
-    const int64_t i2 = r % p.shape[2];
-    const int64_t q = r / p.shape[2];
-    const int64_t i1 = q % p.shape[1];
-    const int64_t i0 = q / p.shape[1];
-    return i0 * p.stride[0] + i1 * p.stride[1] + i2 * p.stride[2];
-}
-
 // The body of the three kernels: SIGNED ends the walk with the pseudo-normal sign (DESIGN.md §4.8) instead of writing
 // the closest point, so |signed distance| is bit for bit the distance rt_closest_point returns; SIGNED_CLOSEST does
 // both (closest, tri and uv as rt_closest_point writes them, no distance).
@@ -59,11 +44,11 @@ __device__ __forceinline__ void point_query(const PointParams& p) {
     S st;
     bool found = false;
     if (i < p.n) {
-        const int64_t o = point_offset(p, p.first + i);
+        const int64_t o = batch_offset(p.shape, p.stride, p.packed, p.first + i);
         const int64_t os = p.stride[3];
         PointTrav t;
         point_init(t, p.origins[o], p.origins[o + os], p.origins[o + 2 * os], fmul(p.max_distance, p.max_distance));
-        PointStack stack;
+        ArrayStack<PointStackEntry> stack;
         while (!point_step(nodes, tris, t, st, stack)) {}
         found = t.prim != kNoPrim;
         if (found) {
@@ -140,18 +125,9 @@ using namespace rt;
 static int point_params(const char* fn, const void* blob, const rt_ray_desc* points, const rt_trace_opts* opts,
                         uint64_t* counters_dev, void* stream, PointParams& p, int64_t* count) {
     RT_REQUIRE(blob != nullptr && ((uintptr_t)blob & 15) == 0, RT_ERR_INVALID, "%s: blob null or not 16-byte aligned", fn);
-    RT_REQUIRE(points != nullptr, RT_ERR_INVALID, "%s: null point descriptor", fn);
-    RT_REQUIRE(points->nray >= 0 && points->shape[3] == 3, RT_ERR_INVALID, "%s: point batch must be [*b, 3]", fn);
-    RT_REQUIRE(points->shape[0] >= 0 && points->shape[1] >= 0 && points->shape[2] >= 0 &&
-                   points->shape[0] * points->shape[1] * points->shape[2] == points->nray,
-               RT_ERR_INVALID, "%s: nray %lld does not match shape", fn, (long long)points->nray);
-    static const rt_trace_opts kDefaults = {};
-    const rt_trace_opts& o = opts ? *opts : kDefaults;
-    RT_REQUIRE(o.ray_first >= 0 && o.ray_first <= points->nray, RT_ERR_INVALID, "%s: ray_first %lld outside [0, %lld]", fn,
-               (long long)o.ray_first, (long long)points->nray);
-    const int64_t n = o.ray_count <= 0 ? points->nray - o.ray_first : o.ray_count;
-    RT_REQUIRE(n <= points->nray - o.ray_first, RT_ERR_INVALID, "%s: window [%lld, +%lld) exceeds the batch of %lld", fn,
-               (long long)o.ray_first, (long long)n, (long long)points->nray);
+    int64_t first = 0, n = 0;
+    const int rc = batch_window(fn, points, opts, &first, &n);
+    if (rc != RT_OK) return rc;
     if (counters_dev) RT_CUDA_TRY(cudaMemsetAsync(counters_dev, 0, 4 * sizeof(uint64_t), (cudaStream_t)stream));
     *count = n;
     if (n == 0) return RT_OK;
@@ -162,8 +138,8 @@ static int point_params(const char* fn, const void* blob, const rt_ray_desc* poi
     p.blob = reinterpret_cast<const uint8_t*>(blob);
     p.origins = points->origins;
     for (int a = 0; a < 4; ++a) { p.shape[a] = points->shape[a]; p.stride[a] = points->o_stride[a]; }
-    p.packed = points_packed(points->shape, points->o_stride) ? 1 : 0;
-    p.first = o.ray_first;
+    p.packed = batch_packed(points->shape, points->o_stride) ? 1 : 0;
+    p.first = first;
     p.n = n;
     p.counters = reinterpret_cast<unsigned long long*>(counters_dev);
     return RT_OK;

@@ -61,6 +61,17 @@ RT_HD float as_float(uint32_t u) { return __uint_as_float(u); }
 RT_HD float as_float(uint32_t u) { union { uint32_t u; float f; } c; c.u = u; return c.f; }
 #endif
 
+// Element offset of row r of a [*b, 3] batch flattened to shape[0..2] with element strides stride[0..2]; packed: the
+// batch is row-major contiguous (batch_packed, rt_api.h).
+RT_HD int64_t batch_offset(const int64_t shape[4], const int64_t stride[4], bool packed, int64_t r) {
+    if (packed) return 3 * r;
+    const int64_t i2 = r % shape[2];
+    const int64_t q = r / shape[2];
+    const int64_t i1 = q % shape[1];
+    const int64_t i0 = q / shape[1];
+    return i0 * stride[0] + i1 * stride[1] + i2 * stride[2];
+}
+
 // ------------------------------------------------------------------ layout in HBM
 // Blob = [header 256 B][triangle records 48 B each][BVH8 nodes 80 B each].
 // All sections are 16-byte aligned so every fetch is a 128-bit ld.global.nc.

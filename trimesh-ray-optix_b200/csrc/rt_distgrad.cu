@@ -43,13 +43,7 @@ __global__ void __launch_bounds__(kDgThreads) k_dg_points(const __grid_constant_
     if (i >= p.n) return;
     const int64_t w = p.base + i;              // position in the caller's window
     const int64_t r = p.first + w;             // index in the batch
-    int64_t o;
-    if (p.packed) {
-        o = 3 * r;
-    } else {
-        const int64_t i2 = r % p.shape[2], qq = r / p.shape[2];
-        o = (qq / p.shape[1]) * p.stride[0] + (qq % p.shape[1]) * p.stride[1] + i2 * p.stride[2];
-    }
+    const int64_t o = batch_offset(p.shape, p.stride, p.packed, r);
     const int64_t os = p.stride[3];
     const int32_t t = p.tri[w];
     float q[3];
@@ -112,12 +106,6 @@ struct RgRowParams {
     uint32_t* vals;              // [3 n]
 };
 
-__device__ __forceinline__ int64_t rg_offset(int64_t r, const int64_t shape[4], const int64_t stride[4], int packed) {
-    if (packed) return 3 * r;
-    const int64_t i2 = r % shape[2], qq = r / shape[2];
-    return (qq / shape[1]) * stride[0] + (qq % shape[1]) * stride[1] + i2 * stride[2];
-}
-
 // ray of row j in the window, or -1 for a row_ray outside [0, window)
 __device__ __forceinline__ int64_t rg_ray_of(const RgRowParams& p, int64_t j) {
     const int64_t ray = p.row_ray ? (int64_t)p.row_ray[j] : j;
@@ -131,7 +119,8 @@ __device__ __forceinline__ bool rg_eval(const RgRowParams& p, int64_t j, RgRow& 
         return rg_row(gz, gz, gz, 0.0f, 0.0f, -1, p.mesh, r);
     }
     const int64_t b = p.first + ray;
-    const int64_t oo = rg_offset(b, p.shape, p.o_stride, p.o_packed), od = rg_offset(b, p.shape, p.d_stride, p.d_packed);
+    const int64_t oo = batch_offset(p.shape, p.o_stride, p.o_packed, b);
+    const int64_t od = batch_offset(p.shape, p.d_stride, p.d_packed, b);
     const int64_t os = p.o_stride[3], ds = p.d_stride[3];
     const float o[3] = {p.origins[oo], p.origins[oo + os], p.origins[oo + 2 * os]};
     const float d[3] = {p.directions[od], p.directions[od + ds], p.directions[od + 2 * ds]};
@@ -278,20 +267,11 @@ extern "C" int rt_distance_grad(const rt_ray_desc* points, const rt_trace_opts* 
                                 float* grad_vertices, void* workspace, size_t workspace_bytes, void* stream_) {
     const char* fn = "rt_distance_grad";
     cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
-    RT_REQUIRE(points != nullptr, RT_ERR_INVALID, "%s: null point descriptor", fn);
-    RT_REQUIRE(points->nray >= 0 && points->shape[3] == 3, RT_ERR_INVALID, "%s: point batch must be [*b, 3]", fn);
-    RT_REQUIRE(points->shape[0] >= 0 && points->shape[1] >= 0 && points->shape[2] >= 0 &&
-                   points->shape[0] * points->shape[1] * points->shape[2] == points->nray,
-               RT_ERR_INVALID, "%s: nray %lld does not match shape", fn, (long long)points->nray);
+    int64_t first = 0, n = 0;
+    const int rc = batch_window(fn, points, opts, &first, &n);
+    if (rc != RT_OK) return rc;
     RT_REQUIRE(n_faces >= 0 && n_verts >= 0 && n_verts < kDgMaxVerts, RT_ERR_INVALID,
                "%s: bad mesh size (%lld faces, %lld vertices)", fn, (long long)n_faces, (long long)n_verts);
-    static const rt_trace_opts kDefaults = {};
-    const rt_trace_opts& o = opts ? *opts : kDefaults;
-    RT_REQUIRE(o.ray_first >= 0 && o.ray_first <= points->nray, RT_ERR_INVALID, "%s: ray_first %lld outside [0, %lld]", fn,
-               (long long)o.ray_first, (long long)points->nray);
-    const int64_t n = o.ray_count <= 0 ? points->nray - o.ray_first : o.ray_count;
-    RT_REQUIRE(n <= points->nray - o.ray_first, RT_ERR_INVALID, "%s: window [%lld, +%lld) exceeds the batch of %lld", fn,
-               (long long)o.ray_first, (long long)n, (long long)points->nray);
     if (grad_vertices) RT_CUDA_TRY(cudaMemsetAsync(grad_vertices, 0, (size_t)n_verts * 12u, stream));
     if (n == 0 || (!grad_points && !grad_vertices)) return RT_OK;
     RT_REQUIRE(points->origins && grad_out && value && closest && tri_idx && uv, RT_ERR_INVALID, "%s: null input", fn);
@@ -300,8 +280,8 @@ extern "C" int rt_distance_grad(const rt_ray_desc* points, const rt_trace_opts* 
     DgPointParams p{};
     p.points = points->origins;
     for (int a = 0; a < 4; ++a) { p.shape[a] = points->shape[a]; p.stride[a] = points->o_stride[a]; }
-    p.packed = points_packed(points->shape, points->o_stride) ? 1 : 0;
-    p.first = o.ray_first;
+    p.packed = batch_packed(points->shape, points->o_stride) ? 1 : 0;
+    p.first = first;
     p.grad_out = grad_out; p.value = value; p.closest = closest; p.tri = tri_idx; p.faces = faces;
     p.n_faces = n_faces; p.n_verts = n_verts;
     p.grad_points = grad_points;
@@ -351,21 +331,12 @@ extern "C" int rt_ray_grad(const rt_ray_desc* rays, const rt_trace_opts* opts, i
                            void* stream_) {
     const char* fn = "rt_ray_grad";
     cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
-    RT_REQUIRE(rays != nullptr, RT_ERR_INVALID, "%s: null ray descriptor", fn);
-    RT_REQUIRE(rays->nray >= 0 && rays->shape[3] == 3, RT_ERR_INVALID, "%s: ray batch must be [*b, 3]", fn);
-    RT_REQUIRE(rays->shape[0] >= 0 && rays->shape[1] >= 0 && rays->shape[2] >= 0 &&
-                   rays->shape[0] * rays->shape[1] * rays->shape[2] == rays->nray,
-               RT_ERR_INVALID, "%s: nray %lld does not match shape", fn, (long long)rays->nray);
+    int64_t first = 0, window = 0;
+    const int rc = batch_window(fn, rays, opts, &first, &window);
+    if (rc != RT_OK) return rc;
     RT_REQUIRE(n_rows >= 0 && n_faces >= 0 && n_verts >= 0 && n_verts < kDgMaxVerts, RT_ERR_INVALID,
                "%s: bad sizes (%lld rows, %lld faces, %lld vertices)", fn, (long long)n_rows, (long long)n_faces,
                (long long)n_verts);
-    static const rt_trace_opts kDefaults = {};
-    const rt_trace_opts& o = opts ? *opts : kDefaults;
-    RT_REQUIRE(o.ray_first >= 0 && o.ray_first <= rays->nray, RT_ERR_INVALID, "%s: ray_first %lld outside [0, %lld]", fn,
-               (long long)o.ray_first, (long long)rays->nray);
-    const int64_t window = o.ray_count <= 0 ? rays->nray - o.ray_first : o.ray_count;
-    RT_REQUIRE(window <= rays->nray - o.ray_first, RT_ERR_INVALID, "%s: window [%lld, +%lld) exceeds the batch of %lld",
-               fn, (long long)o.ray_first, (long long)window, (long long)rays->nray);
     // no rows at all (every ray missed): any row_ray, NULL included, and every gradient is +0
     RT_REQUIRE(row_ray != nullptr || n_rows == window || n_rows == 0, RT_ERR_INVALID,
                "%s: without row_ray there must be one row per ray of the window (%lld rows, %lld rays)", fn,
@@ -384,9 +355,9 @@ extern "C" int rt_ray_grad(const rt_ray_desc* rays, const rt_trace_opts* opts, i
     for (int a = 0; a < 4; ++a) {
         p.shape[a] = rays->shape[a]; p.o_stride[a] = rays->o_stride[a]; p.d_stride[a] = rays->d_stride[a];
     }
-    p.o_packed = points_packed(rays->shape, rays->o_stride) ? 1 : 0;
-    p.d_packed = points_packed(rays->shape, rays->d_stride) ? 1 : 0;
-    p.first = o.ray_first; p.window = window; p.n_rows = n_rows;
+    p.o_packed = batch_packed(rays->shape, rays->o_stride) ? 1 : 0;
+    p.d_packed = batch_packed(rays->shape, rays->d_stride) ? 1 : 0;
+    p.first = first; p.window = window; p.n_rows = n_rows;
     p.row_ray = row_ray; p.tri = tri_idx; p.grad_loc = grad_loc; p.grad_uv = grad_uv;
     p.mesh = RgMesh{vertices, n_verts, faces, n_faces};
     p.grad_origins = grad_origins; p.grad_directions = grad_directions;

@@ -32,6 +32,7 @@ struct SceneParams {
     rt_ray_desc rays;
     int64_t first, n;            // window [first, first + n) of the batch; outputs indexed by (r - first)
     float tmax;
+    int packed;                  // origins and directions both row-major contiguous [.., 3]: offset 3 * r
     uint8_t* hit;
     uint8_t* front;
     int32_t* inst;
@@ -41,18 +42,17 @@ struct SceneParams {
     int32_t* count;
 };
 
-struct SceneStack {
-    uint2 e[kMaxDepth];
-    __device__ __forceinline__ void push(int sp, uint32_t x, uint32_t y) { e[sp] = make_uint2(x, y); }
-    __device__ __forceinline__ void pop(int sp, uint32_t& x, uint32_t& y) { const uint2 v = e[sp]; x = v.x; y = v.y; }
-};
-
 template <int MODE>   // 0 closest, 1 any, 2 count
 __global__ void __launch_bounds__(kSceneThreads) k_scene_trace(const __grid_constant__ SceneParams p) {
     const int64_t i = (int64_t)blockIdx.x * kSceneThreads + threadIdx.x;
     if (i >= p.n) return;
     const int64_t r = p.first + i;
-    const int64_t oo = scene_offset(p.rays.shape, p.rays.o_stride, r), dd = scene_offset(p.rays.shape, p.rays.d_stride, r);
+    // one test of the flag: nvcc does not share the row divisions of two batch_offset calls that each test it
+    int64_t oo = 3 * r, dd = 3 * r;
+    if (!p.packed) {
+        oo = batch_offset(p.rays.shape, p.rays.o_stride, false, r);
+        dd = batch_offset(p.rays.shape, p.rays.d_stride, false, r);
+    }
     const int64_t os = p.rays.o_stride[3], ds = p.rays.d_stride[3];
     const float w[6] = {p.rays.origins[oo], p.rays.origins[oo + os], p.rays.origins[oo + 2 * os],
                         p.rays.directions[dd], p.rays.directions[dd + ds], p.rays.directions[dd + 2 * ds]};
@@ -62,11 +62,11 @@ __global__ void __launch_bounds__(kSceneThreads) k_scene_trace(const __grid_cons
     const SceneView sv = scene_view(p.table);
     Ray wr;
     ray_setup(wr, w[0], w[1], w[2], w[3], w[4], w[5]);
-    SceneStack top, below;
+    PairStack top, below;
     Trav t;
     trav_init(t);
     if (MODE == 0) {
-        SceneClosest<SceneStack> vis{sv, {w[0], w[1], w[2], w[3], w[4], w[5]}, p.tmax};
+        SceneClosest<PairStack> vis{sv, {w[0], w[1], w[2], w[3], w[4], w[5]}, p.tmax};
         vis.stack = &below;
         while (!scene_step(nodes, recs, wr, vis, top, t)) {}
         if (vis.inst >= 0) {
@@ -80,12 +80,12 @@ __global__ void __launch_bounds__(kSceneThreads) k_scene_trace(const __grid_cons
             p.uv[2 * i] = 0.0f; p.uv[2 * i + 1] = 0.0f;
         }
     } else if (MODE == 1) {
-        SceneAny<SceneStack> vis{sv, {w[0], w[1], w[2], w[3], w[4], w[5]}, p.tmax};
+        SceneAny<PairStack> vis{sv, {w[0], w[1], w[2], w[3], w[4], w[5]}, p.tmax};
         vis.stack = &below;
         while (!scene_step(nodes, recs, wr, vis, top, t)) {}
         p.hit[i] = vis.found ? 1 : 0;
     } else {
-        SceneCount<SceneStack> vis{sv, {w[0], w[1], w[2], w[3], w[4], w[5]}, p.tmax};
+        SceneCount<PairStack> vis{sv, {w[0], w[1], w[2], w[3], w[4], w[5]}, p.tmax};
         vis.stack = &below;
         while (!scene_step(nodes, recs, wr, vis, top, t)) {}
         p.count[i] = vis.count;
@@ -178,19 +178,9 @@ extern "C" int rt_scene_trace(const void* table, const void* tlas_blob, const rt
     RT_REQUIRE(tlas_blob != nullptr && ((uintptr_t)tlas_blob & 15) == 0, RT_ERR_INVALID,
                "%s: top-level blob null or not 16-byte aligned", fn);
     RT_REQUIRE(mode >= RT_SCENE_CLOSEST && mode <= RT_SCENE_COUNT, RT_ERR_INVALID, "%s: unknown mode %d", fn, mode);
-    RT_REQUIRE(rays != nullptr, RT_ERR_INVALID, "%s: null ray descriptor", fn);
-    RT_REQUIRE(rays->nray >= 0 && rays->shape[3] == 3, RT_ERR_INVALID, "%s: ray batch must be [*b, 3]", fn);
-    RT_REQUIRE(rays->shape[0] >= 0 && rays->shape[1] >= 0 && rays->shape[2] >= 0 &&
-                   rays->shape[0] * rays->shape[1] * rays->shape[2] == rays->nray,
-               RT_ERR_INVALID, "%s: nray %lld does not match shape", fn, (long long)rays->nray);
-    static const rt_trace_opts kDefaults = {};
-    const rt_trace_opts& o = opts ? *opts : kDefaults;
-    RT_REQUIRE(o.ray_first >= 0 && o.ray_first <= rays->nray, RT_ERR_INVALID, "%s: ray_first %lld outside [0, %lld]", fn,
-               (long long)o.ray_first, (long long)rays->nray);
-    const int64_t n = o.ray_count <= 0 ? rays->nray - o.ray_first : o.ray_count;
-    RT_REQUIRE(n <= rays->nray - o.ray_first, RT_ERR_INVALID, "%s: window [%lld, +%lld) exceeds the batch of %lld", fn,
-               (long long)o.ray_first, (long long)n, (long long)rays->nray);
-    if (n == 0) return RT_OK;
+    int64_t first = 0, n = 0;
+    const int rc = batch_window(fn, rays, opts, &first, &n);
+    if (rc != RT_OK || n == 0) return rc;
     RT_REQUIRE(rays->origins != nullptr && rays->directions != nullptr, RT_ERR_INVALID, "%s: null rays", fn);
     if (mode == RT_SCENE_CLOSEST)
         RT_REQUIRE(hit && front && inst_idx && tri_idx && loc && uv, RT_ERR_INVALID, "%s: null output", fn);
@@ -204,10 +194,11 @@ extern "C" int rt_scene_trace(const void* table, const void* tlas_blob, const rt
     p.table = reinterpret_cast<const uint8_t*>(table);
     p.tlas = reinterpret_cast<const uint8_t*>(tlas_blob);
     p.rays = *rays;
-    p.first = o.ray_first;
+    p.first = first;
     p.n = n;
-    p.tmax = o.tmax > 0.0f ? o.tmax : RT_TMAX_DEFAULT;     // NaN and <= 0 select the default, as rt_trace_* do
+    p.tmax = opts && opts->tmax > 0.0f ? opts->tmax : RT_TMAX_DEFAULT;     // NaN and <= 0 select the default, as rt_trace_* do
     p.hit = hit; p.front = front; p.inst = inst_idx; p.tri = tri_idx; p.loc = loc; p.uv = uv; p.count = count;
+    p.packed = batch_packed(rays->shape, rays->o_stride) && batch_packed(rays->shape, rays->d_stride) ? 1 : 0;
     cudaStream_t st = (cudaStream_t)stream;
     if (mode == RT_SCENE_CLOSEST)
         k_scene_trace<0><<<(unsigned)grid, kSceneThreads, 0, st>>>(p);

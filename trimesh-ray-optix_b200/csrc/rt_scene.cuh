@@ -182,15 +182,6 @@ RT_HD bool box_hit(const Ray& r, const float lo[3], const float hi[3], float tma
     return tn <= tf;
 }
 
-// Element offset of row r of a [*b, 3] batch flattened to shape[0..2] with element strides stride[0..2].
-RT_HD int64_t scene_offset(const int64_t shape[4], const int64_t stride[4], int64_t r) {
-    const int64_t i2 = r % shape[2];
-    const int64_t q = r / shape[2];
-    const int64_t i1 = q % shape[1];
-    const int64_t i0 = q / shape[1];
-    return i0 * stride[0] + i1 * stride[1] + i2 * stride[2];
-}
-
 struct SceneView {
     const SceneInst* inst;
     const uint64_t* blobs;      // BLAS blob address of each mesh

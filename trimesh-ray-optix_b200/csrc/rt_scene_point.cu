@@ -31,6 +31,7 @@ struct ScenePointParams {
     rt_ray_desc points;
     int64_t first, n;            // window [first, first + n) of the batch; outputs indexed by (r - first)
     float max_d2;
+    int packed;                  // row-major contiguous [.., 3]: offset 3 * r
     float* closest;
     float* distance;
     int32_t* inst;
@@ -39,22 +40,16 @@ struct ScenePointParams {
     float* signed_distance;
 };
 
-struct ScenePointStack {
-    PointStackEntry e[kMaxDepth];
-    __device__ __forceinline__ void push(int sp, const PointStackEntry& v) { e[sp] = v; }
-    __device__ __forceinline__ void pop(int sp, PointStackEntry& v) { v = e[sp]; }
-};
-
 // SIGNED: write the signed distance; CLOSEST: write closest, inst, tri and uv (and the distance when not SIGNED).
 template <bool SIGNED, bool CLOSEST>
 __global__ void __launch_bounds__(kScenePointThreads) k_scene_point(const __grid_constant__ ScenePointParams p) {
     const int64_t i = (int64_t)blockIdx.x * kScenePointThreads + threadIdx.x;
     if (i >= p.n) return;
-    const int64_t o = scene_offset(p.points.shape, p.points.o_stride, p.first + i);
+    const int64_t o = batch_offset(p.points.shape, p.points.o_stride, p.packed, p.first + i);
     const int64_t os = p.points.o_stride[3];
     const rt_blob_header* th = reinterpret_cast<const rt_blob_header*>(p.tlas);
-    ScenePointStack top, below;
-    SceneTopSpace<ScenePointStack> sp{scene_view(p.table), p.side, &below};
+    ArrayStack<PointStackEntry> top, below;
+    SceneTopSpace<ArrayStack<PointStackEntry>> sp{scene_view(p.table), p.side, &below};
     PointTrav t;
     point_init(t, p.points.origins[o], p.points.origins[o + os], p.points.origins[o + 2 * os], p.max_d2);
     NoStats st;
@@ -117,18 +112,9 @@ static int scene_point_params(const char* fn, const void* table, const void* tla
     RT_REQUIRE(tlas_blob != nullptr && ((uintptr_t)tlas_blob & 15) == 0, RT_ERR_INVALID,
                "%s: top-level blob null or not 16-byte aligned", fn);
     RT_REQUIRE(side != nullptr && ((uintptr_t)side & 15) == 0, RT_ERR_INVALID, "%s: side null or not 16-byte aligned", fn);
-    RT_REQUIRE(points != nullptr, RT_ERR_INVALID, "%s: null point descriptor", fn);
-    RT_REQUIRE(points->nray >= 0 && points->shape[3] == 3, RT_ERR_INVALID, "%s: point batch must be [*b, 3]", fn);
-    RT_REQUIRE(points->shape[0] >= 0 && points->shape[1] >= 0 && points->shape[2] >= 0 &&
-                   points->shape[0] * points->shape[1] * points->shape[2] == points->nray,
-               RT_ERR_INVALID, "%s: nray %lld does not match shape", fn, (long long)points->nray);
-    static const rt_trace_opts kDefaults = {};
-    const rt_trace_opts& o = opts ? *opts : kDefaults;
-    RT_REQUIRE(o.ray_first >= 0 && o.ray_first <= points->nray, RT_ERR_INVALID, "%s: ray_first %lld outside [0, %lld]", fn,
-               (long long)o.ray_first, (long long)points->nray);
-    const int64_t n = o.ray_count <= 0 ? points->nray - o.ray_first : o.ray_count;
-    RT_REQUIRE(n <= points->nray - o.ray_first, RT_ERR_INVALID, "%s: window [%lld, +%lld) exceeds the batch of %lld", fn,
-               (long long)o.ray_first, (long long)n, (long long)points->nray);
+    int64_t first = 0, n = 0;
+    const int rc = batch_window(fn, points, opts, &first, &n);
+    if (rc != RT_OK) return rc;
     *count = n;
     if (n == 0) return RT_OK;
     RT_REQUIRE(points->origins != nullptr, RT_ERR_INVALID, "%s: null points", fn);
@@ -139,8 +125,9 @@ static int scene_point_params(const char* fn, const void* table, const void* tla
     p.tlas = reinterpret_cast<const uint8_t*>(tlas_blob);
     p.side = reinterpret_cast<const ScenePointSide*>(side);
     p.points = *points;
-    p.first = o.ray_first;
+    p.first = first;
     p.n = n;
+    p.packed = batch_packed(points->shape, points->o_stride) ? 1 : 0;
     return RT_OK;
 }
 

@@ -68,12 +68,6 @@ struct TraceParams {
     float cam_mat[9], cam_origin[3];
 };
 
-struct LocalStack {
-    uint2 e[kMaxDepth];
-    __device__ __forceinline__ void push(int sp, uint32_t x, uint32_t y) { e[sp] = make_uint2(x, y); }
-    __device__ __forceinline__ void pop(int sp, uint32_t& x, uint32_t& y) { const uint2 v = e[sp]; x = v.x; y = v.y; }
-};
-
 // Every launch leaves its scratch zeroed: the last CTA to finish resets the ray counter and the CTA count, so the
 // next call on the same stream can skip its memset (RT_OPT_SCRATCH_ZEROED) and a launch is a single kernel.
 __device__ __forceinline__ void release_scratch(const TraceParams& p);
@@ -203,7 +197,7 @@ __global__ void __launch_bounds__(kTraceThreads, RT_TRACE_MIN_BLOCKS) k_trace(co
     const int lane = threadIdx.x & 31;
     const unsigned lt_mask = (1u << lane) - 1u;
     const int64_t nray = p.nray;
-    LocalStack stack;
+    PairStack stack;
     unsigned long long st_nodes = 0, st_tris = 0, st_rays = 0, st_hits = 0;
     bool any_inside = false, any_broken = false;
 
@@ -360,40 +354,12 @@ __device__ __forceinline__ void release_scratch(const TraceParams& p) {
 #include "rt_trace_coop.cuh"
 namespace rt {
 
-static int fetch_mode(const int64_t shape[4], const int64_t stride[4], int64_t nray);
-static bool is_packed(const int64_t shape[4], const int64_t stride[4]) {
-    // row-major contiguous [s0,s1,s2,3]; dimensions of extent 1 may carry any stride
-    if (stride[3] != 1) return false;
-    int64_t expect = 3;
-    for (int i = 2; i >= 0; --i) {
-        if (shape[i] != 1 && stride[i] != expect) return false;
-        expect *= shape[i];
-    }
-    return true;
-}
-
 static int fetch_mode(const int64_t shape[4], const int64_t stride[4], int64_t nray) {
-    if (is_packed(shape, stride)) return kPacked;
+    if (batch_packed(shape, stride)) return kPacked;
     bool constant = true;
     for (int i = 0; i < 3; ++i) if (shape[i] != 1 && stride[i] != 0) constant = false;
     if (constant) return kConstant;                    // stride-0 broadcast of one vector
     return nray < ((int64_t)1 << 31) ? kGeneral32 : kGeneral;
-}
-
-static int check_rays(const char* fn, const rt_ray_desc* rays, bool need_dirs) {
-    RT_REQUIRE(rays != nullptr, RT_ERR_INVALID, "%s: null ray descriptor", fn);
-    RT_REQUIRE(rays->nray >= 0, RT_ERR_INVALID, "%s: negative ray count", fn);
-    RT_REQUIRE(rays->shape[3] == 3, RT_ERR_INVALID, "%s: last dimension must be 3 (got %lld)", fn,
-               (long long)rays->shape[3]);
-    RT_REQUIRE(rays->shape[0] >= 0 && rays->shape[1] >= 0 && rays->shape[2] >= 0, RT_ERR_INVALID,
-               "%s: negative shape", fn);
-    RT_REQUIRE(rays->shape[0] * rays->shape[1] * rays->shape[2] == rays->nray, RT_ERR_INVALID,
-               "%s: nray %lld does not match shape", fn, (long long)rays->nray);
-    if (rays->nray > 0) {
-        RT_REQUIRE(rays->origins != nullptr, RT_ERR_INVALID, "%s: null origins", fn);
-        RT_REQUIRE(!need_dirs || rays->directions != nullptr, RT_ERR_INVALID, "%s: null directions", fn);
-    }
-    return RT_OK;
 }
 
 // resident CTAs per SM of every kernel variant, per device (filled on first use; benign race: same value)
@@ -416,24 +382,22 @@ static int launch(const char* fn, TraceParams& p, const void* blob, const rt_ray
                   void* scratch, cudaStream_t stream) {
     RT_REQUIRE(blob != nullptr && ((uintptr_t)blob & 15) == 0, RT_ERR_INVALID, "%s: blob null or not 16-byte aligned", fn);
     RT_REQUIRE(scratch != nullptr && ((uintptr_t)scratch & 7) == 0, RT_ERR_INVALID, "%s: scratch null or misaligned", fn);
+    int64_t first = 0, count = 0;
+    const int rc = batch_window(fn, rays, opts, &first, &count);
+    if (rc != RT_OK) return rc;
     const bool pinhole = p.o_mode == kPinhole;     // preset by rt_trace_closest_pinhole: rays are generated, not fetched
-    if (!pinhole) {
-        const int rc = check_rays(fn, rays, MODE != kContains);
-        if (rc != RT_OK) return rc;
+    if (!pinhole && rays->nray > 0) {               // NULL data of a non-empty batch is an error even for an empty window
+        RT_REQUIRE(rays->origins != nullptr, RT_ERR_INVALID, "%s: null origins", fn);
+        RT_REQUIRE(MODE == kContains || rays->directions != nullptr, RT_ERR_INVALID, "%s: null directions", fn);
     }
+    if (count == 0) return RT_OK;
     static const rt_trace_opts kDefaults = {};
     const rt_trace_opts& o = opts ? *opts : kDefaults;
-    RT_REQUIRE(o.ray_first >= 0 && o.ray_first <= rays->nray, RT_ERR_INVALID, "%s: ray_first %lld outside [0, %lld]", fn,
-               (long long)o.ray_first, (long long)rays->nray);
-    const int64_t count = o.ray_count <= 0 ? rays->nray - o.ray_first : o.ray_count;     // 0 (zero-initialised opts) = all
-    RT_REQUIRE(count <= rays->nray - o.ray_first, RT_ERR_INVALID, "%s: ray window [%lld, +%lld) exceeds the batch of %lld", fn,
-               (long long)o.ray_first, (long long)count, (long long)rays->nray);
-    if (count == 0) return RT_OK;
     DeviceInfo dev;
     RT_REQUIRE(device_info(&dev) == RT_OK && dev.sm_count > 0, RT_ERR_CUDA, "%s: no CUDA device", fn);
     p.blob = reinterpret_cast<const uint8_t*>(blob);
     p.rays = *rays;
-    p.ray_first = o.ray_first;
+    p.ray_first = first;
     p.nray = count;
     if (!pinhole) {
         p.o_mode = fetch_mode(rays->shape, rays->o_stride, rays->nray);
@@ -451,7 +415,7 @@ static int launch(const char* fn, TraceParams& p, const void* blob, const rt_ray
     // the warp-cooperative triangle tests of rt_trace_coop.cuh.
     const bool coherent = MODE != kContains && (p.o_mode == kConstant || pinhole);
     p.tile_per_row = 0u;
-    if (coherent && !(o.flags & RT_OPT_NO_TILE_ORDER) && o.ray_first == 0 && count == rays->nray) {
+    if (coherent && !(o.flags & RT_OPT_NO_TILE_ORDER) && first == 0 && count == rays->nray) {
         const int64_t h = rays->shape[1], w = rays->shape[2];
         if (h > 0 && w > 0 && h % kTileH == 0 && w % kTileW == 0 && h * w < ((int64_t)1 << 31) && rays->nray == h * w) {
             p.tile_per_row = (uint32_t)(w / kTileW); p.tile_w = (uint32_t)w;

@@ -126,7 +126,7 @@ k_trace_coop(const __grid_constant__ TraceParams p) {
     const unsigned lt_mask = (1u << lane) - 1u;
     const int64_t nray = p.nray;
     const unsigned long long key_init = (unsigned long long)__float_as_uint(p.tmax) << 32;
-    LocalStack stack;
+    PairStack stack;
     unsigned long long st_nodes = 0, st_tris = 0, st_rays = 0, st_hits = 0;
     bool any_inside = false, any_broken = false;
 

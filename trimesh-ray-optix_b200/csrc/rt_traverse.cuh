@@ -35,6 +35,22 @@ struct Trav {
 };
 RT_HD void trav_init(Trav& t) { t.gx = 0u; t.gy = 0x80000000u; t.sp = 0; }   // root group: node 0, top priority
 
+// Per-thread traversal stacks, one entry per tree level.  PairStack holds the (gx, gy) node groups of trav_step and
+// scene_step; ArrayStack the entries of the point walks (point_step, wind_step).
+#if defined(__CUDACC__)
+struct PairStack {
+    uint2 e[kMaxDepth];
+    __device__ __forceinline__ void push(int sp, uint32_t x, uint32_t y) { e[sp] = make_uint2(x, y); }
+    __device__ __forceinline__ void pop(int sp, uint32_t& x, uint32_t& y) { const uint2 v = e[sp]; x = v.x; y = v.y; }
+};
+#endif
+template <class E>
+struct ArrayStack {
+    E e[kMaxDepth];
+    RT_HD void push(int sp, const E& v) { e[sp] = v; }
+    RT_HD void pop(int sp, E& v) { v = e[sp]; }
+};
+
 // Visitor concept:
 //   float tmax            current far limit of the ray interval (closest-hit shrinks it)
 //   bool hit(const Ray&, const TriHit&, int32_t prim, uint32_t tri_slot)  -> true = terminate ray

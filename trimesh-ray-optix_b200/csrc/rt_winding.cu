@@ -56,21 +56,6 @@ struct WindParams {
     unsigned long long* counters;
 };
 
-struct WindStack {
-    WindStackEntry e[kMaxDepth];
-    __device__ __forceinline__ void push(int sp, const WindStackEntry& v) { e[sp] = v; }
-    __device__ __forceinline__ void pop(int sp, WindStackEntry& v) { v = e[sp]; }
-};
-
-__device__ __forceinline__ int64_t wind_offset(const WindParams& p, int64_t r) {
-    if (p.packed) return 3 * r;
-    const int64_t i2 = r % p.shape[2];
-    const int64_t q = r / p.shape[2];
-    const int64_t i1 = q % p.shape[1];
-    const int64_t i0 = q / p.shape[1];
-    return i0 * p.stride[0] + i1 * p.stride[1] + i2 * p.stride[2];
-}
-
 template <bool STATS>
 __global__ void __launch_bounds__(kWindThreads) k_winding_number(const __grid_constant__ WindParams p) {
     using S = typename std::conditional<STATS, WindStats, WindNoStats>::type;
@@ -80,11 +65,11 @@ __global__ void __launch_bounds__(kWindThreads) k_winding_number(const __grid_co
     const int64_t i = (int64_t)blockIdx.x * kWindThreads + threadIdx.x;
     S st;
     if (i < p.n) {
-        const int64_t o = wind_offset(p, p.first + i);
+        const int64_t o = batch_offset(p.shape, p.stride, p.packed, p.first + i);
         const int64_t os = p.stride[3];
         WindTrav t;
         wind_init(t, p.origins[o], p.origins[o + os], p.origins[o + 2 * os]);
-        WindStack stack;
+        ArrayStack<WindStackEntry> stack;
         while (!wind_step(nodes, tris, p.moments, p.beta, t, st, stack)) {}
         p.winding[i] = wind_result(t);
     }
@@ -168,19 +153,10 @@ extern "C" int rt_winding_number(const void* blob, const void* moments, const rt
     RT_REQUIRE(blob != nullptr && ((uintptr_t)blob & 15) == 0, RT_ERR_INVALID, "%s: blob null or not 16-byte aligned", fn);
     RT_REQUIRE(moments != nullptr && ((uintptr_t)moments & 15) == 0, RT_ERR_INVALID,
                "%s: moments null or not 16-byte aligned", fn);
-    RT_REQUIRE(points != nullptr, RT_ERR_INVALID, "%s: null point descriptor", fn);
     RT_REQUIRE(beta >= 1.0f, RT_ERR_INVALID, "%s: beta must be >= 1 or +inf (got %g)", fn, (double)beta);
-    RT_REQUIRE(points->nray >= 0 && points->shape[3] == 3, RT_ERR_INVALID, "%s: point batch must be [*b, 3]", fn);
-    RT_REQUIRE(points->shape[0] >= 0 && points->shape[1] >= 0 && points->shape[2] >= 0 &&
-                   points->shape[0] * points->shape[1] * points->shape[2] == points->nray,
-               RT_ERR_INVALID, "%s: nray %lld does not match shape", fn, (long long)points->nray);
-    static const rt_trace_opts kDefaults = {};
-    const rt_trace_opts& o = opts ? *opts : kDefaults;
-    RT_REQUIRE(o.ray_first >= 0 && o.ray_first <= points->nray, RT_ERR_INVALID, "%s: ray_first %lld outside [0, %lld]", fn,
-               (long long)o.ray_first, (long long)points->nray);
-    const int64_t count = o.ray_count <= 0 ? points->nray - o.ray_first : o.ray_count;
-    RT_REQUIRE(count <= points->nray - o.ray_first, RT_ERR_INVALID, "%s: window [%lld, +%lld) exceeds the batch of %lld", fn,
-               (long long)o.ray_first, (long long)count, (long long)points->nray);
+    int64_t first = 0, count = 0;
+    const int rc = batch_window(fn, points, opts, &first, &count);
+    if (rc != RT_OK) return rc;
     if (counters_dev) RT_CUDA_TRY(cudaMemsetAsync(counters_dev, 0, 4 * sizeof(uint64_t), (cudaStream_t)stream));
     if (count == 0) return RT_OK;
     RT_REQUIRE(points->origins != nullptr, RT_ERR_INVALID, "%s: null points", fn);
@@ -190,8 +166,8 @@ extern "C" int rt_winding_number(const void* blob, const void* moments, const rt
     p.moments = reinterpret_cast<const uint8_t*>(moments);
     p.origins = points->origins;
     for (int a = 0; a < 4; ++a) { p.shape[a] = points->shape[a]; p.stride[a] = points->o_stride[a]; }
-    p.packed = points_packed(points->shape, points->o_stride) ? 1 : 0;
-    p.first = o.ray_first;
+    p.packed = batch_packed(points->shape, points->o_stride) ? 1 : 0;
+    p.first = first;
     p.n = count;
     p.beta = beta;
     p.winding = winding;

@@ -563,6 +563,29 @@ def _window(nray: int, ray_first: int, ray_count: int) -> int:
     return nray - ray_first if ray_count < 0 else ray_count
 
 
+def _query_batch(points: torch.Tensor, dirs: torch.Tensor | None, ray_first: int, ray_count: int,
+                 counters: torch.Tensor | None = None, table: torch.Tensor | None = None):
+    """Prelude of the point and scene queries: checks the batch (and the counters, and that a scene table lives on the
+    batch's device) and returns (descriptor, output batch shape): the batch's, or 1-D over the window
+    [ray_first, ray_first + ray_count).  An empty window zeroes the counters; the caller launches nothing."""
+    tensor_input_check(points, *(() if dirs is None else (dirs,)))
+    if table is not None and table.device != points.device:
+        kind = "points" if dirs is None else "rays"
+        raise ValueError(f"the scene lives on {table.device} but the {kind} are on {points.device}")
+    rd, batch = make_ray_desc(points, dirs)
+    n = rd.nray
+    if ray_first != 0 or ray_count >= 0:
+        n = _window(rd.nray, ray_first, ray_count)
+        batch = (n,)
+    if counters is not None:
+        if (counters.dtype != torch.int64 or counters.device != points.device or counters.numel() != 4
+                or not counters.is_contiguous()):
+            raise ValueError("counters must be a contiguous int64 tensor of 4 elements on the points' device")
+        if n == 0:
+            counters.zero_()
+    return rd, batch
+
+
 def intersects_closest_into(accel_structure, origins: torch.Tensor, dirs: torch.Tensor, hit_ptr: int, front_ptr: int,
                             tri_ptr: int, loc_ptr: int, uv_ptr: int, ray_first: int = 0, ray_count: int = -1) -> None:
     """rt_trace_closest with caller-provided RAW output addresses (u8 hit, u8 front, i32 tri, f32 loc[3], f32 uv[2]
@@ -818,26 +841,18 @@ def closest_point(accel_structure, points: torch.Tensor, max_distance: float = f
     With a window [ray_first, ray_first + ray_count) of the flattened batch the outputs are 1-D over the window.
     `counters` (Int64[4] on the device, optional) selects the instrumented kernel: nodes fetched, triangles tested,
     points, points with an answer."""
-    tensor_input_check(points)
     md = float(max_distance)
     if md != md or md < 0.0:
         raise ValueError(f"max_distance must be >= 0 or inf (got {max_distance})")
+    rd, batch = _query_batch(points, None, ray_first, ray_count, counters)
     blob = _blob_of(accel_structure, points.device)
-    rd, batch = make_ray_desc(points, None)
-    if ray_first != 0 or ray_count >= 0:
-        batch = (_window(rd.nray, ray_first, ray_count),)
     dev = points.device
-    if counters is not None and (counters.dtype != torch.int64 or counters.device != dev or counters.numel() != 4
-                                 or not counters.is_contiguous()):
-        raise ValueError("counters must be a contiguous int64 tensor of 4 elements on the points' device")
     with _on_device(dev):
         closest = torch.empty((*batch, 3), dtype=torch.float32, device=dev)
         distance = torch.empty(batch, dtype=torch.float32, device=dev)
         tri = torch.empty(batch, dtype=torch.int32, device=dev)
         uv = torch.empty((*batch, 2), dtype=torch.float32, device=dev)
         if tri.numel() == 0:
-            if counters is not None:
-                counters.zero_()
             return closest, distance, tri, uv
         st = _stream(dev)
         _check(get_module().rt_closest_point(_ptr(blob), C.byref(rd), C.byref(trace_opts(accel_structure, ray_first, ray_count)),
@@ -878,23 +893,15 @@ def winding_number(accel_structure, points: torch.Tensor, beta: float = 2.0, ray
     an empty mesh 0.  With a window [ray_first, ray_first + ray_count) of the flattened batch the output is 1-D over the
     window.  `counters` (Int64[4] on the device, optional) selects the instrumented kernel: nodes visited, triangles
     summed exactly, points, far-field terms."""
-    tensor_input_check(points)
     b = float(beta)
     if not (b >= 1.0):
         raise ValueError(f"beta must be >= 1 or inf (got {beta})")
+    rd, batch = _query_batch(points, None, ray_first, ray_count, counters)
     blob = _blob_of(accel_structure, points.device)
-    rd, batch = make_ray_desc(points, None)
-    if ray_first != 0 or ray_count >= 0:
-        batch = (_window(rd.nray, ray_first, ray_count),)
     dev = points.device
-    if counters is not None and (counters.dtype != torch.int64 or counters.device != dev or counters.numel() != 4
-                                 or not counters.is_contiguous()):
-        raise ValueError("counters must be a contiguous int64 tensor of 4 elements on the points' device")
     with _on_device(dev):
         w = torch.empty(batch, dtype=torch.float32, device=dev)
         if w.numel() == 0:
-            if counters is not None:
-                counters.zero_()
             return w
         moments = winding_moments(accel_structure)
         st = _stream(dev)
@@ -935,15 +942,9 @@ def signed_distance_pseudonormal(accel_structure, points: torch.Tensor, ray_firs
     is cached.  |result| is bit for bit closest_point's distance; an exact 0 is +0; a non-finite point or an empty
     mesh gives -inf.  Batch, window and counters as closest_point.  return_closest=True returns
     (signed distance, closest, tri, uv) from the same walk, the last three exactly as closest_point's."""
-    tensor_input_check(points)
+    rd, batch = _query_batch(points, None, ray_first, ray_count, counters)
     blob = _blob_of(accel_structure, points.device)
-    rd, batch = make_ray_desc(points, None)
-    if ray_first != 0 or ray_count >= 0:
-        batch = (_window(rd.nray, ray_first, ray_count),)
     dev = points.device
-    if counters is not None and (counters.dtype != torch.int64 or counters.device != dev or counters.numel() != 4
-                                 or not counters.is_contiguous()):
-        raise ValueError("counters must be a contiguous int64 tensor of 4 elements on the points' device")
     with _on_device(dev):
         sd = torch.empty(batch, dtype=torch.float32, device=dev)
         if return_closest:
@@ -951,8 +952,6 @@ def signed_distance_pseudonormal(accel_structure, points: torch.Tensor, ray_firs
             tri = torch.empty(batch, dtype=torch.int32, device=dev)
             uv = torch.empty((*batch, 2), dtype=torch.float32, device=dev)
         if sd.numel() == 0:
-            if counters is not None:
-                counters.zero_()
             return (sd, closest, tri, uv) if return_closest else sd
         normals, _ = pseudo_normals(accel_structure)
         # an empty mesh has an empty (null) normals tensor: the kernel finds no triangle and reads no row
@@ -1178,12 +1177,7 @@ def scene_trace(table: torch.Tensor, tlas: AccelStructure, origins: torch.Tensor
                 tmax: float = TMAX_DEFAULT, ray_first: int = 0, ray_count: int = -1):
     """rt_scene_trace.  closest: (hit, front, inst, tri, loc, uv); any: hit; count: count — shaped like the batch, or
     1-D over the window [ray_first, ray_first + ray_count)."""
-    tensor_input_check(origins, dirs)
-    if table.device != origins.device:
-        raise ValueError(f"the scene lives on {table.device} but the rays are on {origins.device}")
-    rd, batch = make_ray_desc(origins, dirs)
-    if ray_first != 0 or ray_count >= 0:
-        batch = (_window(rd.nray, ray_first, ray_count),)
+    rd, batch = _query_batch(origins, dirs, ray_first, ray_count, table=table)
     dev = origins.device
     opts = TraceOpts()
     opts.tmax = float(tmax)
@@ -1222,18 +1216,6 @@ def scene_point_prepare(table: torch.Tensor, n_inst: int) -> torch.Tensor:
     return side
 
 
-def _scene_points(table: torch.Tensor, points: torch.Tensor, ray_first: int, ray_count: int):
-    tensor_input_check(points)
-    if table.device != points.device:
-        raise ValueError(f"the scene lives on {table.device} but the points are on {points.device}")
-    rd, batch = make_ray_desc(points, None)
-    if ray_first != 0 or ray_count >= 0:
-        batch = (_window(rd.nray, ray_first, ray_count),)
-    opts = TraceOpts()
-    opts.ray_first, opts.ray_count = int(ray_first), max(int(ray_count), 0)
-    return rd, batch, opts
-
-
 def scene_closest_point(table: torch.Tensor, tlas: AccelStructure, side: torch.Tensor, points: torch.Tensor,
                         max_distance: float = float("inf"), ray_first: int = 0, ray_count: int = -1):
     """rt_scene_closest_point: (closest Float32[*b,3], distance Float32[*b], inst Int32[*b], tri Int32[*b],
@@ -1242,7 +1224,8 @@ def scene_closest_point(table: torch.Tensor, tlas: AccelStructure, side: torch.T
     md = float(max_distance)
     if md != md or md < 0.0:
         raise ValueError(f"max_distance must be >= 0 or inf (got {max_distance})")
-    rd, batch, opts = _scene_points(table, points, ray_first, ray_count)
+    rd, batch = _query_batch(points, None, ray_first, ray_count, table=table)
+    opts = trace_opts(None, ray_first, ray_count)
     dev = points.device
     with _on_device(dev):
         e = lambda shape, dt: torch.empty(shape, dtype=dt, device=dev)   # noqa: E731
@@ -1260,7 +1243,8 @@ def scene_signed_distance(table: torch.Tensor, tlas: AccelStructure, side: torch
     """rt_scene_signed_distance: Float32[*b], positive inside by the world pseudo-normal of the closest feature, -inf
     for a point without answer; return_closest=True returns (signed distance, closest, inst, tri, uv) from the same
     walk.  `normals_table`: int64 device tensor of each mesh's pseudo-normal rows address."""
-    rd, batch, opts = _scene_points(table, points, ray_first, ray_count)
+    rd, batch = _query_batch(points, None, ray_first, ray_count, table=table)
+    opts = trace_opts(None, ray_first, ray_count)
     dev = points.device
     with _on_device(dev):
         e = lambda shape, dt: torch.empty(shape, dtype=dt, device=dev)   # noqa: E731
