@@ -456,6 +456,53 @@ int rt_scene_signed_distance(const void* table, const void* tlas_blob, const voi
                              const rt_ray_desc* points, const rt_trace_opts* opts, float* signed_distance, float* closest,
                              int32_t* inst_idx, int32_t* tri_idx, float* uv, void* stream);
 
+/* ---- Gradients of instanced-scene queries (DESIGN.md §4.13): the backward of rt_scene_trace's closest-hit loc and uv
+ *      (dense or compacted) and of rt_scene_closest_point's distance / rt_scene_signed_distance's value, with respect
+ *      to the rays or points, the instance transforms and the member vertices, without a walk.
+ *      `members`: DEVICE array of one rt_scene_member per mesh of the table: the member's vertices f32 [n_verts, 3] and
+ *      faces i32 [n_faces, 3] as of the forward, and vertex_base, the row of its vertex 0 in grad_vertices
+ *      ([n_verts_total, 3]).  `n_inst` and `n_meshes` bound what the rows may index (the table's own counts when
+ *      smaller).  Row j is (instance i = inst_idx[j], triangle t = tri_idx[j]); with A | b the table's transform of i,
+ *      v_k the member's vertices of face t and w its barycentrics:
+ *        hit rows: the hit is recomputed as rt_ray_grad does on the WORLD triangle W_k = affine_row(A row, b (0 as -0),
+ *          v_k); lambda, t lambda, q = lambda - g_L and w are rt_ray_grad's, and so are the per-ray sums into
+ *          grad_origins / grad_directions (rows of one ray contiguous, row_ray NULL: row j is ray j).
+ *        point rows: q = rt_distance_grad's grad_points row (from grad_out, value, closest), w = (uv0, uv1).
+ *        Then, with w2 = (1 - w0) - w1, x = (w0 v0 + w1 v1) + w2 v2 and q_obj_j = affine_row(A column j, -0, q):
+ *          grad_transforms[i][r][j] += -x_j q_r (j < 3),  grad_transforms[i][r][3] += -q_r,
+ *          grad_vertices[vertex_base + faces[t][k]] += -w_k q_obj.
+ *      A row contributes 0 everywhere (its own grad_points row included) when inst is outside [0, n_inst), its mesh
+ *      outside [0, n_meshes), t outside the member's faces, a vertex index outside its vertices or vertex_base + index
+ *      outside [0, n_verts_total), det = 0 (hit rows), value +-0, +-inf or NaN (point rows), a hit row's ray outside
+ *      the window, or when any of lambda, t lambda, q, w, x, q_obj is not finite.  The transform columns and the vertices
+ *      are summed as rt_distance_grad sums vertices: one stable sort of (key, pair) over the joint key space
+ *      [member vertices | 4 I transform columns], the fixed 32-ary tree per key in ascending (row, corner) order, in
+ *      row windows of the size that fits workspace_bytes (at most 2^30 / 7 rows), added in window order from +0.
+ *      grad_origins / grad_directions / grad_points (dense [window, 3]), grad_transforms (f32 [n_inst, 3, 4],
+ *      overwritten) and grad_vertices ([n_verts_total, 3], overwritten) may each be NULL.  n_verts_total + 4 n_inst
+ *      must stay below 2^32 - 1.  rt_scene_grad_sizes: workspace for one window of n_rows, `outputs` =
+ *      RT_SCENE_GRAD_TRANSFORMS | RT_SCENE_GRAD_VERTICES as the call will request (0 bytes when neither: none is needed
+ *      then).  Workspace 256-byte aligned. */
+typedef struct rt_scene_member {
+    const float* vertices;
+    const int32_t* faces;
+    int64_t n_verts, n_faces;
+    int64_t vertex_base;
+} rt_scene_member;
+#define RT_SCENE_GRAD_TRANSFORMS 1
+#define RT_SCENE_GRAD_VERTICES 2
+int rt_scene_grad_sizes(int64_t n_rows, int64_t n_inst, int64_t n_verts_total, int outputs, size_t* workspace_bytes);
+int rt_scene_ray_grad(const void* table, int64_t n_inst, const rt_scene_member* members, int64_t n_meshes,
+                      int64_t n_verts_total, const rt_ray_desc* rays, const rt_trace_opts* opts, int64_t n_rows,
+                      const int32_t* row_ray, const int32_t* inst_idx, const int32_t* tri_idx, const float* grad_loc,
+                      const float* grad_uv, float* grad_origins, float* grad_directions, float* grad_transforms,
+                      float* grad_vertices, void* workspace, size_t workspace_bytes, void* stream);
+int rt_scene_distance_grad(const void* table, int64_t n_inst, const rt_scene_member* members, int64_t n_meshes,
+                           int64_t n_verts_total, const rt_ray_desc* points, const rt_trace_opts* opts,
+                           const float* grad_out, const float* value, const float* closest, const int32_t* inst_idx,
+                           const int32_t* tri_idx, const float* uv, float* grad_points, float* grad_transforms,
+                           float* grad_vertices, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- Host-buffer entry points (end-to-end path): rays and results live in (pinned) HOST memory.
  *      Copies ray chunks H2D, traces and copies results D2H on internal streams, overlapping
  *      the three; `dev_work` is caller-provided device memory of rt_host_closest_sizes() bytes.

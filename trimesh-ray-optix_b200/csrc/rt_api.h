@@ -8,6 +8,7 @@
 #include <stdlib.h>
 #include "../../include/raymesh_b200.h"
 #include "rt_core.cuh"
+#include "rt_distgrad.cuh"
 
 namespace rt {
 
@@ -37,6 +38,24 @@ int sort_pairs_low(uint64_t* keys, uint32_t* vals, int64_t n, void* workspace, i
                    uint32_t** vals_out, cudaStream_t stream);
 
 inline size_t align_up_sz(size_t x, size_t a) { return (x + a - 1) / a * a; }
+
+// rt_distgrad.cu: steps 2 and 3 of the deterministic per-key sums (DESIGN.md §4.9) on the m pairs at keys / vals:
+// the sort on the low 8 * passes key bits, the run starts, level 0 launched by `level0` (with grid blocks of
+// kDgThreads over the m sorted pairs, level0_arg passed through) and the further tree levels.  Each key below n_keys
+// adds its sum to grad_vertices[key]; start holds n_keys entries, lv two level buffers of dg_next_size(m) slots.
+constexpr int kDgThreads = 256;
+struct DgPairs {
+    uint64_t* keys;
+    uint32_t* vals;
+    void* sort_ws;
+    uint32_t* start;
+    DgLevel lv[2];
+};
+typedef void (*DgLevel0Launch)(const void* arg, const uint64_t* keys, const uint32_t* vals, int64_t m,
+                               const uint32_t* start, uint64_t n_keys, float* grad_vertices, DgLevel next, int grid,
+                               cudaStream_t stream);
+int dg_reduce(const DgPairs& w, int64_t m, int64_t n_keys, int passes, int sm_count, DgLevel0Launch level0,
+              const void* level0_arg, float* grad_vertices, cudaStream_t stream);
 
 // blocks for a grid-stride loop over n items: enough to cover them, at most per_sm blocks per SM
 inline int grid_for(int64_t n, int threads, int sm_count, int per_sm) {

@@ -17,8 +17,6 @@
 
 namespace rt {
 
-constexpr int kDgThreads = 256;
-
 struct DgPointParams {
     const float* points;
     int64_t shape[4], stride[4];
@@ -203,8 +201,6 @@ static DgWorkspace carve_dg(void* base, int64_t w, int64_t n_verts, bool with_w)
     return ws;
 }
 
-constexpr int64_t kDgMaxVerts = 0xffffffffll;     // vertex ids and the sentinel n_verts fit 32 bits
-
 // The largest window of at most n (and kDgMaxPoints) points whose workspace fits workspace_bytes; 0 when not even
 // one point fits.
 static int64_t dg_window(int64_t n, int64_t n_verts, bool with_w, size_t workspace_bytes) {
@@ -220,23 +216,19 @@ static int64_t dg_window(int64_t n, int64_t n_verts, bool with_w, size_t workspa
     return win;
 }
 
-// Steps 2 and 3 for one window of nw points whose pairs are in w.keys / w.vals and whose q and uv (w for hit rows)
-// are at w.q and uv: adds every vertex's sum of the window to grad_vertices.
-static int dg_reduce_window(const DgWorkspace& w, int64_t nw, int64_t n_verts, const float* uv, int passes,
-                            int sm_count, float* grad_vertices, cudaStream_t stream) {
-    const int64_t m = 3 * nw;
+int dg_reduce(const DgPairs& w, int64_t m, int64_t n_keys, int passes, int sm_count, DgLevel0Launch level0,
+              const void* level0_arg, float* grad_vertices, cudaStream_t stream) {
     uint64_t* keys = nullptr;
     uint32_t* vals = nullptr;
     const int rc = sort_pairs_low(w.keys, w.vals, m, w.sort_ws, passes, &keys, &vals, stream);
     if (rc != RT_OK) return rc;
     const int grid = grid_for(m, kDgThreads, sm_count, 8);
-    k_dg_run_start<<<grid, kDgThreads, 0, stream>>>(keys, m, (uint64_t)n_verts, w.start);
+    k_dg_run_start<<<grid, kDgThreads, 0, stream>>>(keys, m, (uint64_t)n_keys, w.start);
     // level l holds `size` slots; runs at most `len` long; it forwards into the next level while len > kDgGroup
     uint64_t size = (uint64_t)m, len = (uint64_t)m;
     int cur = 0;
     if (len > kDgGroup) RT_CUDA_TRY(cudaMemsetAsync(w.lv[0].key, 0xff, dg_next_size(size) * 4u, stream));
-    k_dg_level0<<<grid, kDgThreads, 0, stream>>>(keys, vals, m, w.start, (uint64_t)n_verts, w.q, uv, grad_vertices,
-                                                 w.lv[0]);
+    level0(level0_arg, keys, vals, m, w.start, (uint64_t)n_keys, grad_vertices, w.lv[0], grid, stream);
     RT_CUDA_TRY(cudaGetLastError());
     while (len > kDgGroup) {
         size = dg_next_size(size);
@@ -248,6 +240,24 @@ static int dg_reduce_window(const DgWorkspace& w, int64_t nw, int64_t n_verts, c
         cur ^= 1;
     }
     return RT_OK;
+}
+
+// q and uv (w for hit rows) of a window, for the level-0 launch of dg_reduce_window
+struct DgQUv { const float* q; const float* uv; };
+static void dg_level0_launch(const void* arg, const uint64_t* keys, const uint32_t* vals, int64_t m,
+                             const uint32_t* start, uint64_t n_verts, float* grad_vertices, DgLevel next, int grid,
+                             cudaStream_t stream) {
+    const DgQUv* a = static_cast<const DgQUv*>(arg);
+    k_dg_level0<<<grid, kDgThreads, 0, stream>>>(keys, vals, m, start, n_verts, a->q, a->uv, grad_vertices, next);
+}
+
+// Steps 2 and 3 for one window of nw points whose pairs are in w.keys / w.vals and whose q and uv (w for hit rows)
+// are at w.q and uv: adds every vertex's sum of the window to grad_vertices.
+static int dg_reduce_window(const DgWorkspace& w, int64_t nw, int64_t n_verts, const float* uv, int passes,
+                            int sm_count, float* grad_vertices, cudaStream_t stream) {
+    const DgPairs pairs{w.keys, w.vals, w.sort_ws, w.start, {w.lv[0], w.lv[1]}};
+    const DgQUv arg{w.q, uv};
+    return dg_reduce(pairs, 3 * nw, n_verts, passes, sm_count, dg_level0_launch, &arg, grad_vertices, stream);
 }
 
 }  // namespace rt

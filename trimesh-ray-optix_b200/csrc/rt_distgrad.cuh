@@ -17,6 +17,7 @@ namespace rt {
 constexpr uint32_t kDgGroup = 32;                     // contributions per group of the reduction tree
 constexpr uint32_t kDgEmpty = 0xffffffffu;            // key of an unused slot of a level buffer (levels >= 1)
 constexpr int64_t kDgMaxPoints = ((int64_t)1 << 30) / 3;   // 3 pairs per point must fit one sort call
+constexpr int64_t kDgMaxVerts = 0xffffffffll;              // vertex ids and the sentinel n_verts fit 32 bits
 
 // q of one point; false (and q = +0) when the point contributes nothing: value +-0, +-inf or NaN, or no triangle
 RT_HD bool dg_point_q(float px, float py, float pz, float g, float value, float cx, float cy, float cz, int32_t tri,
@@ -70,22 +71,31 @@ RT_HD void dg_group_end(uint32_t v, uint64_t j, uint32_t g, bool more, const flo
     next.val[3 * o] = s[0]; next.val[3 * o + 1] = s[1]; next.val[3 * o + 2] = s[2];
 }
 
-// Level 0 at sorted position j of m pairs: start[v] = first position of vertex v (written by dg_run_start)
-RT_HD void dg_level0_at(uint64_t j, uint64_t m, const uint64_t* keys, const uint32_t* vals, const uint32_t* start,
-                        uint64_t n_verts, const float* q, const float* uv, float* grad_vertices, DgLevel next) {
+// Level 0 at sorted position j of m pairs: start[v] = first position of vertex v (written by dg_run_start);
+// contrib(e, out) is the contribution of pair e.
+template <class Contrib>
+RT_HD void dg_level0_with(uint64_t j, uint64_t m, const uint64_t* keys, const uint32_t* vals, const uint32_t* start,
+                          uint64_t n_verts, const Contrib& contrib, float* grad_vertices, DgLevel next) {
     const uint64_t key = keys[j];
     if (key >= n_verts) return;
     const uint32_t v = (uint32_t)key;
     const uint32_t g = (uint32_t)(j - start[v]);
     if (g % kDgGroup != 0u) return;
     float s[3], c[3];
-    dg_contrib(q, uv, vals[j], s);
+    contrib(vals[j], s);
     for (uint64_t t = 1; t < kDgGroup && j + t < m && keys[j + t] == key; ++t) {
-        dg_contrib(q, uv, vals[j + t], c);
+        contrib(vals[j + t], c);
         s[0] = fadd(s[0], c[0]); s[1] = fadd(s[1], c[1]); s[2] = fadd(s[2], c[2]);
     }
     const bool more = g > 0u || (j + kDgGroup < m && keys[j + kDgGroup] == key);
     dg_group_end(v, j, g, more, s, grad_vertices, next);
+}
+
+// Level 0 of the point and hit-row sums: pair e = 3 i + k contributes -w_k q_i (dg_contrib)
+RT_HD void dg_level0_at(uint64_t j, uint64_t m, const uint64_t* keys, const uint32_t* vals, const uint32_t* start,
+                        uint64_t n_verts, const float* q, const float* uv, float* grad_vertices, DgLevel next) {
+    dg_level0_with(j, m, keys, vals, start, n_verts, [&](uint32_t e, float out[3]) { dg_contrib(q, uv, e, out); },
+                   grad_vertices, next);
 }
 
 RT_HD void dg_run_start(uint64_t j, const uint64_t* keys, uint64_t n_verts, uint32_t* start) {

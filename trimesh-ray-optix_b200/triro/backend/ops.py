@@ -119,6 +119,10 @@ def _declare(lib):
         "rt_scene_point_prepare": (ci, [vp, i64, vp, sz, vp]),
         "rt_scene_closest_point": (ci, [vp, vp, vp, prd, pto, C.c_float, vp, vp, vp, vp, vp, vp]),
         "rt_scene_signed_distance": (ci, [vp, vp, vp, vp, prd, pto, vp, vp, vp, vp, vp, vp]),
+        "rt_scene_grad_sizes": (ci, [i64, i64, i64, ci, psz]),
+        "rt_scene_ray_grad": (ci, [vp, i64, vp, i64, i64, prd, pto, i64, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]),
+        "rt_scene_distance_grad": (ci, [vp, i64, vp, i64, i64, prd, pto, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz,
+                                        vp]),
         "rt_host_closest_sizes": (ci, [i64, psz]),
         "rt_host_trace_closest": (ci, [vp, i64, vp, ci, vp, pto, vp, vp, vp, vp, vp, vp, sz]),
         "rt_host_trace_closest_compact": (ci, [vp, i64, vp, ci, vp, pto, vp, vp, vp, vp, vp, vp, C.POINTER(C.c_int64), vp, sz]),
@@ -1274,3 +1278,111 @@ def scene_distance_grad(points: torch.Tensor, grad_out: torch.Tensor, value: tor
                                                  _ptr(closest), _ptr(tri), _ptr(uv), None, int(n_faces), 0, _ptr(gp),
                                                  None, None, 0, _stream(dev)), "rt_distance_grad")
     return gp
+
+
+# ------------------------------------------------------------------ gradients on instanced scenes (DESIGN.md §4.13)
+SCENE_GRAD_TRANSFORMS, SCENE_GRAD_VERTICES = 1, 2
+
+
+def scene_members(members: list) -> tuple[torch.Tensor, int]:
+    """The device member table of rt_scene_ray_grad / rt_scene_distance_grad for [(vertices Float32[v,3], faces
+    Int32[f,3]), ...] (contiguous, on one CUDA device; the caller keeps them alive while the table is used): int64
+    [M, 5] rows (vertices address, faces address, v, f, vertex base), and the total vertex count.  A member's vertex
+    base is the sum of the vertex counts before it."""
+    rows, base = [], 0
+    for v, f in members:
+        if v.dtype != torch.float32 or not v.is_contiguous() or f.dtype != torch.int32 or not f.is_contiguous():
+            raise ValueError("member vertices must be contiguous float32 [v,3] and faces contiguous int32 [f,3]")
+        rows.append([v.data_ptr(), f.data_ptr(), v.shape[0], f.shape[0], base])
+        base += v.shape[0]
+    dev = members[0][0].device if members else torch.device("cuda", torch.cuda.current_device())
+    return torch.tensor(rows or [[0] * 5], dtype=torch.int64).to(dev), base
+
+
+def scene_grad_workspace_bytes(n_rows: int, n_inst: int, n_verts: int, outputs: int) -> int:
+    """Workspace rt_scene_ray_grad / rt_scene_distance_grad need to run n_rows rows as one window; `outputs` =
+    SCENE_GRAD_TRANSFORMS | SCENE_GRAD_VERTICES as requested."""
+    wb = C.c_size_t()
+    _check(get_module().rt_scene_grad_sizes(int(n_rows), int(n_inst), int(n_verts), int(outputs), C.byref(wb)),
+           "rt_scene_grad_sizes")
+    return wb.value
+
+
+def _scene_grad_outputs(dev, n_inst: int, n_verts: int, n_rows: int, transforms_grad: bool, vertices_grad: bool,
+                        workspace_bytes: int | None):
+    gt = torch.empty((n_inst, 3, 4), dtype=torch.float32, device=dev) if transforms_grad else None
+    gv = torch.empty((n_verts, 3), dtype=torch.float32, device=dev) if vertices_grad else None
+    outputs = (SCENE_GRAD_TRANSFORMS if transforms_grad else 0) | (SCENE_GRAD_VERTICES if vertices_grad else 0)
+    wb = 0
+    if outputs:
+        wb = scene_grad_workspace_bytes(n_rows, n_inst, n_verts, outputs) if workspace_bytes is None else int(workspace_bytes)
+    ws = torch.empty(max(wb, 256), dtype=torch.uint8, device=dev) if outputs else None
+    return gt, gv, ws, wb
+
+
+def _scene_member_args(table: torch.Tensor, n_inst: int, members: torch.Tensor, n_verts: int, dev):
+    if table.device != dev or members.device != dev or members.dtype != torch.int64 or members.dim() != 2:
+        raise ValueError(f"the scene table and the member table must be on {dev}")
+    return _ptr(table), int(n_inst), _ptr(members), members.shape[0], int(n_verts)
+
+
+def scene_ray_grad(table: torch.Tensor, n_inst: int, members: torch.Tensor, n_verts: int, origins: torch.Tensor,
+                   dirs: torch.Tensor, inst: torch.Tensor, tri: torch.Tensor, grad_loc: torch.Tensor | None,
+                   grad_uv: torch.Tensor | None, ray_idx: torch.Tensor | None = None, origins_grad: bool = True,
+                   directions_grad: bool = True, transforms_grad: bool = True, vertices_grad: bool = True,
+                   workspace_bytes: int | None = None):
+    """Backward of RayMeshScene.intersects_closest's loc and uv (rt_scene_ray_grad): (grad_origins Float32[*b,3],
+    grad_directions Float32[*b,3], grad_transforms Float32[I,3,4], grad_vertices Float32[n_verts,3]), each None when
+    not asked for.  Row i is the hit of (inst[i], tri[i]) by ray ray_idx[i] (None: ray i) of the flattened batch;
+    `members` and n_verts come from scene_members.  Each row recomputes its hit on the world triangle (DESIGN.md
+    §4.13); sums are deterministic to the bit.  `workspace_bytes` bounds the workspace (default: one window)."""
+    tensor_input_check(origins, dirs)
+    rd, batch = make_ray_desc(origins, dirs)
+    dev = origins.device
+    h = tri.shape[0] if tri.dim() == 1 else -1
+    if ray_idx is None and h != rd.nray:
+        raise ValueError(f"tri must have one row per ray ({rd.nray}) without ray_idx, got {tuple(tri.shape)}")
+    for name, t, shape, dt in (("inst", inst, (h,), torch.int32), ("tri", tri, (h,), torch.int32),
+                               ("grad_loc", grad_loc, (h, 3), torch.float32), ("grad_uv", grad_uv, (h, 2), torch.float32),
+                               ("ray_idx", ray_idx, (h,), torch.int32)):
+        if t is not None and (tuple(t.shape) != shape or t.dtype != dt or t.device != dev):
+            raise ValueError(f"{name} must be {dt} {shape} on {dev}, got {t.dtype} {tuple(t.shape)} on {t.device}")
+    scene = _scene_member_args(table, n_inst, members, n_verts, dev)
+    inst, tri, grad_loc, grad_uv, ray_idx = (None if t is None else t.contiguous() for t in
+                                             (inst, tri, grad_loc, grad_uv, ray_idx))
+    with _on_device(dev):
+        go = torch.empty((*batch, 3), dtype=torch.float32, device=dev) if origins_grad else None
+        gd = torch.empty((*batch, 3), dtype=torch.float32, device=dev) if directions_grad else None
+        gt, gv, ws, wb = _scene_grad_outputs(dev, n_inst, n_verts, h, transforms_grad, vertices_grad, workspace_bytes)
+        _check(get_module().rt_scene_ray_grad(*scene, C.byref(rd), C.byref(trace_opts()), h, _ptr(ray_idx), _ptr(inst),
+                                              _ptr(tri), _ptr(grad_loc), _ptr(grad_uv), _ptr(go), _ptr(gd), _ptr(gt),
+                                              _ptr(gv), _ptr(ws), wb, _stream(dev)), "rt_scene_ray_grad")
+    return go, gd, gt, gv
+
+
+def scene_point_grad(table: torch.Tensor, n_inst: int, members: torch.Tensor, n_verts: int, points: torch.Tensor,
+                     grad_out: torch.Tensor, value: torch.Tensor, closest: torch.Tensor, inst: torch.Tensor,
+                     tri: torch.Tensor, uv: torch.Tensor, points_grad: bool = True, transforms_grad: bool = True,
+                     vertices_grad: bool = True, workspace_bytes: int | None = None):
+    """Backward of RayMeshScene.closest_point's distance or signed_distance (rt_scene_distance_grad) from the forward's
+    outputs: (grad_points Float32[*b,3], grad_transforms Float32[I,3,4], grad_vertices Float32[n_verts,3]), each None
+    when not asked for (DESIGN.md §4.13)."""
+    tensor_input_check(points)
+    rd, batch = make_ray_desc(points, None)
+    dev = points.device
+    for name, t, shape, dt in (("grad_out", grad_out, batch, torch.float32), ("value", value, batch, torch.float32),
+                               ("closest", closest, (*batch, 3), torch.float32), ("inst", inst, batch, torch.int32),
+                               ("tri", tri, batch, torch.int32), ("uv", uv, (*batch, 2), torch.float32)):
+        if tuple(t.shape) != tuple(shape) or t.dtype != dt or t.device != dev:
+            raise ValueError(f"{name} must be {dt} {tuple(shape)} on {dev}, got {t.dtype} {tuple(t.shape)} on {t.device}")
+    scene = _scene_member_args(table, n_inst, members, n_verts, dev)
+    grad_out, value, closest, inst, tri, uv = (t.contiguous() for t in (grad_out, value, closest, inst, tri, uv))
+    with _on_device(dev):
+        gp = torch.empty((*batch, 3), dtype=torch.float32, device=dev) if points_grad else None
+        gt, gv, ws, wb = _scene_grad_outputs(dev, n_inst, n_verts, rd.nray, transforms_grad, vertices_grad,
+                                             workspace_bytes)
+        _check(get_module().rt_scene_distance_grad(*scene, C.byref(rd), C.byref(trace_opts()), _ptr(grad_out),
+                                                   _ptr(value), _ptr(closest), _ptr(inst), _ptr(tri), _ptr(uv), _ptr(gp),
+                                                   _ptr(gt), _ptr(gv), _ptr(ws), wb, _stream(dev)),
+               "rt_scene_distance_grad")
+    return gp, gt, gv

@@ -1,10 +1,15 @@
 """RayMeshScene — closest, any and count ray queries against many instances of meshes, each instance with its own
 affine transform, in one launch (the instance acceleration structures of OptiX, which the reference never exposed).
 
-Point queries: `closest_point` and the pseudo-normal `signed_distance` over every instance in one launch, the
-distance and the signed value differentiable with respect to the points (DESIGN.md §4.12).
+Point queries: `closest_point` and the pseudo-normal `signed_distance` over every instance in one launch (DESIGN.md
+§4.12).
 
-Out of scope: ray gradients, gradients with respect to transforms or member vertices, all-hits
+Gradients (DESIGN.md §4.13): `intersects_closest`'s `loc` and `uv` with respect to the rays, and the point queries'
+distance and signed value with respect to the points, are also differentiable with respect to the transforms last
+given to `update()` and every member's `mesh_vertices`, so poses can be fitted to point clouds or depth images
+without flattening the scene.
+
+Out of scope: gradients with respect to tmax or max_distance, visibility (edge) gradients, all-hits
 (`intersects_location` / `intersects_id`), `contains_points`, winding numbers and the winding or contains signs,
 `triro.distributed` and the numpy adapter.  Query a member `RayMeshIntersector` for those.
 """
@@ -33,7 +38,15 @@ class RayMeshScene:
     Culling uses padded world boxes; DESIGN.md §4.11 gives the padding and the ray origins (|o|inf at most 32 times
     the instance's reach from the world origin) for which it provably drops no hit.  The member intersectors are
     not watched: after `refit` or `update_raw` of a member, or new transforms, call `update()`; a query raises until
-    then.  The ray queries are not differentiable; no all-hits or containment queries (see the module docstring).
+    then.  No all-hits or containment queries (see the module docstring).
+
+    Gradients: when `transforms` is a tensor that requires grad, the scene keeps a differentiable handle on it (the
+    [:, :3, :] view of a 4x4, as float32), and the closest hit and the point queries return gradients to it in its own
+    shape, dtype and device (a 4x4's last row gets 0).  Every member's `mesh_vertices` is an autograd input too.  A
+    query's backward uses the table and the member tensors as of that query, so a backward after `update()` still
+    differentiates the pose the forward saw.  After an in-place change of grad-requiring transforms (an optimiser
+    step) call `update(transforms)` again: a query raises until then, rather than differentiate a pose the scene does
+    not show.
     """
 
     def __init__(self, meshes, instance_mesh, transforms, tmax: float = hops.TMAX_DEFAULT):
@@ -47,6 +60,9 @@ class RayMeshScene:
         self.device = devs.pop() if devs else torch.device("cuda", torch.cuda.current_device())
         self.instance_mesh = torch.as_tensor(instance_mesh).reshape(-1).to("cpu", torch.int64)
         self.transforms = None
+        self._transforms_src = None      # what update() was last given (the autograd input), and its version
+        self._transforms_version = 0
+        self._member_table = None        # (key, device table, total vertex count), see _grad_members()
         self.update(transforms)
 
     @staticmethod
@@ -77,6 +93,9 @@ class RayMeshScene:
         transforms when given.  The meshes' own trees are not touched: refit or rebuild them first."""
         n = self.instance_mesh.numel()
         t = self.transforms if transforms is None else self._transforms(transforms, n)
+        if transforms is not None:
+            src = transforms if isinstance(transforms, torch.Tensor) else None
+            self._transforms_src, self._transforms_version = src, (src._version if src is not None else 0)
         if n and (int(self.instance_mesh.min()) < 0 or int(self.instance_mesh.max()) >= len(self.meshes)):
             raise ValueError(f"instance_mesh must index the {len(self.meshes)} meshes")
         blobs = [m.as_wrapper.blob for m in self.meshes]
@@ -93,6 +112,38 @@ class RayMeshScene:
             if inner.blob is not blob or inner.generation != gen:
                 raise RuntimeError(f"mesh {k} of the scene was rebuilt or re-fitted since the last update(): call "
                                    "scene.update() so that the instance boxes follow it")
+        src = self._transforms_src
+        if src is not None and src.requires_grad and src._version != self._transforms_version:
+            raise RuntimeError("the transforms given to update() were modified in place since (an optimiser step?): "
+                               "call scene.update(transforms) so that the scene shows the pose being differentiated")
+
+    # ------------------------------------------------------------------ gradients (DESIGN.md §4.13)
+    def _transforms_handle(self):
+        """The float32 [I,3,4] autograd handle of the transforms last given to update(), or None when they do not
+        require grad.  Its values are those of the table (_check_current guards the version)."""
+        src = self._transforms_src
+        if src is None or not src.requires_grad or not torch.is_grad_enabled():
+            return None
+        return (src[:, :3, :] if src.shape[1] == 4 else src).to(torch.float32)
+
+    def _vertices(self) -> list:
+        return [m.mesh_vertices for m in self.meshes]
+
+    def _tracks_grad(self, *tensors) -> bool:
+        src = self._transforms_src
+        return torch.is_grad_enabled() and (any(t.requires_grad for t in tensors)
+                                            or (src is not None and src.requires_grad)
+                                            or any(v.requires_grad for v in self._vertices()))
+
+    def _grad_members(self):
+        """(device member table, total vertex count, the member tensors it points to) for the current members; cached
+        on the scene until a member's tensors change."""
+        tensors = [(m.mesh_vertices.detach(), m.mesh_faces) for m in self.meshes]
+        key = tuple((v.data_ptr(), v.shape[0], f.data_ptr(), f.shape[0]) for v, f in tensors)
+        if self._member_table is None or self._member_table[0] != key:
+            table, n_verts = hops.scene_members(tensors)
+            self._member_table = (key, table, n_verts, tensors)
+        return self._member_table[1:]
 
     def _trace(self, origins, directions, mode):
         self._check_current()
@@ -103,7 +154,18 @@ class RayMeshScene:
 
         stream_compaction=False -> (hit[*b], front[*b], inst_idx[*b], tri_idx[*b], loc[*b,3], uv[*b,2])
         stream_compaction=True  -> (hit[*b], front[h], ray_idx[h], inst_idx[h], tri_idx[h], loc[h,3], uv[h,2])
-        Misses: inst_idx = tri_idx = -1, loc and uv 0."""
+        Misses: inst_idx = tri_idx = -1, loc and uv 0.
+
+        `loc` and `uv` are differentiable with respect to `origins`, `directions`, the transforms last given to
+        `update()` and every member's `mesh_vertices`: the gradient of the hit inside the visible triangle, recomputed
+        on the world triangle A v + b of the forward's pose and vertices (DESIGN.md §4.13).  Visibility changes
+        contribute nothing: a silhouette, an occlusion boundary or a hit that would move to another triangle or
+        instance has no gradient.  Misses and degenerate triangles give 0.  `hit`, `front`, `ray_idx`, `inst_idx` and
+        `tri_idx` are not differentiable.  Nothing of this runs unless grad mode is on and one of those requires grad;
+        the gradients are deterministic to the bit."""
+        if self._tracks_grad(origins, directions):
+            return _SceneClosestHitFn.apply(self, stream_compaction, origins, directions, self._transforms_handle(),
+                                            *self._vertices())
         hit, front, inst, tri, loc, uv = self._trace(origins, directions, hops.SCENE_CLOSEST)
         if stream_compaction:
             front_c, ray_idx, tri_c, loc_c, uv_c = hops.compact_closest(hit, front, tri, loc, uv)
@@ -145,13 +207,16 @@ class RayMeshScene:
         survive affine maps, so the mesh's `interpolate` works).  A point with nothing in reach gets inst_idx =
         triangle_id = -1, distance inf, closest and uv 0.
 
-        `distance` is differentiable with respect to `points`: (p - closest) / distance, 0 where the distance is 0 or
-        inf.  There is no gradient with respect to the transforms or the member vertices."""
+        `distance` is differentiable with respect to `points` ((p - closest) / distance, 0 where the distance is 0 or
+        inf), the transforms last given to `update()` and every member's `mesh_vertices`: the gradient of the distance
+        to the closest point, held at its triangle and barycentrics (DESIGN.md §4.13).  A closest point that would
+        move to another triangle or instance contributes nothing beyond that."""
         self._check_current()
         md = float("inf") if max_distance is None else float(max_distance)
         side, _ = self._point_state(False)
-        if torch.is_grad_enabled() and points.requires_grad:
-            closest, distance, inst, tri, uv = _SceneClosestPointFn.apply(points, self, side, md)
+        if self._tracks_grad(points):
+            closest, distance, inst, tri, uv = _SceneClosestPointFn.apply(points, self, side, md,
+                                                                          self._transforms_handle(), *self._vertices())
         else:
             closest, distance, inst, tri, uv = hops.scene_closest_point(self._table, self._tlas, side, points, md)
         if return_uv:
@@ -171,53 +236,128 @@ class RayMeshScene:
         wrong near those features; where instances overlap it is the sign of the closest feature's instance, not of
         the union.  It is always defined and deterministic.  Only sign="pseudonormal" exists on scenes.
 
-        Differentiable with respect to `points` like `closest_point`'s distance; not with respect to the transforms
-        or the member vertices."""
+        Differentiable like `closest_point`'s distance, with respect to `points`, the transforms and every member's
+        `mesh_vertices`; the sign is held."""
         if sign != "pseudonormal":
             raise ValueError(f'only sign="pseudonormal" is supported on scenes (got {sign!r})')
         self._check_current()
         side, normals = self._point_state(True)
-        if torch.is_grad_enabled() and points.requires_grad:
-            return _SceneSignedDistanceFn.apply(points, self, side, normals)
+        if self._tracks_grad(points):
+            return _SceneSignedDistanceFn.apply(points, self, side, normals, self._transforms_handle(),
+                                                *self._vertices())
         return hops.scene_signed_distance(self._table, self._tlas, side, normals, points)
 
 
+def _save_scene(ctx, scene):
+    """What the backward needs of the scene as of the forward: the table, the member table and its tensors."""
+    ctx.table = scene._table
+    ctx.n_inst = scene.instance_mesh.numel()
+    ctx.members, ctx.n_verts, ctx.member_tensors = scene._grad_members()
+
+
+def _split_vertices(ctx, gv, first: int):
+    """grad_vertices [n_verts,3] as one gradient per member input (ctx.needs_input_grad[first:])"""
+    out, base = [], 0
+    for k, (v, _) in enumerate(ctx.member_tensors):
+        n = v.shape[0]
+        out.append(gv[base:base + n] if gv is not None and ctx.needs_input_grad[first + k] else None)
+        base += n
+    return out
+
+
+def _transforms_grad(ctx, gt):
+    """grad_transforms on the device of the transforms handle (autograd chains it back to what update() was given)"""
+    return None if gt is None else gt.to(ctx.transforms_device)
+
+
 def _scene_distance_backward(ctx, grad_value):
-    points, value, closest, tri, uv = ctx.saved_tensors
-    return hops.scene_distance_grad(points.detach(), grad_value, value, closest, tri, uv, ctx.n_faces)
+    """(grad_points, grad_transforms, grad_vertices per member) of a scene distance or signed distance; inputs
+    (points, scene, side, extra, transforms, *vertices)"""
+    points, value, closest, inst, tri, uv = ctx.saved_tensors
+    need = ctx.needs_input_grad
+    want_t, want_v = need[4], any(need[5:])
+    if not want_t and not want_v:
+        gp = hops.scene_distance_grad(points.detach(), grad_value, value, closest, tri, uv, ctx.n_faces)
+        return gp, None, [None] * len(ctx.member_tensors)
+    gp, gt, gv = hops.scene_point_grad(ctx.table, ctx.n_inst, ctx.members, ctx.n_verts, points.detach(), grad_value,
+                                       value, closest, inst, tri, uv, points_grad=need[0], transforms_grad=want_t,
+                                       vertices_grad=want_v)
+    return gp, _transforms_grad(ctx, gt), _split_vertices(ctx, gv, 5)
+
+
+def _save_point_forward(ctx, scene, transforms, points, value, closest, inst, tri, uv):
+    ctx.save_for_backward(points, value, closest, inst, tri, uv)
+    ctx.n_faces = scene._n_faces()
+    ctx.transforms_device = None if transforms is None else transforms.device
+    _save_scene(ctx, scene)
 
 
 class _SceneClosestPointFn(torch.autograd.Function):
-    """RayMeshScene.closest_point with a distance differentiable with respect to the points."""
+    """RayMeshScene.closest_point with a distance differentiable with respect to the points, the transforms handle
+    and the members' vertices (DESIGN.md §4.13); those are only autograd inputs, the forward walks the scene."""
 
     @staticmethod
-    def forward(ctx, points, scene, side, max_distance):
+    def forward(ctx, points, scene, side, max_distance, transforms, *vertices):
         out = hops.scene_closest_point(scene._table, scene._tlas, side, points.detach(), max_distance)
         closest, distance, inst, tri, uv = out
         ctx.mark_non_differentiable(closest, inst, tri, uv)
-        ctx.save_for_backward(points, distance, closest, tri, uv)
-        ctx.n_faces = scene._n_faces()
+        _save_point_forward(ctx, scene, transforms, points, distance, closest, inst, tri, uv)
         return out
 
     @staticmethod
     @once_differentiable
     def backward(ctx, grad_closest, grad_distance, grad_inst, grad_tri, grad_uv):
-        return _scene_distance_backward(ctx, grad_distance), None, None, None
+        gp, gt, gv = _scene_distance_backward(ctx, grad_distance)
+        return gp, None, None, None, gt, *gv
 
 
 class _SceneSignedDistanceFn(torch.autograd.Function):
-    """RayMeshScene.signed_distance with its gradient with respect to the points: one walk gives the sign and the
-    closest feature."""
+    """RayMeshScene.signed_distance with its gradient with respect to the points, the transforms handle and the
+    members' vertices: one walk gives the sign and the closest feature."""
 
     @staticmethod
-    def forward(ctx, points, scene, side, normals):
-        sd, closest, _, tri, uv = hops.scene_signed_distance(scene._table, scene._tlas, side, normals, points.detach(),
-                                                             return_closest=True)
-        ctx.save_for_backward(points, sd, closest, tri, uv)
-        ctx.n_faces = scene._n_faces()
+    def forward(ctx, points, scene, side, normals, transforms, *vertices):
+        sd, closest, inst, tri, uv = hops.scene_signed_distance(scene._table, scene._tlas, side, normals,
+                                                                points.detach(), return_closest=True)
+        _save_point_forward(ctx, scene, transforms, points, sd, closest, inst, tri, uv)
         return sd
 
     @staticmethod
     @once_differentiable
     def backward(ctx, grad_sd):
-        return _scene_distance_backward(ctx, grad_sd), None, None, None
+        gp, gt, gv = _scene_distance_backward(ctx, grad_sd)
+        return gp, None, None, None, gt, *gv
+
+
+class _SceneClosestHitFn(torch.autograd.Function):
+    """RayMeshScene.intersects_closest with differentiable loc and uv (DESIGN.md §4.13), dense or compacted; inputs
+    (scene, compaction, origins, dirs, transforms handle or None, *member vertices)."""
+
+    @staticmethod
+    def forward(ctx, scene, compaction, origins, dirs, transforms, *vertices):
+        hit, front, inst, tri, loc, uv = scene._trace(origins.detach(), dirs.detach(), hops.SCENE_CLOSEST)
+        ray_idx = None
+        if compaction:
+            front, ray_idx, tri, loc, uv = hops.compact_closest(hit, front, tri, loc, uv)
+            inst = inst.reshape(-1)[ray_idx.long()]
+        ctx.mark_non_differentiable(*(t for t in (hit, front, ray_idx, inst, tri) if t is not None))
+        ctx.save_for_backward(origins, dirs, inst, tri, ray_idx)
+        ctx.transforms_device = None if transforms is None else transforms.device
+        _save_scene(ctx, scene)
+        if compaction:
+            return hit, front, ray_idx, inst, tri, loc, uv
+        return hit, front, inst, tri, loc, uv
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, *grads):
+        origins, dirs, inst, tri, ray_idx = ctx.saved_tensors
+        need = ctx.needs_input_grad
+        h = tri.numel()
+        grad_loc, grad_uv = grads[-2], grads[-1]
+        go, gd, gt, gv = hops.scene_ray_grad(ctx.table, ctx.n_inst, ctx.members, ctx.n_verts, origins.detach(),
+                                             dirs.detach(), inst.reshape(h), tri.reshape(h), grad_loc.reshape(h, 3),
+                                             None if grad_uv is None else grad_uv.reshape(h, 2), ray_idx=ray_idx,
+                                             origins_grad=need[2], directions_grad=need[3], transforms_grad=need[4],
+                                             vertices_grad=any(need[5:]))
+        return None, None, go, gd, _transforms_grad(ctx, gt), *_split_vertices(ctx, gv, 5)
