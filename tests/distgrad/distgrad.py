@@ -16,19 +16,22 @@ _SIM = None
 GROUP = 32          # rt_distgrad.cuh kDgGroup
 
 
-def _stale(so, deps):
-    return not os.path.exists(so) or any(os.path.getmtime(so) < os.path.getmtime(d) for d in deps)
+def compile_sim(src: str, headers, force: bool = False) -> str:
+    """Compile the simulator source `src` (a .cpp path) to lib<name>.so (g++) next to it, when the library is missing or
+    older than the source, dgreduce.h or the csrc `headers` it includes."""
+    here, name = os.path.split(os.path.abspath(src))
+    so = os.path.join(here, "lib" + name[:-len(".cpp")] + ".so")
+    deps = [src, os.path.join(_HERE, "dgreduce.h")] + [os.path.join(_CSRC, f) for f in headers]
+    if force or not os.path.exists(so) or any(os.path.getmtime(so) < os.path.getmtime(d) for d in deps):
+        cxx = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++"
+        subprocess.check_call([cxx, "-O2", "-std=c++17", "-ffp-contract=off", "-mfma", "-shared", "-fPIC",
+                               "-Wno-unknown-pragmas", "-I", os.path.join(_HERE, "..", "..", "include"), src, "-o", so])
+    return so
 
 
 def build(force: bool = False) -> str:
     """Compile libdgsim.so (g++) next to this file."""
-    so = os.path.join(_HERE, "libdgsim.so")
-    deps = [os.path.join(_HERE, "dgsim.cpp")] + [os.path.join(_CSRC, f) for f in ("rt_core.cuh", "rt_distgrad.cuh")]
-    if force or _stale(so, deps):
-        cxx = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++"
-        subprocess.check_call([cxx, "-O2", "-std=c++17", "-ffp-contract=off", "-mfma", "-shared", "-fPIC",
-                               "-Wno-unknown-pragmas", deps[0], "-o", so])
-    return so
+    return compile_sim(os.path.join(_HERE, "dgsim.cpp"), ("rt_core.cuh", "rt_distgrad.cuh"), force)
 
 
 def _lib():
@@ -79,6 +82,27 @@ def reference(points, g, value, closest, tri, uv, faces, n_verts: int):
     for k in range(3):
         np.add.at(gv, f[tri[live], k], -w[live, k:k + 1] * q[live])
     return q, gv
+
+
+def documented_order(q, w, live, tri, faces, n_verts: int, window: int):
+    """grad_vertices in float32 numpy following DESIGN.md §4.9 for rows with factors q [n,3] and weights w [n,2] (uv,
+    or w of hit rows): per window of `window` rows (0: one window), each vertex's contributions -w_k q of the live
+    rows in (row, corner) order through tree_sum, added to a +0 start in window order"""
+    out = np.zeros((n_verts, 3), np.float32)
+    n = len(q)
+    window = window or n
+    for base in range(0, n, window):
+        lists = {}
+        for i in range(base, min(n, base + window)):
+            if not live[i]:
+                continue
+            u0, u1 = np.float32(w[i, 0]), np.float32(w[i, 1])
+            ws = (u0, u1, np.float32(np.float32(np.float32(1) - u0) - u1))
+            for k in range(3):
+                lists.setdefault(int(faces[tri[i], k]), []).append((-ws[k] * q[i]).astype(np.float32))
+        for vtx, cs in lists.items():
+            out[vtx] = (out[vtx] + tree_sum(np.asarray(cs))).astype(np.float32)
+    return out
 
 
 def tree_sum(c: np.ndarray) -> np.ndarray:

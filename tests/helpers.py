@@ -16,6 +16,16 @@ def assert_bits_equal(a, b, what=""):
     assert not bad.any(), f"{what}: {int(bad.sum())} of {bad.size} elements differ (first at {np.argwhere(bad)[0]})"
 
 
+def window_of(n, sizes_fn, workspace_bytes):
+    """The window a gradient entry point picks for n rows: the largest number of rows, at most n, whose workspace
+    sizes_fn(rows) fits workspace_bytes."""
+    lo, hi = 0, n + 1
+    while hi - lo > 1:
+        mid = (lo + hi) // 2
+        lo, hi = (mid, hi) if sizes_fn(mid) <= workspace_bytes else (lo, mid)
+    return lo
+
+
 def closest_to_numpy(res):
     hit, front, tri, loc, uv = res
     return dict(hit=hit.cpu().numpy().reshape(-1).astype(np.uint8), front=front.cpu().numpy().reshape(-1).astype(np.uint8),

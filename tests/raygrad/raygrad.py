@@ -6,29 +6,21 @@ from __future__ import annotations
 
 import ctypes as C
 import os
-import subprocess
+import sys
 
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-_CSRC = os.path.join(_HERE, "..", "..", "trimesh-ray-optix_b200", "csrc")
+sys.path.insert(0, os.path.join(_HERE, "..", "distgrad"))
+import distgrad  # noqa: E402
+
 _SIM = None
-
-
-def _stale(so, deps):
-    return not os.path.exists(so) or any(os.path.getmtime(so) < os.path.getmtime(d) for d in deps)
 
 
 def build(force: bool = False) -> str:
     """Compile librgsim.so (g++) next to this file."""
-    so = os.path.join(_HERE, "librgsim.so")
-    deps = [os.path.join(_HERE, "rgsim.cpp")] + [os.path.join(_CSRC, f) for f in
-                                                  ("rt_core.cuh", "rt_distgrad.cuh", "rt_raygrad.cuh")]
-    if force or _stale(so, deps):
-        cxx = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++"
-        subprocess.check_call([cxx, "-O2", "-std=c++17", "-ffp-contract=off", "-mfma", "-shared", "-fPIC",
-                               "-Wno-unknown-pragmas", deps[0], "-o", so])
-    return so
+    return distgrad.compile_sim(os.path.join(_HERE, "rgsim.cpp"), ("rt_core.cuh", "rt_distgrad.cuh", "rt_raygrad.cuh"),
+                                force)
 
 
 def _lib():

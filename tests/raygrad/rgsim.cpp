@@ -1,12 +1,12 @@
 // rgsim.cpp — TEST INFRASTRUCTURE ONLY.  Runs the hit gradient of rt_ray_grad (rt_distgrad.cu) on the CPU with its own
-// RT_HD functions (rt_raygrad.cuh, rt_distgrad.cuh), row window by row window, with std::stable_sort in place of the
-// onesweep sort: a stable sort of the same keys yields the same permutation.  Never linked into libtriro_b200.so.
+// RT_HD functions (rt_raygrad.cuh, rt_distgrad.cuh), row window by row window, with the host reduction of
+// tests/distgrad/dgreduce.h.  Never linked into libtriro_b200.so.
 //
 // Build: g++ -O2 -std=c++17 -ffp-contract=off -mfma -shared -fPIC rgsim.cpp -o librgsim.so
 #include <algorithm>
-#include <numeric>
 #include <vector>
 #include "../../trimesh-ray-optix_b200/csrc/rt_raygrad.cuh"
+#include "../distgrad/dgreduce.h"
 
 using namespace rt;
 
@@ -73,30 +73,8 @@ extern "C" int rg_grad(int64_t n_rays, const float* o, const float* d, int64_t n
             w[2 * i] = r.w[0]; w[2 * i + 1] = r.w[1];
             for (uint32_t k = 0; k < 3; ++k) key[3 * i + k] = dg_key(live, faces, tri[base + i], k, n_verts);
         }
-        // steps 2 and 3, as tests/distgrad/dgsim.cpp
-        std::vector<uint32_t> vals(m);
-        std::iota(vals.begin(), vals.end(), 0u);
-        std::stable_sort(vals.begin(), vals.end(), [&](uint32_t a, uint32_t b) { return key[a] < key[b]; });
-        std::vector<uint64_t> keys(m);
-        for (int64_t j = 0; j < m; ++j) keys[j] = key[vals[j]];
-        std::vector<uint32_t> start(n_verts);
-        for (int64_t j = 0; j < m; ++j) dg_run_start(j, keys.data(), n_verts, start.data());
-        const uint64_t slots = dg_next_size(m);
-        std::vector<uint32_t> lk[2], li[2];
-        std::vector<float> lv[2];
-        for (int b = 0; b < 2; ++b) { lk[b].assign(slots, kDgEmpty); li[b].assign(slots, 0); lv[b].assign(3 * slots, 0.0f); }
-        DgLevel lev[2] = {{lk[0].data(), li[0].data(), lv[0].data()}, {lk[1].data(), li[1].data(), lv[1].data()}};
-        for (int64_t j = 0; j < m; ++j)
-            dg_level0_at(j, m, keys.data(), vals.data(), start.data(), n_verts, q.data(), w.data(), grad_vertices, lev[0]);
-        uint64_t size = m, len = m;
-        int cur = 0;
-        while (len > kDgGroup) {
-            size = dg_next_size(size);
-            len = (len + kDgGroup - 1) / kDgGroup;
-            std::fill(lk[cur ^ 1].begin(), lk[cur ^ 1].end(), kDgEmpty);
-            for (uint64_t j = 0; j < size; ++j) dg_level_at(j, size, lev[cur], grad_vertices, lev[cur ^ 1]);
-            cur ^= 1;
-        }
+        dg_reduce_host(key, n_verts, [&](uint32_t e, float out[3]) { dg_contrib(q.data(), w.data(), e, out); },
+                       grad_vertices);
     }
     return 0;
 }

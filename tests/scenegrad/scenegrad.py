@@ -1,5 +1,5 @@
 """Instanced-scene gradient test infrastructure: the ctypes front end of sgsim.cpp (host simulator of
-rt_scene_grad.cu) on a table prepared by tests/scene, and a numpy restatement of the contract of DESIGN.md §4.13
+rt_distgrad.cu) on a table prepared by tests/scene, and a numpy restatement of the contract of DESIGN.md §4.13
 (binary32 per-row arithmetic written out in numpy, and distgrad's fixed tree order).  TEST INFRASTRUCTURE ONLY:
 tests, tools and __graft_entry__ import it, the product never does.
 """
@@ -7,15 +7,16 @@ from __future__ import annotations
 
 import ctypes as C
 import os
-import subprocess
 import sys
 
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-_CSRC = os.path.join(_HERE, "..", "..", "trimesh-ray-optix_b200", "csrc")
 sys.path.insert(0, os.path.join(_HERE, "..", "scene"))
+sys.path.insert(0, os.path.join(_HERE, "..", "distgrad"))
+import distgrad  # noqa: E402
 import scene  # noqa: E402
+from distgrad import tree_sum  # noqa: E402,F401
 
 _SIM = None
 TRANSFORMS, VERTICES = 1, 2
@@ -23,16 +24,8 @@ TRANSFORMS, VERTICES = 1, 2
 
 def build(force: bool = False) -> str:
     """Compile libsgsim.so (g++) next to this file."""
-    so = os.path.join(_HERE, "libsgsim.so")
-    deps = [os.path.join(_HERE, "sgsim.cpp")] + [os.path.join(_CSRC, f) for f in
-                                                 ("rt_core.cuh", "rt_distgrad.cuh", "rt_raygrad.cuh", "rt_scene.cuh",
-                                                  "rt_scenegrad.cuh")]
-    if force or not os.path.exists(so) or any(os.path.getmtime(so) < os.path.getmtime(d) for d in deps):
-        cxx = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++"
-        subprocess.check_call([cxx, "-O2", "-std=c++17", "-ffp-contract=off", "-mfma", "-shared", "-fPIC",
-                               "-Wno-unknown-pragmas", "-I", os.path.join(_HERE, "..", "..", "include"), deps[0],
-                               "-o", so])
-    return so
+    return distgrad.compile_sim(os.path.join(_HERE, "sgsim.cpp"), ("rt_core.cuh", "rt_distgrad.cuh", "rt_raygrad.cuh",
+                                                                   "rt_scene.cuh", "rt_scenegrad.cuh"), force)
 
 
 def _lib():
@@ -124,21 +117,6 @@ def _affine_row(m0, m1, m2, c, x, y, z):
     for m, v in ((m2, z), (m1, y), (m0, x)):
         if m != 0:
             acc = np.float32(np.float64(m) * np.float64(v) + np.float64(acc))
-    return acc
-
-
-def tree_sum(contribs: np.ndarray) -> np.ndarray:
-    """distgrad's fixed order for one key's list [n,3] float32: groups of 32 left to right, level after level"""
-    s = np.asarray(contribs, np.float32)
-    while len(s) > 32:
-        s = np.stack([_left_sum(s[i:i + 32]) for i in range(0, len(s), 32)])
-    return _left_sum(s)
-
-
-def _left_sum(g):
-    acc = g[0].copy()
-    for r in g[1:]:
-        acc = (acc + r).astype(np.float32)
     return acc
 
 

@@ -1,15 +1,14 @@
-// sgsim.cpp — TEST INFRASTRUCTURE ONLY.  Runs the instanced-scene gradients of rt_scene_grad.cu on the CPU with their
-// own RT_HD functions (rt_scenegrad.cuh, rt_raygrad.cuh, rt_distgrad.cuh), row window by row window, with
-// std::stable_sort in place of the onesweep sort: a stable sort of the same keys yields the same permutation.  The scene
-// table comes from tests/scene (ss_prepare) and the member table holds host addresses.  Never linked into
-// libtriro_b200.so.
+// sgsim.cpp — TEST INFRASTRUCTURE ONLY.  Runs the instanced-scene gradients of rt_distgrad.cu on the CPU with their
+// own RT_HD functions (rt_scenegrad.cuh, rt_raygrad.cuh, rt_distgrad.cuh), row window by row window, with the host
+// reduction of tests/distgrad/dgreduce.h.  The scene table comes from tests/scene (ss_prepare) and the member table
+// holds host addresses.  Never linked into libtriro_b200.so.
 //
 // Build: g++ -O2 -std=c++17 -ffp-contract=off -mfma -shared -fPIC sgsim.cpp -o libsgsim.so
 #include <algorithm>
 #include <functional>
-#include <numeric>
 #include <vector>
 #include "../../trimesh-ray-optix_b200/csrc/rt_scenegrad.cuh"
+#include "../distgrad/dgreduce.h"
 
 using namespace rt;
 
@@ -17,7 +16,7 @@ namespace {
 // one row of a window: writes its factors and keys; returns nothing (dead rows write +0 and sentinel keys)
 using RowFn = std::function<void(int64_t row, SgRow& r, bool& live, uint64_t key[3], int32_t& inst)>;
 
-// steps 1 (pairs), 2 and 3 of every window, then the outputs, as sg_run does
+// steps 1 (pairs), 2 and 3 of every window, then the outputs, as rt_distgrad.cu's sg_run does
 void reduce(int64_t n_rows, int64_t n_inst, int64_t n_verts, int outputs, int64_t window, const RowFn& row,
             float* grad_transforms, float* grad_vertices) {
     const bool want_t = (outputs & 1) != 0, want_v = (outputs & 2) != 0;
@@ -40,31 +39,8 @@ void reduce(int64_t n_rows, int64_t n_inst, int64_t n_verts, int outputs, int64_
             sg_store(r, rec.data() + kSgRowFloats * i);
             for (int s = 0; s < n_slots; ++s) key[n_slots * i + s] = sg_key(live, vk, inst, slot0 + s, n_verts, n_keys);
         }
-        std::vector<uint32_t> vals(m);
-        std::iota(vals.begin(), vals.end(), 0u);
-        std::stable_sort(vals.begin(), vals.end(), [&](uint32_t a, uint32_t b) { return key[a] < key[b]; });
-        std::vector<uint64_t> keys(m);
-        for (int64_t j = 0; j < m; ++j) keys[j] = key[vals[j]];
-        std::vector<uint32_t> start(n_keys);
-        for (int64_t j = 0; j < m; ++j) dg_run_start(j, keys.data(), n_keys, start.data());
-        const uint64_t slots = dg_next_size(m);
-        std::vector<uint32_t> lk[2], li[2];
-        std::vector<float> lv[2];
-        for (int b = 0; b < 2; ++b) { lk[b].assign(slots, kDgEmpty); li[b].assign(slots, 0); lv[b].assign(3 * slots, 0.0f); }
-        DgLevel lev[2] = {{lk[0].data(), li[0].data(), lv[0].data()}, {lk[1].data(), li[1].data(), lv[1].data()}};
-        for (int64_t j = 0; j < m; ++j)
-            dg_level0_with(j, m, keys.data(), vals.data(), start.data(), n_keys,
-                           [&](uint32_t e, float out[3]) { sg_contrib(rec.data(), slot0, n_slots, e, out); }, acc.data(),
-                           lev[0]);
-        uint64_t size = m, len = m;
-        int cur = 0;
-        while (len > kDgGroup) {
-            size = dg_next_size(size);
-            len = (len + kDgGroup - 1) / kDgGroup;
-            std::fill(lk[cur ^ 1].begin(), lk[cur ^ 1].end(), kDgEmpty);
-            for (uint64_t j = 0; j < size; ++j) dg_level_at(j, size, lev[cur], acc.data(), lev[cur ^ 1]);
-            cur ^= 1;
-        }
+        dg_reduce_host(key, n_keys, [&](uint32_t e, float out[3]) { sg_contrib(rec.data(), slot0, n_slots, e, out); },
+                       acc.data());
     }
     if (grad_vertices) std::copy(acc.begin(), acc.begin() + 3 * n_verts, grad_vertices);
     if (grad_transforms)

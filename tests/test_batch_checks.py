@@ -55,6 +55,12 @@ ENTRY = {
     # one hit row, no row_ray: the rows must be the window's rays
     "rt_ray_grad": ("raygrad", lambda L, a, rd, o: L.rt_ray_grad(rd, o, 1, None, a, a, a, a, 3, a, 1, a, a, None, None, 0,
                                                                  None)),
+    # one instance of one 3-vertex member; grad_origins only, no workspace
+    "rt_scene_ray_grad": ("raygrad", lambda L, a, rd, o: L.rt_scene_ray_grad(a, 1, a, 1, 3, rd, o, 1, None, a, a, a, a, a,
+                                                                             None, None, None, None, 0, None)),
+    # grad_points only, no workspace
+    "rt_scene_distance_grad": ("point", lambda L, a, rd, o: L.rt_scene_distance_grad(a, 1, a, 1, 3, rd, o, a, a, a, a, a,
+                                                                                       a, a, None, None, None, 0, None)),
 }
 
 # case -> (descriptor edit, (ray_first, ray_count) or None for NULL opts, expected code per column)

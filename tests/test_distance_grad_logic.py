@@ -161,25 +161,10 @@ def test_finite_differences_of_the_binary64_oracle():
             assert abs(gv[j, a] - fd) <= 1e-4 * max(1.0, abs(fd)), (j, a, gv[j, a], fd)
 
 
-def documented_order(gp, value, t, uv, faces, n_verts, window):
-    """grad_vertices in float32 numpy following DESIGN.md §4.9: per window, each vertex's contributions in (point,
-    corner) order through tree_sum, added to a +0 start in window order"""
-    out = np.zeros((n_verts, 3), np.float32)
-    n = len(gp)
-    window = window or n
-    for base in range(0, n, window):
-        lists = {}
-        for i in range(base, min(n, base + window)):
-            a = abs(float(value[i]))
-            if not (0 < a < np.inf) or t[i] < 0:
-                continue
-            u0, u1 = np.float32(uv[i, 0]), np.float32(uv[i, 1])
-            ws = (u0, u1, np.float32(np.float32(np.float32(1) - u0) - u1))
-            for k in range(3):
-                lists.setdefault(int(faces[t[i], k]), []).append((-ws[k] * gp[i]).astype(np.float32))
-        for vtx, cs in lists.items():
-            out[vtx] = (out[vtx] + D.tree_sum(np.asarray(cs))).astype(np.float32)
-    return out
+def live_points(value, t):
+    """the points that contribute: |value| positive and finite, and a triangle"""
+    a = np.abs(np.asarray(value, np.float64))
+    return (a > 0) & (a < np.inf) & (np.asarray(t) >= 0)
 
 
 @pytest.mark.parametrize("window", [0, 1000, 777])
@@ -191,7 +176,7 @@ def test_summation_order_is_the_documented_tree(window):
     p = np.concatenate([corner, rng.uniform(-1, 1, (1500, 3)).astype(np.float32)])
     g = rng.normal(size=len(p)).astype(np.float32)
     gp, gv, (_, value, c, t, uv) = grads(v, f, p, g=g, window=window)
-    bits_equal(gv, documented_order(gp, value, t, uv, f, len(v), window), f"window {window}")
+    bits_equal(gv, D.documented_order(gp, uv, live_points(value, t), t, f, len(v), window), f"window {window}")
 
 
 def test_result_of_a_vertex_depends_on_its_own_list_only():
@@ -212,6 +197,6 @@ def test_result_of_a_vertex_depends_on_its_own_list_only():
     # one window per point: the sums are added point by point in order
     _, gv1, _ = grads(v, f, p[:200], window=1)
     _, gv0, inputs = grads(v, f, p[:200])
-    bits_equal(gv1, documented_order(D.sim_grad(p[:200], *inputs, f, len(v))[0], inputs[1], inputs[3], inputs[4], f,
-                                     len(v), 1), "window 1")
+    bits_equal(gv1, D.documented_order(D.sim_grad(p[:200], *inputs, f, len(v))[0], inputs[4],
+                                       live_points(inputs[1], inputs[3]), inputs[3], f, len(v), 1), "window 1")
     np.testing.assert_allclose(gv1, gv0, atol=1e-5)

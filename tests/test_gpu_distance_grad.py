@@ -14,6 +14,7 @@ import torch
 
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "distgrad"))
 import distgrad as D  # noqa: E402
+from helpers import window_of  # noqa: E402
 from test_closest_point_logic import MESHES, sample_points  # noqa: E402
 from test_gpu_closest_point import distributions  # noqa: E402
 from triro import synth  # noqa: E402
@@ -72,15 +73,6 @@ def test_cuda_matches_hostsim_true_size(cuda_device, cfg):
     gpu_vs_sim(r, p, g, True, what=cfg + " signed")
 
 
-def window_of(n, n_verts, workspace_bytes):
-    """the window rt_distance_grad picks: the largest whose workspace fits"""
-    lo, hi = 0, n + 1
-    while hi - lo > 1:
-        mid = (lo + hi) // 2
-        lo, hi = (mid, hi) if hops.distance_grad_workspace_bytes(mid, n_verts) <= workspace_bytes else (lo, mid)
-    return lo
-
-
 def test_windows_and_repeatability(cuda_device):
     v, f = synth.icosphere(5)
     r = make(v, f)
@@ -93,7 +85,7 @@ def test_windows_and_repeatability(cuda_device):
     gp2, gv2 = hops.distance_grad(pt, gt, d, c, t, uv, r.mesh_faces, len(v))
     assert same(gp1, gp2) and same(gv1, gv2)
     for ws in (hops.distance_grad_workspace_bytes(100_000, len(v)) + 1000, hops.distance_grad_workspace_bytes(7777, len(v))):
-        w = window_of(len(p), len(v), ws)
+        w = window_of(len(p), lambda k: hops.distance_grad_workspace_bytes(k, len(v)), ws)
         assert w < len(p)
         gpu_vs_sim(r, p, g, workspace_bytes=ws, window=w, what=f"window {w}")
     with pytest.raises(ValueError, match="workspace"):

@@ -14,6 +14,7 @@ import torch
 
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "raygrad"))
 import deep_overlap_cases as DO  # noqa: E402
+from helpers import window_of  # noqa: E402
 import raygrad as R  # noqa: E402
 from test_closest_point_logic import MESHES  # noqa: E402
 from test_ray_grad_logic import random_rays  # noqa: E402
@@ -99,15 +100,6 @@ def test_deep_overlap_all_hits(cuda_device, scene, max_hits):
         gpu_vs_sim(r, o, d, "compact", seed=3, what=scene)
 
 
-def window_of(n, n_verts, workspace_bytes):
-    """the window rt_ray_grad picks: the largest whose workspace fits"""
-    lo, hi = 0, n + 1
-    while hi - lo > 1:
-        mid = (lo + hi) // 2
-        lo, hi = (mid, hi) if hops.ray_grad_workspace_bytes(mid, n_verts) <= workspace_bytes else (lo, mid)
-    return lo
-
-
 def test_windows_and_repeatability(cuda_device):
     v, f = synth.icosphere(5)
     r = make(v, f, max_hits=16)
@@ -120,7 +112,7 @@ def test_windows_and_repeatability(cuda_device):
         assert all(same(a, b) for a, b in zip(g1, g2))
         n_rows = int(rows[0].shape[0])
         for ws in (hops.ray_grad_workspace_bytes(100_000, len(v)) + 1000, hops.ray_grad_workspace_bytes(7777, len(v))):
-            w = window_of(n_rows, len(v), ws)
+            w = window_of(n_rows, lambda k: hops.ray_grad_workspace_bytes(k, len(v)), ws)
             assert w < n_rows
             gpu_vs_sim(r, o, d, mode, seed=4, workspace_bytes=ws, window=w, what=f"window {w}", rows=rows)
     ot, dt = torch.from_numpy(o).cuda(), torch.from_numpy(d).cuda()

@@ -1,6 +1,6 @@
 """Gradients of instanced-scene queries on the GPU (rt_scene_ray_grad, rt_scene_distance_grad and the autograd of
 RayMeshScene.intersects_closest / closest_point / signed_distance): every gradient against the host simulator of
-rt_scene_grad.cu bit for bit over batch layouts, row windows and repeat runs; one identity instance against
+rt_distgrad.cu bit for bit over batch layouts, row windows and repeat runs; one identity instance against
 RayMeshIntersector; autograd behaviour (leaf dtypes and devices, shared members, grad mode, double backward,
 update() and in-place changes); empty cases; and two pose fits by gradient descent."""
 from __future__ import annotations
@@ -20,7 +20,7 @@ import scenegrad as sg  # noqa: E402
 import scenepoint as sp  # noqa: E402
 import scene_cases as cases  # noqa: E402
 import scene_point_cases as spc  # noqa: E402
-from helpers import assert_bits_equal  # noqa: E402
+from helpers import assert_bits_equal, window_of  # noqa: E402
 from triro import synth  # noqa: E402
 from triro.backend import ops as hops  # noqa: E402
 from triro.ray.ray_optix import RayMeshIntersector  # noqa: E402
@@ -98,17 +98,6 @@ def point_case(scene, sim, p, signed, seed, workspace_bytes=None, window=0, what
     return got
 
 
-def window_of(n, n_inst, n_verts, workspace_bytes):
-    """the window the kernels pick: the largest whose workspace fits"""
-    lo, hi = 1, n
-    if hops.scene_grad_workspace_bytes(n, n_inst, n_verts, 3) <= workspace_bytes:
-        return n
-    while hi - lo > 1:
-        mid = (lo + hi) // 2
-        lo, hi = (mid, hi) if hops.scene_grad_workspace_bytes(mid, n_inst, n_verts, 3) <= workspace_bytes else (lo, mid)
-    return lo
-
-
 def test_kernels_equal_the_simulator(big):
     scene, sim, o, d, p = big
     for compact in (False, True):
@@ -141,12 +130,16 @@ def test_windows(big):
     scene, sim, o, d, p = big
     n_inst, n_verts = scene.instance_mesh.numel(), scene._grad_members()[1]
     h = o.shape[0]
+
+    def sizes(k):
+        return hops.scene_grad_workspace_bytes(k, n_inst, n_verts, 3)
+
     for ws in (hops.scene_grad_workspace_bytes(1000, n_inst, n_verts, 3),
                hops.scene_grad_workspace_bytes(333, n_inst, n_verts, 3)):
-        w = window_of(h, n_inst, n_verts, ws)
+        w = window_of(h, sizes, ws)
         assert w < h
         ray_case(scene, sim, o, d, False, seed=5, workspace_bytes=ws, window=w, what=f"ray window {w}")
-        w = window_of(p.shape[0], n_inst, n_verts, ws)
+        w = window_of(p.shape[0], sizes, ws)
         point_case(scene, sim, p, False, seed=6, workspace_bytes=ws, window=w, what=f"point window {w}")
     with pytest.raises(ValueError, match="workspace"):
         ray_case(scene, sim, o, d, False, seed=5, workspace_bytes=1024)

@@ -224,24 +224,6 @@ def test_per_ray_sums_run_in_row_order():
     assert (go[counts == 0] == 0).all()
 
 
-def documented_order(q, w, live, tri, faces, n_verts, window):
-    out = np.zeros((n_verts, 3), np.float32)
-    n = len(q)
-    window = window or n
-    for base in range(0, n, window):
-        lists = {}
-        for i in range(base, min(n, base + window)):
-            if not live[i]:
-                continue
-            u0, u1 = np.float32(w[i, 0]), np.float32(w[i, 1])
-            ws = (u0, u1, np.float32(np.float32(np.float32(1) - u0) - u1))
-            for k in range(3):
-                lists.setdefault(int(faces[tri[i], k]), []).append((-ws[k] * q[i]).astype(np.float32))
-        for vtx, cs in lists.items():
-            out[vtx] = (out[vtx] + D.tree_sum(np.asarray(cs))).astype(np.float32)
-    return out
-
-
 @pytest.mark.parametrize("window", [0, 1000, 777, 1])
 def test_vertex_sums_are_the_documented_tree(window):
     v, f = synth.icosphere(2)
@@ -255,7 +237,7 @@ def test_vertex_sums_are_the_documented_tree(window):
     gu = rng.normal(size=(len(o), 2)).astype(np.float32)
     _, _, gv = R.sim_grad(o, d, tri, gl, gu, v, f, window=window)
     _, _, q, w, live = R.sim_rows(o, d, tri, gl, gu, v, f)
-    bits_equal(gv, documented_order(q, w, live, tri, f, len(v), window), f"window {window}")
+    bits_equal(gv, D.documented_order(q, w, live, tri, f, len(v), window), f"window {window}")
 
 
 def test_workspace_sizes_and_argument_checks():
@@ -268,6 +250,16 @@ def test_workspace_sizes_and_argument_checks():
     assert 100 < per_row < 110                     # DESIGN §4.10: about 105 B per row
     assert hops.ray_grad_workspace_bytes(1000, 10_000) - hops.ray_grad_workspace_bytes(1000, 0) == 40_192   # 4 B per vertex
     assert hops.ray_grad_workspace_bytes(10**10, 5) == hops.ray_grad_workspace_bytes((1 << 30) // 3, 5)
+    # the exact layouts (DESIGN §4.9, §4.10, §4.13): (n_rows, n_verts) -> (distance, ray) bytes
+    for (n, nv), (dist, ray) in {(1, 0): (19456, 19712), (1000, 10000): (148736, 156928), (7777, 642): (773376, 835840),
+                                 (10_000_000, 163842): (975670784, 1055670784),
+                                 (10**10, 5): (34896617984, 37759929600)}.items():
+        assert hops.distance_grad_workspace_bytes(n, nv) == dist, (n, nv)
+        assert hops.ray_grad_workspace_bytes(n, nv) == ray, (n, nv)
+    for args, want in {(1, 1, 3, 1): 19968, (1, 1, 3, 2): 19968, (1, 1, 3, 3): 19968,
+                       (2_073_600, 1000, 10242, 1): 327865344, (2_073_600, 1000, 10242, 3): 505160192,
+                       (1_000_000, 64, 163842, 2): 132140032, (10**10, 7, 9, 3): 37350885632}.items():
+        assert hops.scene_grad_workspace_bytes(*args) == want, args
     wb = C.c_size_t()
     assert lib.rt_ray_grad_sizes(-1, 3, C.byref(wb)) != 0
     assert lib.rt_ray_grad_sizes(3, 1 << 32, C.byref(wb)) != 0

@@ -1,4 +1,4 @@
-"""Gradients of instanced-scene queries on the CPU (DESIGN.md §4.13): the host simulator of rt_scene_grad.cu (the
+"""Gradients of instanced-scene queries on the CPU (DESIGN.md §4.13): the host simulator of rt_distgrad.cu (the
 kernels' own RT_HD code) against a numpy restatement of the contract, bit for bit; against the single-mesh
 simulators on the scene flattened with the kernels' binary32 world vertices, bit for bit; against central
 differences of the binary64 contract; the translation and direction-scaling identities; and row windows."""

@@ -1,4 +1,4 @@
-"""Gradients of instanced-scene queries on one GPU (rt_scene_grad.cu through RayMeshScene's autograd, DESIGN.md
+"""Gradients of instanced-scene queries on one GPU (rt_distgrad.cu through RayMeshScene's autograd, DESIGN.md
 §4.13): backward against forward time, and one pose-optimisation step against what a user does without the feature.
 
 - Ray rows: the scenes of BASELINE §11, "icos20k_x1000" (1 000 instances of a 20 480-triangle icosphere, random

@@ -1,4 +1,4 @@
-// rt_scenegrad.cuh — the arithmetic of the instanced-scene gradients (rt_scene_grad.cu, DESIGN.md §4.13): the per-row
+// rt_scenegrad.cuh — the arithmetic of the instanced-scene gradients (rt_distgrad.cu, DESIGN.md §4.13): the per-row
 // factors of hit rows and point rows, the pairs of the joint key space and their level-0 contributions.  Everything
 // here is RT_HD, like rt_raygrad.cuh, so that tests/scenegrad/ runs exactly the code the kernels run.
 //

@@ -972,6 +972,22 @@ def signed_distance_pseudonormal(accel_structure, points: torch.Tensor, ray_firs
     return sd
 
 
+def _check_grad_inputs(dev, specs):
+    """ValueError unless every (name, tensor, shape, dtype) of specs whose tensor is not None is dtype shape on dev"""
+    for name, t, shape, dt in specs:
+        if t is not None and (tuple(t.shape) != tuple(shape) or t.dtype != dt or t.device != dev):
+            raise ValueError(f"{name} must be {dt} {tuple(shape)} on {dev}, got {t.dtype} {tuple(t.shape)} on {t.device}")
+
+
+def _grad_workspace(dev, reduce: bool, sizes, workspace_bytes: int | None):
+    """(workspace, its size in bytes) of a gradient call: none when it forms no vertex or transform sums, else
+    workspace_bytes (default sizes(): one window for every row)"""
+    if not reduce:
+        return None, 0
+    wb = sizes() if workspace_bytes is None else int(workspace_bytes)
+    return torch.empty(max(wb, 256), dtype=torch.uint8, device=dev), wb
+
+
 def distance_grad_workspace_bytes(n_points: int, n_verts: int) -> int:
     """Workspace rt_distance_grad needs to run a batch of n_points as one window."""
     wb = C.c_size_t()
@@ -993,21 +1009,16 @@ def distance_grad(points: torch.Tensor, grad_out: torch.Tensor, value: torch.Ten
     rd, batch = make_ray_desc(points, None)
     dev = points.device
     n = rd.nray
-    for name, t, shape, dt in (("grad_out", grad_out, batch, torch.float32), ("value", value, batch, torch.float32),
-                               ("closest", closest, (*batch, 3), torch.float32), ("tri", tri, batch, torch.int32),
-                               ("uv", uv, (*batch, 2), torch.float32)):
-        if tuple(t.shape) != tuple(shape) or t.dtype != dt or t.device != dev:
-            raise ValueError(f"{name} must be {dt} {tuple(shape)} on {dev}, got {t.dtype} {tuple(t.shape)} on {t.device}")
+    _check_grad_inputs(dev, (("grad_out", grad_out, batch, torch.float32), ("value", value, batch, torch.float32),
+                             ("closest", closest, (*batch, 3), torch.float32), ("tri", tri, batch, torch.int32),
+                             ("uv", uv, (*batch, 2), torch.float32)))
     if faces.dtype != torch.int32 or faces.dim() != 2 or faces.shape[1] != 3 or faces.device != dev:
         raise ValueError("faces must be int32 [f, 3] on the points' device")
     grad_out, value, closest, tri, uv, faces = (t.contiguous() for t in (grad_out, value, closest, tri, uv, faces))
     with _on_device(dev):
         gp = torch.empty((*batch, 3), dtype=torch.float32, device=dev) if points_grad else None
         gv = torch.empty((int(n_verts), 3), dtype=torch.float32, device=dev) if vertices_grad else None
-        wb = 0
-        if gv is not None:
-            wb = distance_grad_workspace_bytes(n, n_verts) if workspace_bytes is None else int(workspace_bytes)
-        ws = torch.empty(max(wb, 256), dtype=torch.uint8, device=dev) if gv is not None else None
+        ws, wb = _grad_workspace(dev, vertices_grad, lambda: distance_grad_workspace_bytes(n, n_verts), workspace_bytes)
         _check(get_module().rt_distance_grad(C.byref(rd), C.byref(trace_opts()), _ptr(grad_out), _ptr(value),
                                              _ptr(closest), _ptr(tri), _ptr(uv), _ptr(faces), faces.shape[0],
                                              int(n_verts), _ptr(gp), _ptr(gv), _ptr(ws), wb, _stream(dev)),
@@ -1041,10 +1052,8 @@ def ray_grad(origins: torch.Tensor, dirs: torch.Tensor, tri: torch.Tensor, grad_
     h = tri.shape[0] if tri.dim() == 1 else -1
     if ray_idx is None and h != rd.nray:
         raise ValueError(f"tri must have one row per ray ({rd.nray}) without ray_idx, got {tuple(tri.shape)}")
-    for name, t, shape, dt in (("tri", tri, (h,), torch.int32), ("grad_loc", grad_loc, (h, 3), torch.float32),
-                               ("grad_uv", grad_uv, (h, 2), torch.float32), ("ray_idx", ray_idx, (h,), torch.int32)):
-        if t is not None and (tuple(t.shape) != shape or t.dtype != dt or t.device != dev):
-            raise ValueError(f"{name} must be {dt} {shape} on {dev}, got {t.dtype} {tuple(t.shape)} on {t.device}")
+    _check_grad_inputs(dev, (("tri", tri, (h,), torch.int32), ("grad_loc", grad_loc, (h, 3), torch.float32),
+                             ("grad_uv", grad_uv, (h, 2), torch.float32), ("ray_idx", ray_idx, (h,), torch.int32)))
     if vertices.dim() != 2 or vertices.shape[1] != 3 or vertices.device != dev:
         raise ValueError("vertices must be float32 [n, 3] on the rays' device")
     if faces.dtype != torch.int32 or faces.dim() != 2 or faces.shape[1] != 3 or faces.device != dev:
@@ -1056,10 +1065,7 @@ def ray_grad(origins: torch.Tensor, dirs: torch.Tensor, tri: torch.Tensor, grad_
         go = torch.empty((*batch, 3), dtype=torch.float32, device=dev) if origins_grad else None
         gd = torch.empty((*batch, 3), dtype=torch.float32, device=dev) if directions_grad else None
         gv = torch.empty((n_verts, 3), dtype=torch.float32, device=dev) if vertices_grad else None
-        wb = 0
-        if gv is not None:
-            wb = ray_grad_workspace_bytes(h, n_verts) if workspace_bytes is None else int(workspace_bytes)
-        ws = torch.empty(max(wb, 256), dtype=torch.uint8, device=dev) if gv is not None else None
+        ws, wb = _grad_workspace(dev, vertices_grad, lambda: ray_grad_workspace_bytes(h, n_verts), workspace_bytes)
         _check(get_module().rt_ray_grad(C.byref(rd), C.byref(trace_opts()), h, _ptr(ray_idx), _ptr(tri), _ptr(grad_loc),
                                         _ptr(grad_uv), _ptr(vertices), n_verts, _ptr(faces), faces.shape[0], _ptr(go),
                                         _ptr(gd), _ptr(gv), _ptr(ws), wb, _stream(dev)), "rt_ray_grad")
@@ -1313,10 +1319,8 @@ def _scene_grad_outputs(dev, n_inst: int, n_verts: int, n_rows: int, transforms_
     gt = torch.empty((n_inst, 3, 4), dtype=torch.float32, device=dev) if transforms_grad else None
     gv = torch.empty((n_verts, 3), dtype=torch.float32, device=dev) if vertices_grad else None
     outputs = (SCENE_GRAD_TRANSFORMS if transforms_grad else 0) | (SCENE_GRAD_VERTICES if vertices_grad else 0)
-    wb = 0
-    if outputs:
-        wb = scene_grad_workspace_bytes(n_rows, n_inst, n_verts, outputs) if workspace_bytes is None else int(workspace_bytes)
-    ws = torch.empty(max(wb, 256), dtype=torch.uint8, device=dev) if outputs else None
+    ws, wb = _grad_workspace(dev, outputs != 0, lambda: scene_grad_workspace_bytes(n_rows, n_inst, n_verts, outputs),
+                             workspace_bytes)
     return gt, gv, ws, wb
 
 
@@ -1342,11 +1346,9 @@ def scene_ray_grad(table: torch.Tensor, n_inst: int, members: torch.Tensor, n_ve
     h = tri.shape[0] if tri.dim() == 1 else -1
     if ray_idx is None and h != rd.nray:
         raise ValueError(f"tri must have one row per ray ({rd.nray}) without ray_idx, got {tuple(tri.shape)}")
-    for name, t, shape, dt in (("inst", inst, (h,), torch.int32), ("tri", tri, (h,), torch.int32),
-                               ("grad_loc", grad_loc, (h, 3), torch.float32), ("grad_uv", grad_uv, (h, 2), torch.float32),
-                               ("ray_idx", ray_idx, (h,), torch.int32)):
-        if t is not None and (tuple(t.shape) != shape or t.dtype != dt or t.device != dev):
-            raise ValueError(f"{name} must be {dt} {shape} on {dev}, got {t.dtype} {tuple(t.shape)} on {t.device}")
+    _check_grad_inputs(dev, (("inst", inst, (h,), torch.int32), ("tri", tri, (h,), torch.int32),
+                             ("grad_loc", grad_loc, (h, 3), torch.float32), ("grad_uv", grad_uv, (h, 2), torch.float32),
+                             ("ray_idx", ray_idx, (h,), torch.int32)))
     scene = _scene_member_args(table, n_inst, members, n_verts, dev)
     inst, tri, grad_loc, grad_uv, ray_idx = (None if t is None else t.contiguous() for t in
                                              (inst, tri, grad_loc, grad_uv, ray_idx))
@@ -1370,11 +1372,9 @@ def scene_point_grad(table: torch.Tensor, n_inst: int, members: torch.Tensor, n_
     tensor_input_check(points)
     rd, batch = make_ray_desc(points, None)
     dev = points.device
-    for name, t, shape, dt in (("grad_out", grad_out, batch, torch.float32), ("value", value, batch, torch.float32),
-                               ("closest", closest, (*batch, 3), torch.float32), ("inst", inst, batch, torch.int32),
-                               ("tri", tri, batch, torch.int32), ("uv", uv, (*batch, 2), torch.float32)):
-        if tuple(t.shape) != tuple(shape) or t.dtype != dt or t.device != dev:
-            raise ValueError(f"{name} must be {dt} {tuple(shape)} on {dev}, got {t.dtype} {tuple(t.shape)} on {t.device}")
+    _check_grad_inputs(dev, (("grad_out", grad_out, batch, torch.float32), ("value", value, batch, torch.float32),
+                             ("closest", closest, (*batch, 3), torch.float32), ("inst", inst, batch, torch.int32),
+                             ("tri", tri, batch, torch.int32), ("uv", uv, (*batch, 2), torch.float32)))
     scene = _scene_member_args(table, n_inst, members, n_verts, dev)
     grad_out, value, closest, inst, tri, uv = (t.contiguous() for t in (grad_out, value, closest, inst, tri, uv))
     with _on_device(dev):
